@@ -2,7 +2,7 @@
 """Benchmark of the grid->region aggregation hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload config2|config3|config4|config1|config5] [--no-also]
+                    [--workload config2|config3|config4|config1|config5] [--no-also] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic batch of the workload
 (config2: 4 x 365 days of 0.25-degree tas [1460][720][1440] f32 -> 24,378 regions, popwt).
@@ -12,13 +12,19 @@ N > 1 (torchrun, one rank per GPU): `value` is weak scaling -- every rank aggreg
 time over the ranks, compute + the final NCCL gather of the region x time outputs (overlapped).
 Prints ONE JSON line on rank 0.  `also` (N = 1) carries device-timed lines of the other
 BASELINE.json configs and of input variants (NaN over the ocean, annual sums).
+`--dump-outputs DIR` writes rank 0's result block of the last timed step, one DIR/<output>.npy per output
+(float64, [regions][days]); the inputs are seeded, so two builds run with the same arguments can be compared
+output for output.  The benchmark writes nothing into the repository tree.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import sys
+import tempfile
 import threading
 import time
 
@@ -48,6 +54,9 @@ YEARS_PER_STEP, POOL, ENSEMBLE_YEARS = 8, 4, 21 * 2 * 95
 METRIC = "region-days/sec"
 PARAMS = {"identity": (), "poly": (273.15, 1, 2, 3, 4), "edd": (283.15, 303.15)}
 KERNEL = {"identity": "agg_stream_kernel", "poly": "agg_stream_kernel", "edd": "agg_stream_kernel"}
+# --dump-outputs: one file per output of the kind (the names the e2e leg gives them)
+OUTPUT_NAMES = {"identity": ("tas",), "poly": ("p1", "p2", "p3", "p4"), "edd": ("edd10", "edd30")}
+DUMP_BYTES = 63_000_000          # array bytes: with the .npy headers the files stay under 64 MB
 # fp64-pipe lane slots per CSR entry and day of the Snyder kernel (2 thresholds): executed DFMA + DMUL + DADD +
 # DSETP warp instructions x 32 / entry-days (profiles/r2_ncu_full_agg_stream_kernel_config4.json: 690 M warp
 # instructions for 3.07e8 entry-days; the zero-weight padding of the quads is overhead, not work); 64 fp64
@@ -61,6 +70,22 @@ def _peaks():
     if os.path.exists(p):
         return float(json.load(open(p))["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs, burst copy)"
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+def dump_outputs(out, kind, dirname, budget=DUMP_BYTES):
+    """Write the result block ``out`` [n_out][R][n_cols] (float64) as dirname/<output>.npy, one [R][n_cols]
+    array per output.  A block larger than ``budget`` keeps a fixed, seeded sample of its region rows (sorted,
+    the same for every run and build of the workload) and all of its columns."""
+    import torch
+    n_out, R, n_cols = out.shape
+    rows = min(R, max(1, budget // (8 * n_out * max(1, n_cols))))
+    if rows < R:
+        pick = np.sort(np.random.default_rng(0).choice(R, size=rows, replace=False))
+        out = out.index_select(1, torch.from_numpy(pick).to(out.device))
+    host = out.cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in zip(OUTPUT_NAMES[kind], host):
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def config_dict(workload, T, world):
@@ -223,7 +248,13 @@ class Bench:
         import torch
         import torch.distributed as dist
         import __graft_entry__ as G
-        G.build()
+        if G._stale() and not os.environ.get("CTB_LIBRARY"):
+            # the tree may be read-only: a library missing from it or older than its sources is built in a
+            # temporary directory instead, removed at exit
+            tmp = tempfile.mkdtemp(prefix="ctb_bench_")
+            atexit.register(shutil.rmtree, tmp, True)
+            os.environ["CTB_LIBRARY"] = os.path.join(tmp, "libctb.so")
+            G.compile_library(os.environ["CTB_LIBRARY"])
         from climate_toolbox_b200 import _engine as E
         from climate_toolbox_b200 import _native as N
         from climate_toolbox_b200 import synthetic
@@ -430,6 +461,8 @@ def run_ours(args):
     head = B.device_run(args.workload, args.steps, args.warmup, T=T)
     clocks = sampler.result()
     plan, xs, out = head["plan"], head["xs"], head["out"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, kind, args.dump_outputs)
     info = plan.info
     roofline = B.roofline(args.workload, plan, T, head["kern_ms"], traffic_all.get(args.workload))
     streaming = args.workload == "config5"
@@ -678,7 +711,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the device-timed lines of the other configs")
     ap.add_argument("--no-pageable", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs as DIR/<output>.npy (float64, at most 64 MB in all: "
+                         "a fixed, seeded sample of regions when the block is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    sys.dont_write_bytecode = True          # nothing lands in the tree, which may be read-only
     if args.impl == "reference":
         run_reference(args)
     else:
