@@ -196,7 +196,9 @@ def _time_group_ids(ds, dim, n, spec):
 
 def _group_requests(reqs):
     """Fuse requests that read the same sources: poly orders / EDD thresholds /
-    GDD pairs become extra outputs of ONE pass over the data (config 3/4)."""
+    GDD pairs / contiguous temperature bins become extra outputs of ONE pass over
+    the data (config 3/4).  A bin (offset, lo, hi) joins a group of bins whose
+    last edge is lo: the group's params are (offset, e_0, ..., e_n)."""
     groups = []
     for name, kind, params, srcs in reqs:
         placed = False
@@ -207,10 +209,12 @@ def _group_requests(reqs):
                 for a, b in zip(g["srcs"], srcs))
             if not same_src or g["kind"] != kind or len(g["names"]) >= N.MAX_OUT:
                 continue
-            if kind == "identity" or (kind == "poly" and g["params"][0] != params[0]):
+            if kind == "identity" or (kind in ("poly", "bins") and g["params"][0] != params[0]):
+                continue
+            if kind == "bins" and g["params"][-1] != params[1]:
                 continue
             g["names"].append(name)
-            g["params"] = g["params"] + (params[1:] if kind == "poly" else params)
+            g["params"] = g["params"] + (params[1:] if kind == "poly" else params[2:] if kind == "bins" else params)
             placed = True
             break
         if not placed:
@@ -455,7 +459,7 @@ def weighted_aggregate_grid_to_regions(ds, variable, aggwt, agglev, weights=None
         arrays (host; copied in time chunks) or CUDA tensors (device-resident),
         in ``(time, lat, lon)`` or ``(lat, lon, time)`` order, float32/float64.
     variable : str or list of str
-        Variable(s) to aggregate.  Deferred transforms (``tas_poly``,
+        Variable(s) to aggregate.  Deferred transforms (``tas_poly``, ``tas_bins``,
         ``snyder_edd``, ``snyder_gdd``) of the same source are fused into one pass.
     aggwt, agglev : str
         Weight / region-id column names in ``weights``.

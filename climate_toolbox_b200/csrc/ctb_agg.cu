@@ -179,6 +179,7 @@ int run_kind(const ctb_plan* P, const AggArgs& a, int layout, int variant, bool 
     case CTB_TR_POLY: return run_nout<TIN, CTB_TR_POLY>(P, a, layout, variant, vec, n_out, st);
     case CTB_TR_EDD: return run_nout<TIN, CTB_TR_EDD>(P, a, layout, variant, vec, n_out, st);
     case CTB_TR_GDD: return run_nout<TIN, CTB_TR_GDD>(P, a, layout, variant, vec, n_out, st);
+    case CTB_TR_BINS: return run_nout<TIN, CTB_TR_BINS>(P, a, layout, variant, vec, n_out, st);
   }
   ctb_set_error("transform=%d unsupported", kind);
   return CTB_ERR_INVALID;
@@ -337,6 +338,34 @@ int ctb_pack_transform(int transform, const double* params, int n_params, int n_
         const float f = (float)e;          // nearest; then the neighbours that bracket e
         out->up[j] = (double)f < e ? std::nextafterf(f, INFINITY) : f;
         out->dn[j] = (double)f > e ? std::nextafterf(f, -INFINITY) : f;
+      }
+      return CTB_OK;
+    }
+    case CTB_TR_BINS: {
+      // {offset, e_0..e_nout}: n_out contiguous bins [e_j, e_j+1) (at most 1 + 5 of the 8 slots of CtbTr::a)
+      if (!need(n_out + 2)) return CTB_ERR_INVALID;
+      if (!std::isfinite(params[0])) {
+        ctb_set_error("BINS offset %g is not finite", params[0]);
+        return CTB_ERR_INVALID;
+      }
+      // strictly increasing edges can be infinite only at the ends: -inf first, +inf last
+      for (int j = 0; j <= n_out; ++j) {
+        const double e = params[1 + j];
+        if (std::isnan(e) || (j > 0 && !(e > params[j]))) {
+          ctb_set_error("BINS edges must be strictly increasing and not NaN: edge %d is %g", j, e);
+          return CTB_ERR_INVALID;
+        }
+      }
+      for (int j = 0; j < n_out + 2; ++j) out->a[j] = params[j];
+      // float inputs: up[j] = the least float f with fl64(f - offset) >= e_j (-inf for e_0 = -inf, +inf for
+      // e_nout = +inf), so that f >= up[j] decides the edge on the stored type (ctb_bins_in_f32)
+      for (int j = 0; j <= n_out; ++j) {
+        const double e = params[1 + j];
+        auto ge = [&](float f) { return (double)f - params[0] >= e; };
+        float f = (float)(e + params[0]);
+        while (f > -INFINITY && ge(f)) f = std::nextafterf(f, -INFINITY);
+        while (!ge(f)) f = std::nextafterf(f, INFINITY);
+        out->up[j] = f;
       }
       return CTB_OK;
     }

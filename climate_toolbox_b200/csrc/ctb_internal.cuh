@@ -276,10 +276,40 @@ __device__ __forceinline__ double ctb_edd(double tmin, double tmax, double M, do
   return ctb_edd_cases(tmin < e, tmax > e, M, W, rW, e);
 }
 
+// Temperature bins: in[j] = e_j <= x - offset < e_{j+1} for the contiguous edges a[1..NOUT+1] (offset
+// a[0]); one fp64 comparison per edge.  x is the stored value widened exactly to double, so the subtraction
+// rounds like the oracle's.  NaN lies in no bin (every comparison is false).
+template <int NOUT>
+__device__ __forceinline__ void ctb_bins_in(const CtbTr& P, double x, bool (&in)[NOUT]) {
+  const double d = x - P.a[0];
+  int k = 0;   // edges at or below d; the edges increase, so d lies in bin j exactly when k == j + 1
+#pragma unroll
+  for (int j = 0; j <= NOUT; ++j) k += d >= P.a[1 + j];
+#pragma unroll
+  for (int j = 0; j < NOUT; ++j) in[j] = k == j + 1;
+}
+
+// The same decisions for a float x on the stored type: up[j] is the least float whose widened value minus
+// the offset is >= e_j (ctb_pack_transform), and that predicate grows with x, so x >= up[j] decides it for
+// every float -- NaN, infinities and negative values included -- with one fp32 comparison per edge.
+template <int NOUT>
+__device__ __forceinline__ void ctb_bins_in_f32(const CtbTr& P, float x, bool (&in)[NOUT]) {
+  bool ge[NOUT + 1];
+#pragma unroll
+  for (int j = 0; j <= NOUT; ++j) ge[j] = x >= P.up[j];
+#pragma unroll
+  for (int j = 0; j < NOUT; ++j) in[j] = ge[j] && !ge[j + 1];
+}
+
 template <int KIND, int NOUT>
 __device__ __forceinline__ void ctb_apply(const CtbTr& P, double x0, double x1, double (&f)[NOUT]) {
   if constexpr (KIND == CTB_TR_IDENTITY) {
     f[0] = x0;
+  } else if constexpr (KIND == CTB_TR_BINS) {
+    bool in[NOUT];
+    ctb_bins_in<NOUT>(P, x0, in);
+#pragma unroll
+    for (int j = 0; j < NOUT; ++j) f[j] = x0 != x0 ? x0 : (in[j] ? 1.0 : 0.0);   // NaN stays NaN (.values)
   } else if constexpr (KIND == CTB_TR_POLY_SEQ) {
     const double d = x0 - P.a[0];
     double p = d;

@@ -194,6 +194,14 @@ __device__ __forceinline__ void add_value(const CtbTr& tr, double w, TIN x, bool
     } else {
       if (on) acc[0] = fma(w, (double)x, acc[0]);
     }
+  } else if constexpr (KIND == CTB_TR_BINS) {
+    // an indicator adds the weight or nothing: no product, and NaN lies in no bin (no check needed)
+    // (float inputs never come here: reduce_region_widen decides their bins for every value)
+    bool in[NOUT];
+    ctb_bins_in<NOUT>(tr, (double)x, in);
+#pragma unroll
+    for (int j = 0; j < NOUT; ++j)
+      if (on && in[j]) acc[j] += w;
   } else {
     double f[NOUT];
     ctb_apply<KIND, NOUT>(tr, (double)x, 0.0, f);
@@ -310,6 +318,13 @@ __device__ __forceinline__ bool reduce_region_widen(const CtbTr& tr, uint32_t ti
       const double x = widen(bb[g]);
       if constexpr (KIND == CTB_TR_IDENTITY) {
         if (on[g]) acc[g][0] = fma(w, x, acc[g][0]);
+      } else if constexpr (KIND == CTB_TR_BINS) {
+        // no widening: the float thresholds decide every float exactly (ctb_bins_in_f32)
+        bool in[NOUT];
+        ctb_bins_in_f32<NOUT>(tr, __uint_as_float(bb[g]), in);
+#pragma unroll
+        for (int j = 0; j < NOUT; ++j)
+          if (on[g] && in[j]) acc[g][j] += w;
       } else {
         double f[NOUT];
         ctb_apply<KIND, NOUT>(tr, x, 0.0, f);
@@ -321,6 +336,7 @@ __device__ __forceinline__ bool reduce_region_widen(const CtbTr& tr, uint32_t ti
   }
 #pragma unroll
   for (int j = 0; j < NOUT; ++j) v[j] = fold_quads(acc[0][j], acc[1][j], acc[2][j], acc[3][j], lane);
+  if constexpr (KIND == CTB_TR_BINS) return true;   // compared on the stored type: no range to check
   const bool ok = bmin >= 0x00800000u && bmax < 0x7f800000u;
   return __all_sync(0xffffffffu, ok);
 }
@@ -684,6 +700,9 @@ __global__ void __launch_bounds__(THREADS, 1) agg_stream_kernel(const AggArgs a)
 #ifndef CTB_POLY34_THREADS
 #define CTB_POLY34_THREADS 640
 #endif
+#ifndef CTB_BINS34_THREADS
+#define CTB_BINS34_THREADS CTB_POLY34_THREADS
+#endif
 #ifndef CTB_EDD1_THREADS
 #define CTB_EDD1_THREADS 640
 #endif
@@ -700,13 +719,17 @@ int launch(const ctb_plan* P, AggArgs a, cudaStream_t st) {
   // three and four polynomial outputs keep 4 fp64 accumulators per output and lane: 20 warps of 96
   constexpr int NIN = NIn<KIND>::v;
   constexpr bool POLY = KIND == CTB_TR_POLY || KIND == CTB_TR_POLY_SEQ;
+  // temperature bins: the polynomial shapes (the same 4 x NOUT accumulators per lane; measured, config 2 shapes,
+  // 4 bins: 512 / 640 / 768 threads = 1.278 / 1.233 / 1.228 ms, profiles/micro/r3_bins_cost.log -- 768 is within
+  // the spread, so the bins keep the polynomial's 640)
+  constexpr bool BINS = KIND == CTB_TR_BINS;
   // Snyder forms: threshold evaluations per gridcell-day -- few warps with many registers: the compiler
   // interleaves the 4 days x EVALS dependency chains of a quad inside one warp (measured, config 4:
   // 768/640/512/448/384/256 threads = 4.53/4.33/4.12/4.49/3.91/5.31 ms; consumer warps a multiple of 4;
   // EDD with 3 or 4 thresholds: 512 threads 3.00/3.92 ms per 730 days, 384 threads 3.03/4.24;
   // GDD with 2 outputs: 3.57 / 3.28)
   constexpr int EVALS = KIND == CTB_TR_GDD ? 2 * NOUT : NOUT;
-  constexpr int THREADS = NIN == 2 ? (EVALS == 1 ? CTB_EDD1_THREADS : (EVALS == 2 || KIND == CTB_TR_GDD) ? CTB_EDD2_THREADS : CTB_EDD34_THREADS) : (POLY && NOUT > 2) ? CTB_POLY34_THREADS : (POLY && NOUT > 1) ? 768 : CTB_STREAM_THREADS;
+  constexpr int THREADS = NIN == 2 ? (EVALS == 1 ? CTB_EDD1_THREADS : (EVALS == 2 || KIND == CTB_TR_GDD) ? CTB_EDD2_THREADS : CTB_EDD34_THREADS) : (POLY && NOUT > 2) ? CTB_POLY34_THREADS : (BINS && NOUT > 2) ? CTB_BINS34_THREADS : ((POLY || BINS) && NOUT > 1) ? 768 : CTB_STREAM_THREADS;
   constexpr int S = CTB_STAGES;   // tile stages: one being reduced, up to two landing
   constexpr size_t SMEM = (size_t)S * Geo<NIN>::TILE_BYTES + 2 * CTB_META_CAP;
   static_assert(SMEM <= 227 * 1024 - 512, "shared memory budget");
@@ -769,6 +792,7 @@ int launch_kind(const ctb_plan* P, const AggArgs& a, int kind, int n_out, cudaSt
   }
   if (kind == CTB_TR_EDD) { CTB_NOUT_SWITCH(CTB_TR_EDD) }
   if (kind == CTB_TR_GDD) { CTB_NOUT_SWITCH(CTB_TR_GDD) }
+  if (kind == CTB_TR_BINS) { CTB_NOUT_SWITCH(CTB_TR_BINS) }
 #undef CTB_NOUT_SWITCH
   ctb_set_error("streaming kernel: transform=%d n_out=%d unsupported", kind, n_out);
   return CTB_ERR_INVALID;

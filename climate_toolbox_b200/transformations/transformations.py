@@ -14,7 +14,7 @@ import torch
 from .._xr import DataArray, Dataset, Deferred, Variable, from_any, to_like
 from ..utils.utils import remove_leap_days, convert_kelvin_to_celsius  # noqa: F401
 
-__all__ = ["snyder_edd", "snyder_gdd", "validate_edd_snyder_agriculture", "tas_poly", "ordinal"]
+__all__ = ["snyder_edd", "snyder_gdd", "validate_edd_snyder_agriculture", "tas_poly", "tas_bins", "ordinal"]
 
 
 def _source(da):
@@ -132,6 +132,78 @@ def tas_poly(ds, power, varname):
         # do transformation: (tas - 273.15) ** power, deferred
         ds1._vars[name] = Variable(tas.dims, None, attrs, None,
                                    Deferred("poly", (273.15, float(p)), (tas,)))
+    return to_like(ds1, like)
+
+
+def _bin_edges(edges):
+    """``edges`` as a float64 array of K+1 >= 2 strictly increasing, non-NaN values; only the first may
+    be -inf and only the last +inf."""
+    e = np.asarray(edges, dtype=np.float64)
+    if e.ndim != 1 or e.size < 2:
+        raise ValueError("edges must be a 1-D sequence of at least 2 values, got {!r}".format(edges))
+    if np.isnan(e).any():
+        raise ValueError("edges must not be NaN: {!r}".format(edges))
+    # strictly increasing edges can be infinite only at the ends (inf - inf is NaN): -inf first, +inf last
+    with np.errstate(invalid="ignore"):
+        increasing = (np.diff(e) > 0).all()
+    if not increasing:
+        raise ValueError("edges must be strictly increasing, infinite only at the ends: {!r}".format(edges))
+    return e
+
+
+def tas_bins(ds, edges, varname="tas_bin"):
+    """
+    Daily average temperature (degrees C) binned: one variable per bin ``[lo, hi)``, 1.0 on the days the
+    temperature lies in the bin, 0.0 otherwise and NaN where ``tas`` is NaN.  Aggregated with
+    ``time_groups="year"`` it gives the (weighted) number of days per year each region spends in the bin.
+
+    Same conventions as :func:`tas_poly` (reads ``ds["tas"]`` in K, leap years removed, at most 365
+    steps, ``time`` as ``YYYYDDD``), so the two can be swapped in a pipeline.  A gridcell-day lies in a bin
+    when ``lo <= tas - 273.15 < hi``, the value widened to float64 before the subtraction.  ``edges``:
+    K+1 strictly increasing values in degrees C for K bins; the first may be ``-inf`` and the last
+    ``+inf``.  ``varname``: a prefix (variables ``"{varname}_{k}"``) or a list of K names.  Contiguous
+    bins of one ``tas`` are fused into one pass per 4 bins when aggregated.
+    """
+    e = _bin_edges(edges)
+    K = e.size - 1
+    names = ["{}_{}".format(varname, k) for k in range(K)] if isinstance(varname, str) else list(varname)
+    if len(names) != K:
+        raise ValueError("{} edges give {} bins, but {} names were given".format(e.size, K, len(names)))
+    like = ds
+    ds = from_any(ds)
+
+    # remove leap years
+    ds = remove_leap_days(ds)
+    tas = _source(ds["tas"])
+
+    # Replace datetime64[ns] 'time' with YYYYDDD int 'day'
+    if ds.dims["time"] > 365:
+        raise ValueError
+    ds1 = Dataset()
+    for k, c in ds._coords.items():
+        if k != "time":
+            ds1._coords[k] = c
+    year = np.asarray(ds["time.year"].values, dtype=np.int64)
+    ds1._coords["time"] = Variable(("time",), year * 1000 + np.arange(1, len(year) + 1))
+
+    for lo, hi, name in zip(e[:-1], e[1:], names):
+        description = (
+            """
+            Days with daily average temperature (degrees C) in [{lo:g}, {hi:g})
+
+            1 on a day whose average temperature lies in the bin, 0 otherwise;
+            summed over a year, the number of days per year in the bin.
+
+            Leap years are removed before counting days (uses a 365 day
+            calendar).
+            """.format(lo=lo, hi=hi)
+        ).strip()
+        attrs = {"units": "days", "bin_lower": float(lo), "bin_upper": float(hi),
+                 "long_title": description.splitlines()[0], "description": description,
+                 "variable": name}
+        # do transformation: lo <= tas - 273.15 < hi, deferred
+        ds1._vars[name] = Variable(tas.dims, None, attrs, None,
+                                   Deferred("bins", (273.15, float(lo), float(hi)), (tas,)))
     return to_like(ds1, like)
 
 

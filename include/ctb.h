@@ -58,8 +58,10 @@ enum { CTB_LAYOUT_TIME_MAJOR = 0, CTB_LAYOUT_CELL_MAJOR = 1 };
  *   IDENTITY  n_in=1            f = x
  *   POLY      n_in=1  params = {offset, p_1..p_nout}   f_j = (x - offset)^p_j   transformations.py:189
  *   EDD       n_in=2  params = {e_1..e_nout}           f_j = SnyderEDD(tmin=x0,tmax=x1,e_j)  transformations.py:69-89
- *   GDD       n_in=2  params = {lo_1,hi_1,..}          f_j = EDD(lo_j) - EDD(hi_j)           transformations.py:139-141 */
-enum { CTB_TR_IDENTITY = 0, CTB_TR_POLY = 1, CTB_TR_EDD = 2, CTB_TR_GDD = 3 };
+ *   GDD       n_in=2  params = {lo_1,hi_1,..}          f_j = EDD(lo_j) - EDD(hi_j)           transformations.py:139-141
+ *   BINS      n_in=1  params = {offset, e_0..e_nout}   f_j = [e_j <= x - offset < e_{j+1}]   (NaN for NaN x; edges strictly
+ *                     increasing, not NaN, only e_0 may be -inf and only e_nout +inf; n_params = n_out + 2) */
+enum { CTB_TR_IDENTITY = 0, CTB_TR_POLY = 1, CTB_TR_EDD = 2, CTB_TR_GDD = 3, CTB_TR_BINS = 4 };
 #define CTB_MAX_OUT 4
 
 typedef struct ctb_plan ctb_plan;
