@@ -25,7 +25,8 @@ __all__ = ["Plan", "GridSpec", "TimeGroups", "get_plan", "get_time_groups", "agg
 
 _NP2CTB = {np.dtype("float32"): N.F32, np.dtype("float64"): N.F64}
 _T2CTB = {torch.float32: N.F32, torch.float64: N.F64}
-_KIND = {"identity": N.TR_IDENTITY, "poly": N.TR_POLY, "edd": N.TR_EDD, "gdd": N.TR_GDD, "bins": N.TR_BINS}
+_KIND = {"identity": N.TR_IDENTITY, "poly": N.TR_POLY, "edd": N.TR_EDD, "gdd": N.TR_GDD, "bins": N.TR_BINS,
+         "rcspline": N.TR_RCSPLINE}
 
 
 def default_device():

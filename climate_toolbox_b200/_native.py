@@ -15,7 +15,7 @@ LIB_PATH = os.environ.get("CTB_LIBRARY") or os.path.join(_HERE, "libctb.so")
 OK, ERR_LABEL_NOT_FOUND, ERR_CUDA, ERR_INVALID, ERR_UNSUPPORTED = range(5)
 F32, F64 = 0, 1
 LAYOUT_TIME_MAJOR, LAYOUT_CELL_MAJOR = 0, 1
-TR_IDENTITY, TR_POLY, TR_EDD, TR_GDD, TR_BINS = range(5)
+TR_IDENTITY, TR_POLY, TR_EDD, TR_GDD, TR_BINS, TR_RCSPLINE = range(6)
 MAX_OUT = 4
 VARIANT_AUTO, VARIANT_STAGED, VARIANT_DIRECT = 0, 1, 2
 

@@ -12,7 +12,7 @@ become index metadata here:
   time mask) does not move data; it records ``positions`` for that dim.  The
   aggregation planner folds those into CSR column indices / the time-index
   list (SURVEY.md section 3.2).
-* **deferred transforms** -- ``tas_poly`` / ``tas_bins`` / ``snyder_edd`` / ``snyder_gdd`` return
+* **deferred transforms** -- ``tas_poly`` / ``tas_bins`` / ``tas_rcspline`` / ``snyder_edd`` / ``snyder_gdd`` return
   variables that remember (kind, params, sources); aggregation fuses them into
   the gather kernel, ``.values`` materialises them with the pointwise CUDA
   kernel.
@@ -49,11 +49,11 @@ def _as_data(a):
 class Deferred:
     """A pointwise gridcell transform that has not been evaluated yet.
 
-    kind   : "poly" | "bins" | "edd" | "gdd" | "reindex" (pointwise lat/lon gather,
+    kind   : "poly" | "bins" | "rcspline" | "edd" | "gdd" | "reindex" (pointwise lat/lon gather,
              params = (materialise closure, origin Dataset))
-    params : tuple of floats (poly: (offset, power); bins: (offset, lo, hi); edd: (threshold,);
-             gdd: (threshold_low, threshold_high))
-    sources: tuple of :class:`Variable` (poly / bins: (tas,); edd/gdd: (tasmin, tasmax))
+    params : tuple of floats (poly: (offset, power); bins: (offset, lo, hi); rcspline: (offset, term,
+             k_1, ..., k_n); edd: (threshold,); gdd: (threshold_low, threshold_high))
+    sources: tuple of :class:`Variable` (poly / bins / rcspline: (tas,); edd/gdd: (tasmin, tasmax))
     """
 
     __slots__ = ("kind", "params", "sources", "shape")

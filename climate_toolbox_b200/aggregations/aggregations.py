@@ -198,7 +198,9 @@ def _group_requests(reqs):
     """Fuse requests that read the same sources: poly orders / EDD thresholds /
     GDD pairs / contiguous temperature bins become extra outputs of ONE pass over
     the data (config 3/4).  A bin (offset, lo, hi) joins a group of bins whose
-    last edge is lo: the group's params are (offset, e_0, ..., e_n)."""
+    last edge is lo: the group's params are (offset, e_0, ..., e_n).  A spline term
+    (offset, i, k_1, ..., k_n) joins a group of the same offset and knots whose
+    terms run first .. i - 1: the group keeps the params (offset, first, k_1, ..., k_n)."""
     groups = []
     for name, kind, params, srcs in reqs:
         placed = False
@@ -213,8 +215,12 @@ def _group_requests(reqs):
                 continue
             if kind == "bins" and g["params"][-1] != params[1]:
                 continue
+            if kind == "rcspline" and (g["params"][:1] + g["params"][2:] != params[:1] + params[2:] or
+                                       g["params"][1] + len(g["names"]) != params[1]):
+                continue
             g["names"].append(name)
-            g["params"] = g["params"] + (params[1:] if kind == "poly" else params[2:] if kind == "bins" else params)
+            if kind != "rcspline":
+                g["params"] = g["params"] + (params[1:] if kind == "poly" else params[2:] if kind == "bins" else params)
             placed = True
             break
         if not placed:
@@ -459,7 +465,7 @@ def weighted_aggregate_grid_to_regions(ds, variable, aggwt, agglev, weights=None
         arrays (host; copied in time chunks) or CUDA tensors (device-resident),
         in ``(time, lat, lon)`` or ``(lat, lon, time)`` order, float32/float64.
     variable : str or list of str
-        Variable(s) to aggregate.  Deferred transforms (``tas_poly``, ``tas_bins``,
+        Variable(s) to aggregate.  Deferred transforms (``tas_poly``, ``tas_bins``, ``tas_rcspline``,
         ``snyder_edd``, ``snyder_gdd``) of the same source are fused into one pass.
     aggwt, agglev : str
         Weight / region-id column names in ``weights``.

@@ -180,6 +180,7 @@ int run_kind(const ctb_plan* P, const AggArgs& a, int layout, int variant, bool 
     case CTB_TR_EDD: return run_nout<TIN, CTB_TR_EDD>(P, a, layout, variant, vec, n_out, st);
     case CTB_TR_GDD: return run_nout<TIN, CTB_TR_GDD>(P, a, layout, variant, vec, n_out, st);
     case CTB_TR_BINS: return run_nout<TIN, CTB_TR_BINS>(P, a, layout, variant, vec, n_out, st);
+    case CTB_TR_RCSPLINE: return run_nout<TIN, CTB_TR_RCSPLINE>(P, a, layout, variant, vec, n_out, st);
   }
   ctb_set_error("transform=%d unsupported", kind);
   return CTB_ERR_INVALID;
@@ -366,6 +367,56 @@ int ctb_pack_transform(int transform, const double* params, int n_params, int n_
         while (f > -INFINITY && ge(f)) f = std::nextafterf(f, -INFINITY);
         while (!ge(f)) f = std::nextafterf(f, INFINITY);
         out->up[j] = f;
+      }
+      return CTB_OK;
+    }
+    case CTB_TR_RCSPLINE: {
+      // {offset, first, k_1..k_n}: outputs B_first .. B_{first+n_out-1} of the n - 1 basis functions
+      const int n = n_params - 2;
+      if (n < 3 || n > 7 || !params) {
+        ctb_set_error("RCSPLINE takes 3..7 knots: n_params = n + 2 = 5..9, got %d", n_params);
+        return CTB_ERR_INVALID;
+      }
+      const double off = params[0], first = params[1];
+      const double* k = params + 2;   // k[0] = k_1
+      if (!std::isfinite(off)) {
+        ctb_set_error("RCSPLINE offset %g is not finite", off);
+        return CTB_ERR_INVALID;
+      }
+      for (int i = 0; i < n; ++i) {
+        if (!std::isfinite(k[i]) || (i > 0 && !(k[i] > k[i - 1]))) {
+          ctb_set_error("RCSPLINE knots must be finite and strictly increasing: knot %d is %g", i + 1, k[i]);
+          return CTB_ERR_INVALID;
+        }
+      }
+      if (first != std::floor(first) || first < 0 || first + n_out > n - 1) {
+        ctb_set_error("RCSPLINE first=%g with n_out=%d: need an integer first >= 0 and first + n_out <= %d (n - 1 "
+                      "basis functions of %d knots)", first, n_out, n - 1, n);
+        return CTB_ERR_INVALID;
+      }
+      // packed for ctb_rcs: a[0] = offset, a[1 + j] = the knot k_i of output j, i = first + j, and its
+      // b_i = (k_{n-1} - k_i) / (k_n - k_{n-1}) in the bytes of dn[2j..2j+1] (ctb_rcs_b); a[1] stays 0 when
+      // output 0 is the linear term B_0 (ip[0] = 1); a[5] = k_{n-1}, a[6] = k_n
+      const int f0 = (int)first;
+      out->a[0] = off;
+      out->ip[0] = f0 == 0;
+      out->a[5] = k[n - 2];
+      out->a[6] = k[n - 1];
+      for (int j = 0; j < n_out; ++j) {
+        if (f0 + j == 0) continue;
+        const double ki = k[f0 + j - 1], b = (k[n - 2] - ki) / (k[n - 1] - k[n - 2]);
+        out->a[1 + j] = ki;
+        std::memcpy(&out->dn[2 * j], &b, sizeof b);
+      }
+      // float inputs: up[m] = the least float f with fl64(f) - offset > a[m], so that f >= up[m] decides
+      // c(a[m]) != 0 on the stored type (NaN aside)
+      for (int m = 1; m <= 6; ++m) {
+        if (m > n_out && m < 5) continue;
+        auto gt = [&](float f) { return (double)f - off > out->a[m]; };
+        float f = (float)(out->a[m] + off);
+        while (f > -INFINITY && gt(f)) f = std::nextafterf(f, -INFINITY);
+        while (!gt(f)) f = std::nextafterf(f, INFINITY);
+        out->up[m] = f;
       }
       return CTB_OK;
     }

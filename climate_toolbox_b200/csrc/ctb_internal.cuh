@@ -7,6 +7,8 @@
 
 #include <atomic>
 #include <cstdarg>
+#include <cstddef>
+#include <cstring>
 #include <cstdio>
 #include <string>
 #include <vector>
@@ -166,6 +168,7 @@ struct CtbTr {
   // and x > e <=> x > dn(e), so the case tests of float inputs run on the fp32 pipe
   float up[8], dn[8];
 };
+static_assert(offsetof(CtbTr, dn) % 8 == 0, "ctb_rcs_b reads doubles from dn[]");
 
 // internal transform kind: CTB_TR_POLY whose orders are 1..n_out (checked on the host by the
 // launcher), so that the kernel carries one running product and no order tests (config 3)
@@ -301,10 +304,44 @@ __device__ __forceinline__ void ctb_bins_in_f32(const CtbTr& P, float x, bool (&
   for (int j = 0; j < NOUT; ++j) in[j] = ge[j] && !ge[j + 1];
 }
 
+// Restricted cubic spline terms f_j = B_{first+j}(d), d = x - offset (CTB_TR_RCSPLINE; packed by
+// ctb_pack_transform: a[1 + j] = output j's knot k_i, a[5] = k_{n-1}, a[6] = k_n, b_i of output j in
+// ctb_rcs_b(P, j), ip[0] = output 0 is B_0 = d).  With c(k) = max(d - k, 0)^3 and b_i = (k_{n-1} - k_i) / (k_n - k_{n-1}),
+//   B_i = c(k_i) - c(k_{n-1}) - b_i (c(k_{n-1}) - c(k_n)),
+// the definition with a_i = 1 + b_i: the cubes of k_{n-1} and k_n are computed once per value for every output,
+// and both differences are of non-negative terms, so the rounding stays within a few ulps of the scale
+// c(k_i) + a_i c(k_{n-1}) + b_i c(k_n) whatever the knots' magnitude.  Below k_{n-1} the result is c(k_i)
+// exactly, below k_i exactly 0.  pos(m, t) decides t = d - a[m] > 0 (NaN has to give true, t * t * t = NaN,
+// wherever a NaN can reach a kept result).
+// b_i of output j: kept in the kernel parameters, where every DFMA reads it as a constant operand (computed in
+// the loop or held in registers, the coefficients made the 2- to 4-output streaming kernels spill).  CtbTr::a is
+// full, so the four doubles sit in the bytes of dn[], which the spline does not use otherwise.
+__host__ __device__ __forceinline__ double ctb_rcs_b(const CtbTr& P, int j) {
+  double b;
+  memcpy(&b, &P.dn[2 * j], sizeof b);
+  return b;
+}
+
+template <int NOUT, typename Pos>
+__device__ __forceinline__ void ctb_rcs(const CtbTr& P, double d, Pos pos, double (&f)[NOUT]) {
+  auto c = [&](int m) {
+    const double t = d - P.a[m];
+    return pos(m, t) ? t * t * t : 0.0;
+  };
+  const double cm = c(5), dc = cm - c(6);
+#pragma unroll
+  for (int j = 0; j < NOUT; ++j) {
+    f[j] = fma(-ctb_rcs_b(P, j), dc, c(1 + j) - cm);
+  }
+  if (P.ip[0]) f[0] = d;
+}
+
 template <int KIND, int NOUT>
 __device__ __forceinline__ void ctb_apply(const CtbTr& P, double x0, double x1, double (&f)[NOUT]) {
   if constexpr (KIND == CTB_TR_IDENTITY) {
     f[0] = x0;
+  } else if constexpr (KIND == CTB_TR_RCSPLINE) {
+    ctb_rcs<NOUT>(P, x0 - P.a[0], [](int, double t) { return !(t <= 0.0); }, f);
   } else if constexpr (KIND == CTB_TR_BINS) {
     bool in[NOUT];
     ctb_bins_in<NOUT>(P, x0, in);

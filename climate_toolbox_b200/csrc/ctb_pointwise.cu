@@ -1,7 +1,8 @@
 // Pointwise helpers: materialise what the reference materialises when a caller
 // asks for it (`.values` of a transformed or reindexed variable).  Not on the
 // fused hot path, which never materialises these intermediates.
-//   ctb_transform   : transformations.py:69-89 (Snyder EDD), :139-141 (GDD), :189 (poly), temperature bins
+//   ctb_transform   : transformations.py:69-89 (Snyder EDD), :139-141 (GDD), :189 (poly), temperature bins,
+//                     restricted cubic spline terms
 //   ctb_gather_rows : aggregations.py:27 (ds.sel pointwise gather)
 #include <algorithm>
 
@@ -52,6 +53,7 @@ int tr_kind(const void* x0, const void* x1, int64_t n, const CtbTr& tr, int kind
     case CTB_TR_EDD: return tr_nout<TIN, CTB_TR_EDD>(x0, x1, n, tr, n_out, out, st);
     case CTB_TR_GDD: return tr_nout<TIN, CTB_TR_GDD>(x0, x1, n, tr, n_out, out, st);
     case CTB_TR_BINS: return tr_nout<TIN, CTB_TR_BINS>(x0, x1, n, tr, n_out, out, st);
+    case CTB_TR_RCSPLINE: return tr_nout<TIN, CTB_TR_RCSPLINE>(x0, x1, n, tr, n_out, out, st);
   }
   return CTB_ERR_INVALID;
 }

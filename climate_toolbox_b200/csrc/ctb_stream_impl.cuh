@@ -325,6 +325,16 @@ __device__ __forceinline__ bool reduce_region_widen(const CtbTr& tr, uint32_t ti
 #pragma unroll
         for (int j = 0; j < NOUT; ++j)
           if (on[g] && in[j]) acc[g][j] += w;
+      } else if constexpr (KIND == CTB_TR_RCSPLINE) {
+        // d > k decided on the stored type against the float thresholds up[] (ctb_pack_transform): fp32
+        // compares instead of fp64 ones, the same decisions for every float but NaN -- and a NaN fails the
+        // range check, so this result is then not kept
+        const float xf = __uint_as_float(bb[g]);
+        double f[NOUT];
+        ctb_rcs<NOUT>(tr, x - tr.a[0], [&](int m, double) { return xf >= tr.up[m]; }, f);
+#pragma unroll
+        for (int j = 0; j < NOUT; ++j)
+          if (on[g]) acc[g][j] = fma(w, f[j], acc[g][j]);
       } else {
         double f[NOUT];
         ctb_apply<KIND, NOUT>(tr, x, 0.0, f);
@@ -703,6 +713,12 @@ __global__ void __launch_bounds__(THREADS, 1) agg_stream_kernel(const AggArgs a)
 #ifndef CTB_BINS34_THREADS
 #define CTB_BINS34_THREADS CTB_POLY34_THREADS
 #endif
+#ifndef CTB_RCS34_THREADS
+#define CTB_RCS34_THREADS 512
+#endif
+#ifndef CTB_RCS2_THREADS
+#define CTB_RCS2_THREADS 640
+#endif
 #ifndef CTB_EDD1_THREADS
 #define CTB_EDD1_THREADS 640
 #endif
@@ -723,13 +739,18 @@ int launch(const ctb_plan* P, AggArgs a, cudaStream_t st) {
   // 4 bins: 512 / 640 / 768 threads = 1.278 / 1.233 / 1.228 ms, profiles/micro/r3_bins_cost.log -- 768 is within
   // the spread, so the bins keep the polynomial's 640)
   constexpr bool BINS = KIND == CTB_TR_BINS;
+  // restricted cubic spline terms: more temporaries per value than the polynomial (six cubes shared or not) --
+  // 3 or 4 terms spill at 640 threads (96 registers) when gated, 2 terms at 768 (80): 16 warps of 128 registers
+  // (measured, config 2 shapes with a time index, 4 terms: 384 / 512 / 640 threads = 2.078 / 1.814 / 1.809 ms,
+  // profiles/micro/r3_rcspline_cost.log), 2 terms the largest CTA without spills (not swept)
+  constexpr bool RCS = KIND == CTB_TR_RCSPLINE;
   // Snyder forms: threshold evaluations per gridcell-day -- few warps with many registers: the compiler
   // interleaves the 4 days x EVALS dependency chains of a quad inside one warp (measured, config 4:
   // 768/640/512/448/384/256 threads = 4.53/4.33/4.12/4.49/3.91/5.31 ms; consumer warps a multiple of 4;
   // EDD with 3 or 4 thresholds: 512 threads 3.00/3.92 ms per 730 days, 384 threads 3.03/4.24;
   // GDD with 2 outputs: 3.57 / 3.28)
   constexpr int EVALS = KIND == CTB_TR_GDD ? 2 * NOUT : NOUT;
-  constexpr int THREADS = NIN == 2 ? (EVALS == 1 ? CTB_EDD1_THREADS : (EVALS == 2 || KIND == CTB_TR_GDD) ? CTB_EDD2_THREADS : CTB_EDD34_THREADS) : (POLY && NOUT > 2) ? CTB_POLY34_THREADS : (BINS && NOUT > 2) ? CTB_BINS34_THREADS : ((POLY || BINS) && NOUT > 1) ? 768 : CTB_STREAM_THREADS;
+  constexpr int THREADS = NIN == 2 ? (EVALS == 1 ? CTB_EDD1_THREADS : (EVALS == 2 || KIND == CTB_TR_GDD) ? CTB_EDD2_THREADS : CTB_EDD34_THREADS) : (POLY && NOUT > 2) ? CTB_POLY34_THREADS : (BINS && NOUT > 2) ? CTB_BINS34_THREADS : (RCS && NOUT > 2) ? CTB_RCS34_THREADS : (RCS && NOUT > 1) ? CTB_RCS2_THREADS : ((POLY || BINS) && NOUT > 1) ? 768 : CTB_STREAM_THREADS;
   constexpr int S = CTB_STAGES;   // tile stages: one being reduced, up to two landing
   constexpr size_t SMEM = (size_t)S * Geo<NIN>::TILE_BYTES + 2 * CTB_META_CAP;
   static_assert(SMEM <= 227 * 1024 - 512, "shared memory budget");
@@ -793,6 +814,7 @@ int launch_kind(const ctb_plan* P, const AggArgs& a, int kind, int n_out, cudaSt
   if (kind == CTB_TR_EDD) { CTB_NOUT_SWITCH(CTB_TR_EDD) }
   if (kind == CTB_TR_GDD) { CTB_NOUT_SWITCH(CTB_TR_GDD) }
   if (kind == CTB_TR_BINS) { CTB_NOUT_SWITCH(CTB_TR_BINS) }
+  if (kind == CTB_TR_RCSPLINE) { CTB_NOUT_SWITCH(CTB_TR_RCSPLINE) }
 #undef CTB_NOUT_SWITCH
   ctb_set_error("streaming kernel: transform=%d n_out=%d unsupported", kind, n_out);
   return CTB_ERR_INVALID;

@@ -14,7 +14,8 @@ import torch
 from .._xr import DataArray, Dataset, Deferred, Variable, from_any, to_like
 from ..utils.utils import remove_leap_days, convert_kelvin_to_celsius  # noqa: F401
 
-__all__ = ["snyder_edd", "snyder_gdd", "validate_edd_snyder_agriculture", "tas_poly", "tas_bins", "ordinal"]
+__all__ = ["snyder_edd", "snyder_gdd", "validate_edd_snyder_agriculture", "tas_poly", "tas_bins", "tas_rcspline",
+           "ordinal"]
 
 
 def _source(da):
@@ -85,6 +86,26 @@ def validate_edd_snyder_agriculture(ds, thresholds):
     return
 
 
+def _daily_tas_365(ds):
+    """The shared first steps of ``tas_poly`` / ``tas_bins`` / ``tas_rcspline``: ``ds["tas"]`` without leap
+    days, and an empty Dataset with the coordinates of ``ds`` and ``time`` as ``YYYYDDD``.  Returns
+    ``(ds1, tas)``; more than 365 steps raise ``ValueError``."""
+    # remove leap years
+    ds = remove_leap_days(ds)
+    tas = _source(ds["tas"])
+
+    # Replace datetime64[ns] 'time' with YYYYDDD int 'day'
+    if ds.dims["time"] > 365:
+        raise ValueError
+    ds1 = Dataset()
+    for k, c in ds._coords.items():
+        if k != "time":
+            ds1._coords[k] = c
+    year = np.asarray(ds["time.year"].values, dtype=np.int64)
+    ds1._coords["time"] = Variable(("time",), year * 1000 + np.arange(1, len(year) + 1))
+    return ds1, tas
+
+
 def tas_poly(ds, power, varname):
     """
     Daily average temperature (degrees C), raised to a power (reference ``:160-208``).
@@ -100,19 +121,7 @@ def tas_poly(ds, power, varname):
     if len(powers) != len(names):
         raise ValueError("power and varname must have the same length")
 
-    # remove leap years
-    ds = remove_leap_days(ds)
-    tas = _source(ds["tas"])
-
-    # Replace datetime64[ns] 'time' with YYYYDDD int 'day'
-    if ds.dims["time"] > 365:
-        raise ValueError
-    ds1 = Dataset()
-    for k, c in ds._coords.items():
-        if k != "time":
-            ds1._coords[k] = c
-    year = np.asarray(ds["time.year"].values, dtype=np.int64)
-    ds1._coords["time"] = Variable(("time",), year * 1000 + np.arange(1, len(year) + 1))
+    ds1, tas = _daily_tas_365(ds)
 
     for p, name in zip(powers, names):
         powername = ordinal(p)
@@ -172,19 +181,7 @@ def tas_bins(ds, edges, varname="tas_bin"):
     like = ds
     ds = from_any(ds)
 
-    # remove leap years
-    ds = remove_leap_days(ds)
-    tas = _source(ds["tas"])
-
-    # Replace datetime64[ns] 'time' with YYYYDDD int 'day'
-    if ds.dims["time"] > 365:
-        raise ValueError
-    ds1 = Dataset()
-    for k, c in ds._coords.items():
-        if k != "time":
-            ds1._coords[k] = c
-    year = np.asarray(ds["time.year"].values, dtype=np.int64)
-    ds1._coords["time"] = Variable(("time",), year * 1000 + np.arange(1, len(year) + 1))
+    ds1, tas = _daily_tas_365(ds)
 
     for lo, hi, name in zip(e[:-1], e[1:], names):
         description = (
@@ -204,6 +201,68 @@ def tas_bins(ds, edges, varname="tas_bin"):
         # do transformation: lo <= tas - 273.15 < hi, deferred
         ds1._vars[name] = Variable(tas.dims, None, attrs, None,
                                    Deferred("bins", (273.15, float(lo), float(hi)), (tas,)))
+    return to_like(ds1, like)
+
+
+def _rcspline_knots(knots):
+    """``knots`` as a float64 array of 3 to 7 finite, strictly increasing values."""
+    k = np.asarray(knots, dtype=np.float64)
+    if k.ndim != 1 or not 3 <= k.size <= 7:
+        raise ValueError("knots must be a 1-D sequence of 3 to 7 values, got {!r}".format(knots))
+    if not np.isfinite(k).all() or not (np.diff(k) > 0).all():
+        raise ValueError("knots must be finite and strictly increasing: {!r}".format(knots))
+    return k
+
+
+def tas_rcspline(ds, knots, varname="tas_rcspline"):
+    """
+    Restricted (natural) cubic spline terms of daily average temperature (degrees C): one variable per
+    basis function of the knots ``k_1 < ... < k_n`` (3 <= n <= 7, degrees C), n - 1 in all.  With
+    ``d = tas - 273.15`` (the value widened to float64 before the subtraction) and
+    ``c(k) = max(d - k, 0)**3``::
+
+        B_0 = d                                                               (units C)
+        B_i = c(k_i) - c(k_{n-1}) (k_n - k_i) / (k_n - k_{n-1})
+                     + c(k_n) (k_{n-1} - k_i) / (k_n - k_{n-1}),   1 <= i <= n-2   (units C^3)
+
+    Each ``B_i`` is cubic between the knots and linear below ``k_1`` and above ``k_n``; NaN stays NaN, and
+    ``tas = +inf`` gives NaN for ``i >= 1``.  This is Harrell's unnormalised form: his default
+    normalisation divides ``B_i`` (i >= 1) by ``(k_n - k_1)**2``, and since aggregation is linear that
+    scale can be applied to the aggregated values.
+
+    Same conventions as :func:`tas_poly` (reads ``ds["tas"]`` in K, leap years removed, at most 365
+    steps, ``time`` as ``YYYYDDD``).  ``varname``: a prefix (variables ``"{varname}_{i}"``, ``i = 0`` the
+    linear term) or a list of n - 1 names.  The terms of one ``tas`` are fused into one pass per 4 terms
+    when aggregated, sharing the cubes of the two last knots.
+    """
+    k = _rcspline_knots(knots)
+    n = k.size
+    names = ["{}_{}".format(varname, i) for i in range(n - 1)] if isinstance(varname, str) else list(varname)
+    if len(names) != n - 1:
+        raise ValueError("{} knots give {} terms, but {} names were given".format(n, n - 1, len(names)))
+    like = ds
+    ds1, tas = _daily_tas_365(from_any(ds))
+
+    knot_list = ", ".join("{:g}".format(v) for v in k)
+    for i, name in enumerate(names):
+        description = (
+            """
+            {what} of daily average temperature (degrees C)
+
+            Restricted cubic spline basis of the knots ({knots}) degrees C,
+            unnormalised: cubic between the knots, linear outside them.
+
+            Leap years are removed before counting days (uses a 365 day
+            calendar).
+            """.format(what="Linear term" if i == 0 else "Restricted cubic spline term {}".format(i),
+                       knots=knot_list)
+        ).strip()
+        attrs = {"units": "C" if i == 0 else "C^3", "knots": [float(v) for v in k], "rcspline_term": i,
+                 "long_title": description.splitlines()[0], "description": description,
+                 "variable": name}
+        # do transformation: B_i(tas - 273.15), deferred
+        ds1._vars[name] = Variable(tas.dims, None, attrs, None,
+                                   Deferred("rcspline", (273.15, float(i)) + tuple(float(v) for v in k), (tas,)))
     return to_like(ds1, like)
 
 

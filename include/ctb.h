@@ -60,8 +60,15 @@ enum { CTB_LAYOUT_TIME_MAJOR = 0, CTB_LAYOUT_CELL_MAJOR = 1 };
  *   EDD       n_in=2  params = {e_1..e_nout}           f_j = SnyderEDD(tmin=x0,tmax=x1,e_j)  transformations.py:69-89
  *   GDD       n_in=2  params = {lo_1,hi_1,..}          f_j = EDD(lo_j) - EDD(hi_j)           transformations.py:139-141
  *   BINS      n_in=1  params = {offset, e_0..e_nout}   f_j = [e_j <= x - offset < e_{j+1}]   (NaN for NaN x; edges strictly
- *                     increasing, not NaN, only e_0 may be -inf and only e_nout +inf; n_params = n_out + 2) */
-enum { CTB_TR_IDENTITY = 0, CTB_TR_POLY = 1, CTB_TR_EDD = 2, CTB_TR_GDD = 3, CTB_TR_BINS = 4 };
+ *                     increasing, not NaN, only e_0 may be -inf and only e_nout +inf; n_params = n_out + 2)
+ *   RCSPLINE  n_in=1  params = {offset, first, k_1..k_n}   f_j = B_{first+j}(x - offset), the restricted cubic spline
+ *                     basis of the knots k (Harrell's unnormalised form), d = x - offset, c(k) = max(d - k, 0)^3:
+ *                       B_0(d) = d
+ *                       B_i(d) = c(k_i) - c(k_{n-1}) (k_n - k_i)/(k_n - k_{n-1}) + c(k_n) (k_{n-1} - k_i)/(k_n - k_{n-1})
+ *                     for 1 <= i <= n-2 (NaN propagates; +inf gives NaN for i >= 1).  3 <= n <= 7 finite, strictly
+ *                     increasing knots, a finite offset, an integer first >= 0 with first + n_out <= n - 1;
+ *                     n_params = n + 2 */
+enum { CTB_TR_IDENTITY = 0, CTB_TR_POLY = 1, CTB_TR_EDD = 2, CTB_TR_GDD = 3, CTB_TR_BINS = 4, CTB_TR_RCSPLINE = 5 };
 #define CTB_MAX_OUT 4
 
 typedef struct ctb_plan ctb_plan;
