@@ -11,14 +11,10 @@
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
-#include <type_traits>
 
 #include "ctb_internal.cuh"
 
 namespace {
-
-template <int KIND>
-struct NIn { static constexpr int v = (KIND == CTB_TR_EDD || KIND == CTB_TR_GDD) ? 2 : 1; };
 
 // one CSR entry: acc_j += w * f_j(x), NaN products skipped (skipna sum, aggregations.py:78)
 template <typename TIN, int KIND, int NOUT>
@@ -98,7 +94,7 @@ __global__ void agg_group_finish_kernel(const AggArgs a, int n_out) {
 // ---- direct kernel: warp per (region, 32-day tile) ---------------------------
 template <typename TIN, int KIND, int NOUT, int LAYOUT>
 __global__ void __launch_bounds__(256) agg_direct_kernel(const AggArgs a) {
-  constexpr int NIN = NIn<KIND>::v;
+  constexpr int NIN = ctb_tr_nin(KIND);
   const int lane = threadIdx.x & 31;
   const int n_tiles = (a.T + 31) / 32;
   const int64_t n_work = (int64_t)a.R * n_tiles;
@@ -148,42 +144,6 @@ int launch_direct(const AggArgs& a, int layout, cudaStream_t st) {
     agg_direct_kernel<TIN, KIND, NOUT, CTB_LAYOUT_TIME_MAJOR><<<grid, 256, 0, st>>>(b);
   CTB_LAUNCH_CHECK();
   return CTB_OK;
-}
-
-// variant 1 = the streaming kernel (ctb_stream_impl.cuh), 2 = direct
-template <typename TIN, int KIND, int NOUT>
-int run(const ctb_plan* P, const AggArgs& a, int layout, int variant, bool vec, cudaStream_t st) {
-  (void)vec;
-  if (variant == 2) return launch_direct<TIN, KIND, NOUT>(a, layout, st);
-  return ctb_launch_stream(P, a, std::is_same<TIN, float>::value ? CTB_F32 : CTB_F64, KIND, NOUT, st);
-}
-
-template <typename TIN, int KIND>
-int run_nout(const ctb_plan* P, const AggArgs& a, int layout, int variant, bool vec, int n_out,
-             cudaStream_t st) {
-  switch (n_out) {
-    case 1: return run<TIN, KIND, 1>(P, a, layout, variant, vec, st);
-    case 2: return run<TIN, KIND, 2>(P, a, layout, variant, vec, st);
-    case 3: return run<TIN, KIND, 3>(P, a, layout, variant, vec, st);
-    case 4: return run<TIN, KIND, 4>(P, a, layout, variant, vec, st);
-  }
-  ctb_set_error("n_out=%d unsupported", n_out);
-  return CTB_ERR_INVALID;
-}
-
-template <typename TIN>
-int run_kind(const ctb_plan* P, const AggArgs& a, int layout, int variant, bool vec, int kind,
-             int n_out, cudaStream_t st) {
-  switch (kind) {
-    case CTB_TR_IDENTITY: return run<TIN, CTB_TR_IDENTITY, 1>(P, a, layout, variant, vec, st);
-    case CTB_TR_POLY: return run_nout<TIN, CTB_TR_POLY>(P, a, layout, variant, vec, n_out, st);
-    case CTB_TR_EDD: return run_nout<TIN, CTB_TR_EDD>(P, a, layout, variant, vec, n_out, st);
-    case CTB_TR_GDD: return run_nout<TIN, CTB_TR_GDD>(P, a, layout, variant, vec, n_out, st);
-    case CTB_TR_BINS: return run_nout<TIN, CTB_TR_BINS>(P, a, layout, variant, vec, n_out, st);
-    case CTB_TR_RCSPLINE: return run_nout<TIN, CTB_TR_RCSPLINE>(P, a, layout, variant, vec, n_out, st);
-  }
-  ctb_set_error("transform=%d unsupported", kind);
-  return CTB_ERR_INVALID;
 }
 
 size_t scratch_bytes(const ctb_plan* plan, int64_t T, int n_out) {
@@ -280,8 +240,12 @@ int aggregate_impl(const ctb_plan* P, const void* x0, const void* x1, int dtype,
 #endif
   cudaStream_t st = (cudaStream_t)stream;
   if (T > 0) {
-    rc = dtype == CTB_F32 ? run_kind<float>(P, a, layout, variant, vec, transform, n_out, st)
-                          : run_kind<double>(P, a, layout, variant, vec, transform, n_out, st);
+    // variant 1 = the streaming kernel (ctb_stream_impl.cuh), 2 = direct
+    rc = variant == 1 ? ctb_launch_stream(P, a, dtype, transform, n_out, st)
+                      : ctb_dispatch_transform(transform, n_out, [&](auto kind, auto nout) {
+                          return dtype == CTB_F32 ? launch_direct<float, kind, nout>(a, layout, st)
+                                                  : launch_direct<double, kind, nout>(a, layout, st);
+                        });
     if (rc) return rc;
   }
   if (G && !flush) return CTB_OK;

@@ -11,6 +11,7 @@
 #include <cstring>
 #include <cstdio>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "ctb.h"
@@ -173,6 +174,9 @@ static_assert(offsetof(CtbTr, dn) % 8 == 0, "ctb_rcs_b reads doubles from dn[]")
 // internal transform kind: CTB_TR_POLY whose orders are 1..n_out (checked on the host by the
 // launcher), so that the kernel carries one running product and no order tests (config 3)
 constexpr int CTB_TR_POLY_SEQ = 16;
+
+// inputs a transform reads per gridcell-day: the Snyder forms take tasmin and tasmax
+__host__ __device__ constexpr int ctb_tr_nin(int kind) { return (kind == CTB_TR_EDD || kind == CTB_TR_GDD) ? 2 : 1; }
 
 __device__ __forceinline__ double ctb_ipow(double d, int p) {
   // integer power by squaring; p is warp-uniform
@@ -515,7 +519,37 @@ struct CtbDeviceGuard {
   }
 };
 
-static inline int ctb_tr_nin(int kind) { return (kind == CTB_TR_EDD || kind == CTB_TR_GDD) ? 2 : 1; }
-
 // host: validate + pack transform params. returns CTB_OK or error.
 int ctb_pack_transform(int transform, const double* params, int n_params, int n_out, CtbTr* out);
+
+// The (transform, outputs) pairs the kernels are compiled for: f(std::integral_constant<int, KIND>{},
+// std::integral_constant<int, NOUT>{}) launches the pair's instantiation.  Any other pair is an error.
+template <int KIND, typename F>
+int ctb_dispatch_nout(int n_out, F&& f) {
+  using K = std::integral_constant<int, KIND>;
+  switch (n_out) {
+    case 1: return f(K{}, std::integral_constant<int, 1>{});
+    case 2: return f(K{}, std::integral_constant<int, 2>{});
+    case 3: return f(K{}, std::integral_constant<int, 3>{});
+    case 4: return f(K{}, std::integral_constant<int, 4>{});
+  }
+  ctb_set_error("transform=%d n_out=%d unsupported", KIND, n_out);
+  return CTB_ERR_INVALID;
+}
+
+// Adding a transform kind: one case here, plus its branches in ctb_apply and ctb_pack_transform.
+template <typename F>
+int ctb_dispatch_transform(int kind, int n_out, F&& f) {
+  switch (kind) {
+    case CTB_TR_IDENTITY:
+      if (n_out != 1) break;
+      return f(std::integral_constant<int, CTB_TR_IDENTITY>{}, std::integral_constant<int, 1>{});
+    case CTB_TR_POLY: return ctb_dispatch_nout<CTB_TR_POLY>(n_out, f);
+    case CTB_TR_EDD: return ctb_dispatch_nout<CTB_TR_EDD>(n_out, f);
+    case CTB_TR_GDD: return ctb_dispatch_nout<CTB_TR_GDD>(n_out, f);
+    case CTB_TR_BINS: return ctb_dispatch_nout<CTB_TR_BINS>(n_out, f);
+    case CTB_TR_RCSPLINE: return ctb_dispatch_nout<CTB_TR_RCSPLINE>(n_out, f);
+  }
+  ctb_set_error("transform=%d n_out=%d unsupported", kind, n_out);
+  return CTB_ERR_INVALID;
+}

@@ -17,7 +17,7 @@ __global__ void transform_kernel(const TIN* __restrict__ x0, const TIN* __restri
        i += (int64_t)gridDim.x * blockDim.x) {
     const double a = (double)x0[i];
     double b = 0.0;
-    if constexpr (KIND == CTB_TR_EDD || KIND == CTB_TR_GDD) b = (double)x1[i];
+    if constexpr (ctb_tr_nin(KIND) == 2) b = (double)x1[i];
     double f[NOUT];
     ctb_apply<KIND, NOUT>(tr, a, b, f);
 #pragma unroll
@@ -31,31 +31,6 @@ int launch_tr(const void* x0, const void* x1, int64_t n, const CtbTr& tr, double
   transform_kernel<TIN, KIND, NOUT><<<grid, 256, 0, st>>>((const TIN*)x0, (const TIN*)x1, n, tr, out);
   CTB_LAUNCH_CHECK();
   return CTB_OK;
-}
-
-template <typename TIN, int KIND>
-int tr_nout(const void* x0, const void* x1, int64_t n, const CtbTr& tr, int n_out, double* out, cudaStream_t st) {
-  switch (n_out) {
-    case 1: return launch_tr<TIN, KIND, 1>(x0, x1, n, tr, out, st);
-    case 2: return launch_tr<TIN, KIND, 2>(x0, x1, n, tr, out, st);
-    case 3: return launch_tr<TIN, KIND, 3>(x0, x1, n, tr, out, st);
-    case 4: return launch_tr<TIN, KIND, 4>(x0, x1, n, tr, out, st);
-  }
-  return CTB_ERR_INVALID;
-}
-
-template <typename TIN>
-int tr_kind(const void* x0, const void* x1, int64_t n, const CtbTr& tr, int kind, int n_out, double* out,
-            cudaStream_t st) {
-  switch (kind) {
-    case CTB_TR_IDENTITY: return launch_tr<TIN, CTB_TR_IDENTITY, 1>(x0, x1, n, tr, out, st);
-    case CTB_TR_POLY: return tr_nout<TIN, CTB_TR_POLY>(x0, x1, n, tr, n_out, out, st);
-    case CTB_TR_EDD: return tr_nout<TIN, CTB_TR_EDD>(x0, x1, n, tr, n_out, out, st);
-    case CTB_TR_GDD: return tr_nout<TIN, CTB_TR_GDD>(x0, x1, n, tr, n_out, out, st);
-    case CTB_TR_BINS: return tr_nout<TIN, CTB_TR_BINS>(x0, x1, n, tr, n_out, out, st);
-    case CTB_TR_RCSPLINE: return tr_nout<TIN, CTB_TR_RCSPLINE>(x0, x1, n, tr, n_out, out, st);
-  }
-  return CTB_ERR_INVALID;
 }
 
 template <typename TIN, int LAYOUT>
@@ -74,6 +49,17 @@ __global__ void gather_rows_kernel(const TIN* __restrict__ x, int64_t stride,
   }
 }
 
+template <typename TIN>
+int launch_gather(const ctb_plan* P, const void* x, int layout, int64_t stride, const int32_t* tix, int64_t T,
+                  void* out, cudaStream_t st) {
+  const unsigned grid = (unsigned)std::min<int64_t>((P->n_rows * T + 255) / 256, 148 * 32);
+  auto k = layout == CTB_LAYOUT_TIME_MAJOR ? gather_rows_kernel<TIN, CTB_LAYOUT_TIME_MAJOR>
+                                           : gather_rows_kernel<TIN, CTB_LAYOUT_CELL_MAJOR>;
+  k<<<grid, 256, 0, st>>>((const TIN*)x, stride, P->d_row_cell, P->n_rows, tix, T, (TIN*)out);
+  CTB_LAUNCH_CHECK();
+  return CTB_OK;
+}
+
 }  // namespace
 
 extern "C" int ctb_transform(const void* x0, const void* x1, int dtype, int64_t n, int transform,
@@ -86,28 +72,22 @@ extern "C" int ctb_transform(const void* x0, const void* x1, int dtype, int64_t 
   if (ctb_tr_nin(transform) == 2 && !x1) { ctb_set_error("transform needs two inputs"); return CTB_ERR_INVALID; }
   if (n == 0) return CTB_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  return dtype == CTB_F32 ? tr_kind<float>(x0, x1, n, tr, transform, n_out, out, st)
-                          : tr_kind<double>(x0, x1, n, tr, transform, n_out, out, st);
+  return ctb_dispatch_transform(transform, n_out, [&](auto kind, auto nout) {
+    return dtype == CTB_F32 ? launch_tr<float, kind, nout>(x0, x1, n, tr, out, st)
+                            : launch_tr<double, kind, nout>(x0, x1, n, tr, out, st);
+  });
 }
 
 extern "C" int ctb_gather_rows(const ctb_plan* P, const void* x, int dtype, int layout, int64_t stride,
                                const int32_t* time_index, int64_t T, void* out, void* stream) {
   if (!P || !x || (!out && T > 0 && P->n_rows > 0) || T < 0) { ctb_set_error("ctb_gather_rows: bad argument"); return CTB_ERR_INVALID; }
   if (dtype != CTB_F32 && dtype != CTB_F64) { ctb_set_error("dtype=%d unsupported", dtype); return CTB_ERR_INVALID; }
-  const int64_t total = P->n_rows * T;
-  if (total == 0) return CTB_OK;
-  int prev = 0;
-  CTB_CUDA(cudaGetDevice(&prev));
-  if (prev != P->device) CTB_CUDA(cudaSetDevice(P->device));
-  const unsigned grid = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 32);
+  if (P->n_rows * T == 0) return CTB_OK;
+  CtbDeviceGuard guard(P->device);
+  CTB_CUDA(guard.err);
   cudaStream_t st = (cudaStream_t)stream;
-#define CTB_G(TIN, L) gather_rows_kernel<TIN, L><<<grid, 256, 0, st>>>((const TIN*)x, stride, P->d_row_cell, P->n_rows, time_index, T, (TIN*)out)
-  if (dtype == CTB_F32) { if (layout == CTB_LAYOUT_TIME_MAJOR) CTB_G(float, CTB_LAYOUT_TIME_MAJOR); else CTB_G(float, CTB_LAYOUT_CELL_MAJOR); }
-  else { if (layout == CTB_LAYOUT_TIME_MAJOR) CTB_G(double, CTB_LAYOUT_TIME_MAJOR); else CTB_G(double, CTB_LAYOUT_CELL_MAJOR); }
-#undef CTB_G
-  CTB_LAUNCH_CHECK();
-  if (prev != P->device) cudaSetDevice(prev);
-  return CTB_OK;
+  return dtype == CTB_F32 ? launch_gather<float>(P, x, layout, stride, time_index, T, out, st)
+                          : launch_gather<double>(P, x, layout, stride, time_index, T, out, st);
 }
 
 // Rows of a pitched DEVICE array to a pitched HOST array on `stream` (one DMA): the time-chunked

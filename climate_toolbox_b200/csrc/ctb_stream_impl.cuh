@@ -72,8 +72,6 @@ struct Geo {
   static constexpr int TILE_BYTES = NIN * IN_BYTES;   // 66,048 / 66,560 bytes per stage
   static constexpr int GROUPS_IN = UNITS / 8;         // groups of 8 units per input
 };
-template <int KIND>
-struct NIn { static constexpr int v = (KIND == CTB_TR_EDD || KIND == CTB_TR_GDD) ? 2 : 1; };
 enum { F_SLOT = 1, F_FIRST = 2, F_LAST = 4, F_EXIT = 8 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
@@ -411,7 +409,7 @@ __device__ __forceinline__ void reduce_region2(const CtbTr& tr, uint32_t tile_a,
 // and carrying both costs the plain one 2 %)
 template <typename TIN, int KIND, int NOUT, int THREADS, int S, bool GATE, bool TIX>
 __global__ void __launch_bounds__(THREADS, 1) agg_stream_kernel(const AggArgs a) {
-  constexpr int NIN = NIn<KIND>::v;
+  constexpr int NIN = ctb_tr_nin(KIND);
   using G = Geo<NIN>;
   constexpr int CTB_ROWB = G::ROWB, CTB_STREAM_TILE_BYTES = G::TILE_BYTES;
   constexpr int NWARP = THREADS / 32;
@@ -728,29 +726,43 @@ __global__ void __launch_bounds__(THREADS, 1) agg_stream_kernel(const AggArgs a)
 #ifndef CTB_EDD34_THREADS
 #define CTB_EDD34_THREADS 512
 #endif
+// CTA size of the streaming kernel, one branch per transform family
+constexpr int stream_threads(int kind, int nout) {
+  if (kind == CTB_TR_POLY || kind == CTB_TR_POLY_SEQ) {
+    // three and four polynomial outputs keep 4 fp64 accumulators per output and lane: 20 warps of 96
+    return nout > 2 ? CTB_POLY34_THREADS : nout > 1 ? 768 : CTB_STREAM_THREADS;
+  }
+  if (kind == CTB_TR_BINS) {
+    // temperature bins: the polynomial shapes (the same 4 x NOUT accumulators per lane; measured, config 2
+    // shapes, 4 bins: 512 / 640 / 768 threads = 1.278 / 1.233 / 1.228 ms, profiles/micro/r3_bins_cost.log --
+    // 768 is within the spread, so the bins keep the polynomial's 640)
+    return nout > 2 ? CTB_BINS34_THREADS : nout > 1 ? 768 : CTB_STREAM_THREADS;
+  }
+  if (kind == CTB_TR_RCSPLINE) {
+    // restricted cubic spline terms: more temporaries per value than the polynomial (six cubes shared or
+    // not) -- 3 or 4 terms spill at 640 threads (96 registers) when gated, 2 terms at 768 (80): 16 warps of
+    // 128 registers (measured, config 2 shapes with a time index, 4 terms: 384 / 512 / 640 threads = 2.078 /
+    // 1.814 / 1.809 ms, profiles/micro/r3_rcspline_cost.log), 2 terms the largest CTA without spills (not swept)
+    return nout > 2 ? CTB_RCS34_THREADS : nout > 1 ? CTB_RCS2_THREADS : CTB_STREAM_THREADS;
+  }
+  if (kind == CTB_TR_EDD || kind == CTB_TR_GDD) {
+    // Snyder forms: threshold evaluations per gridcell-day -- few warps with many registers: the compiler
+    // interleaves the 4 days x evals dependency chains of a quad inside one warp (measured, config 4:
+    // 768/640/512/448/384/256 threads = 4.53/4.33/4.12/4.49/3.91/5.31 ms; consumer warps a multiple of 4;
+    // EDD with 3 or 4 thresholds: 512 threads 3.00/3.92 ms per 730 days, 384 threads 3.03/4.24;
+    // GDD with 2 outputs: 3.57 / 3.28)
+    if (kind == CTB_TR_GDD) return CTB_EDD2_THREADS;
+    return nout == 1 ? CTB_EDD1_THREADS : nout == 2 ? CTB_EDD2_THREADS : CTB_EDD34_THREADS;
+  }
+  // 24 warps of 80 registers (measured, config 2: 1024 / 896 / 768 / 640 / 512 threads = 0.619 / 0.609 /
+  // 0.599 / 0.611 / 0.672 ms; the reduction alone is fastest with 32 warps, the whole kernel with 24)
+  return CTB_STREAM_THREADS;
+}
+
 template <typename TIN, int KIND, int NOUT>
 int launch(const ctb_plan* P, AggArgs a, cudaStream_t st) {
-  // 24 warps of 80 registers (measured, config 2: 1024 / 896 / 768 / 640 / 512 threads = 0.619 / 0.609 /
-  // 0.599 / 0.611 / 0.672 ms; the reduction alone is fastest with 32 warps, the whole kernel with 24);
-  // three and four polynomial outputs keep 4 fp64 accumulators per output and lane: 20 warps of 96
-  constexpr int NIN = NIn<KIND>::v;
-  constexpr bool POLY = KIND == CTB_TR_POLY || KIND == CTB_TR_POLY_SEQ;
-  // temperature bins: the polynomial shapes (the same 4 x NOUT accumulators per lane; measured, config 2 shapes,
-  // 4 bins: 512 / 640 / 768 threads = 1.278 / 1.233 / 1.228 ms, profiles/micro/r3_bins_cost.log -- 768 is within
-  // the spread, so the bins keep the polynomial's 640)
-  constexpr bool BINS = KIND == CTB_TR_BINS;
-  // restricted cubic spline terms: more temporaries per value than the polynomial (six cubes shared or not) --
-  // 3 or 4 terms spill at 640 threads (96 registers) when gated, 2 terms at 768 (80): 16 warps of 128 registers
-  // (measured, config 2 shapes with a time index, 4 terms: 384 / 512 / 640 threads = 2.078 / 1.814 / 1.809 ms,
-  // profiles/micro/r3_rcspline_cost.log), 2 terms the largest CTA without spills (not swept)
-  constexpr bool RCS = KIND == CTB_TR_RCSPLINE;
-  // Snyder forms: threshold evaluations per gridcell-day -- few warps with many registers: the compiler
-  // interleaves the 4 days x EVALS dependency chains of a quad inside one warp (measured, config 4:
-  // 768/640/512/448/384/256 threads = 4.53/4.33/4.12/4.49/3.91/5.31 ms; consumer warps a multiple of 4;
-  // EDD with 3 or 4 thresholds: 512 threads 3.00/3.92 ms per 730 days, 384 threads 3.03/4.24;
-  // GDD with 2 outputs: 3.57 / 3.28)
-  constexpr int EVALS = KIND == CTB_TR_GDD ? 2 * NOUT : NOUT;
-  constexpr int THREADS = NIN == 2 ? (EVALS == 1 ? CTB_EDD1_THREADS : (EVALS == 2 || KIND == CTB_TR_GDD) ? CTB_EDD2_THREADS : CTB_EDD34_THREADS) : (POLY && NOUT > 2) ? CTB_POLY34_THREADS : (BINS && NOUT > 2) ? CTB_BINS34_THREADS : (RCS && NOUT > 2) ? CTB_RCS34_THREADS : (RCS && NOUT > 1) ? CTB_RCS2_THREADS : ((POLY || BINS) && NOUT > 1) ? 768 : CTB_STREAM_THREADS;
+  constexpr int NIN = ctb_tr_nin(KIND);
+  constexpr int THREADS = stream_threads(KIND, NOUT);
   constexpr int S = CTB_STAGES;   // tile stages: one being reduced, up to two landing
   constexpr size_t SMEM = (size_t)S * Geo<NIN>::TILE_BYTES + 2 * CTB_META_CAP;
   static_assert(SMEM <= 227 * 1024 - 512, "shared memory budget");
@@ -795,35 +807,16 @@ int launch(const ctb_plan* P, AggArgs a, cudaStream_t st) {
   return CTB_OK;
 }
 
-template <typename TIN>
-int launch_kind(const ctb_plan* P, const AggArgs& a, int kind, int n_out, cudaStream_t st) {
-  if (kind == CTB_TR_IDENTITY) return launch<TIN, CTB_TR_IDENTITY, 1>(P, a, st);
-#define CTB_NOUT_SWITCH(K)                                   \
-  switch (n_out) {                                           \
-    case 1: return launch<TIN, K, 1>(P, a, st);              \
-    case 2: return launch<TIN, K, 2>(P, a, st);              \
-    case 3: return launch<TIN, K, 3>(P, a, st);              \
-    case 4: return launch<TIN, K, 4>(P, a, st);              \
-  }
-  if (kind == CTB_TR_POLY) {
-    bool seq = true;   // orders 1..n_out (tas_poly's usual call): no order tests in the kernel
-    for (int j = 0; j < n_out; ++j) seq = seq && a.tr.ip[j] == j + 1;
-    if (seq) { CTB_NOUT_SWITCH(CTB_TR_POLY_SEQ) }
-    CTB_NOUT_SWITCH(CTB_TR_POLY)
-  }
-  if (kind == CTB_TR_EDD) { CTB_NOUT_SWITCH(CTB_TR_EDD) }
-  if (kind == CTB_TR_GDD) { CTB_NOUT_SWITCH(CTB_TR_GDD) }
-  if (kind == CTB_TR_BINS) { CTB_NOUT_SWITCH(CTB_TR_BINS) }
-  if (kind == CTB_TR_RCSPLINE) { CTB_NOUT_SWITCH(CTB_TR_RCSPLINE) }
-#undef CTB_NOUT_SWITCH
-  ctb_set_error("streaming kernel: transform=%d n_out=%d unsupported", kind, n_out);
-  return CTB_ERR_INVALID;
-}
-
 }  // namespace
 
 // One translation unit per input type (ctb_stream_f32.cu / ctb_stream_f64.cu: they compile in parallel; the
 // instantiations of one type take about a minute and a half).
 int CTB_STREAM_ENTRY(const ctb_plan* P, const AggArgs& a, int kind, int n_out, cudaStream_t st) {
-  return launch_kind<CTB_STREAM_TIN>(P, a, kind, n_out, st);
+  auto go = [&](auto k, auto nout) { return launch<CTB_STREAM_TIN, k, nout>(P, a, st); };
+  if (kind == CTB_TR_POLY) {
+    bool seq = true;   // orders 1..n_out (tas_poly's usual call): no order tests in the kernel
+    for (int j = 0; j < n_out; ++j) seq = seq && a.tr.ip[j] == j + 1;
+    if (seq) return ctb_dispatch_nout<CTB_TR_POLY_SEQ>(n_out, go);
+  }
+  return ctb_dispatch_transform(kind, n_out, go);
 }

@@ -56,6 +56,49 @@ def test_invalid_calls_fail_cleanly_without_gpu(built):
     assert built.ctb_push_rows(None, 10, 0, 0, 1, 1, None, 0, None) == 0          # nothing to copy
 
 
+# (transform, params, n_out, error text): pairs no kernel is compiled for
+UNSUPPORTED_PAIRS = [(9, [0.0], 1, "transform=9"),
+                     (_native.TR_POLY, [0.0, 1, 2, 3, 4, 5], 5, "n_out=5"),
+                     (_native.TR_IDENTITY, [], 2, "n_out=1")]
+
+
+def _params(params):
+    return (ctypes.c_double * max(len(params), 1))(*params), len(params)
+
+
+def test_transform_rejects_unsupported_pairs_without_gpu(built):
+    dummy = ctypes.c_double(0.0)
+    for kind, params, n_out, text in UNSUPPORTED_PAIRS:
+        p, n_p = _params(params)
+        # n = 0: the call validates its arguments and returns before any CUDA call
+        rc = built.ctb_transform(ctypes.addressof(dummy), ctypes.addressof(dummy), _native.F64, 0, kind, p, n_p,
+                                 n_out, None, None)
+        assert rc == _native.ERR_INVALID and text in _native.last_error(), (kind, n_out, _native.last_error())
+
+
+@pytest.mark.gpu
+def test_aggregate_rejects_unsupported_pairs(built):
+    import torch
+    from climate_toolbox_b200 import _engine as E
+    from climate_toolbox_b200 import synthetic
+
+    lat, lon = synthetic.grid_labels(1.0)
+    plan = E.get_plan(E.GridSpec(lat, lon), synthetic.weights_table(1.0, 20, seed=5), "popwt", "hierid",
+                      device=torch.device("cuda", 0), cache=False)
+    T, ncell = 32, len(lat) * len(lon)
+    x = torch.zeros((T, ncell), dtype=torch.float32, device="cuda:0")
+    out = torch.zeros((_native.MAX_OUT + 1, plan.R, T), dtype=torch.float64, device="cuda:0")
+    for variant in (_native.VARIANT_STAGED, _native.VARIANT_DIRECT):
+        for kind, params, n_out, text in UNSUPPORTED_PAIRS:
+            p, n_p = _params(params)
+            rc = built.ctb_aggregate_ex(plan._h, x.data_ptr(), x.data_ptr(), _native.F32, _native.LAYOUT_TIME_MAJOR,
+                                        ncell, None, T, kind, p, n_p, n_out, None, out.data_ptr(), 0, None, 0, variant,
+                                        None)
+            assert rc == _native.ERR_INVALID and text in _native.last_error(), (variant, kind, n_out)
+    torch.cuda.synchronize()
+    assert not out.any()
+
+
 def test_missing_library_fails_loudly(monkeypatch):
     monkeypatch.setattr(_native, "_lib", None)
     monkeypatch.setattr(_native, "LIB_PATH", "/nonexistent/libctb.so")

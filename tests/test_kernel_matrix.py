@@ -111,7 +111,7 @@ def _public(kind):
 
 
 def _stream_kind(kind, params, n_out):
-    """The kind of the streaming instantiation ``launch_kind`` picks: POLY with orders 1..n is POLY_SEQ."""
+    """The kind of the streaming instantiation ``CTB_STREAM_ENTRY`` picks: POLY with orders 1..n is POLY_SEQ."""
     if kind in ("poly", "poly_seq") and tuple(params[1:]) == tuple(float(p) for p in range(1, n_out + 1)):
         return POLY_SEQ
     return _CODE[_public(kind)]
