@@ -21,7 +21,7 @@ import torch
 from . import _native as N
 
 __all__ = ["Plan", "GridSpec", "TimeGroups", "get_plan", "get_time_groups", "aggregate_device", "aggregate_host",
-           "materialize_deferred", "default_device", "launch_count"]
+           "aggregate_daily", "DailySource", "materialize_deferred", "default_device", "launch_count"]
 
 _NP2CTB = {np.dtype("float32"): N.F32, np.dtype("float64"): N.F64}
 _T2CTB = {torch.float32: N.F32, torch.float64: N.F64}
@@ -494,36 +494,28 @@ def pack_threads():
     return max(1, (3 * ncpu) // 4)
 
 
-def _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, groups, out, host_out=None,
-                    chunk_bytes=4 << 30, doy=None):
-    """Pinned host arrays + compact plan: the GPU packs for itself (``ctb_pull_pack`` reads the
-    referenced pieces over PCIe into a packed device buffer), then the kernel aggregates the packed
-    planes.  No host core touches the data; pulls and kernels queue on one stream.  With ``host_out``
-    (a pinned [n_out, R, T] tensor) the result goes back in time chunks on a second stream while the
-    next chunk is pulled (PCIe is full duplex); the caller then only has to synchronise."""
+def _aggregate_packed(plan, pack, n_planes, itemsize, T, kind, params, n_out, variant, groups, out, host_out=None,
+                      chunk_bytes=4 << 30, doy=None):
+    """Compact plan whose inputs the GPU packs itself: ``pack(t0, n, bufs)`` queues on the current stream
+    what fills ``bufs`` (``n_planes`` device tensors [n, n_packed_cells] of ``itemsize``-byte elements) with
+    days t0 .. t0 + n - 1, then the kernel aggregates the packed planes.  Packs and kernels queue on one
+    stream.  With ``host_out`` (a pinned [n_out, R, T] tensor) the result goes back in time chunks on a
+    second stream while the next chunk is packed (PCIe is full duplex); the caller then only has to
+    synchronise.  Returns ``(out, host_out filled)``."""
     dev = plan.device
-    itemsize = xs[0].dtype.itemsize
     width = plan.info["n_packed_cells"]
     tdt = torch.float32 if itemsize == 4 else torch.float64
-    days = max(32, int(chunk_bytes // max(width * itemsize * len(xs), 1)) // 32 * 32)
+    days = max(32, int(chunk_bytes // max(width * itemsize * n_planes, 1)) // 32 * 32)
     if host_out is not None and groups is None:
         days = min(days, max(32, (-(-T // 4) + 31) // 32 * 32))      # about four chunks: the last D2H is exposed
-    tix_d = plan.time_index_device(tix)
     ws = _workspace(plan, min(days, T), n_out, N.LAYOUT_TIME_MAJOR, variant, groups, None)
     starts = list(range(0, T, days))
     main = torch.cuda.current_stream(dev)
     back = torch.cuda.Stream(dev) if host_out is not None and groups is None else None
     for t0 in starts:
         n = min(T, t0 + days) - t0
-        bufs = []
-        for x in xs:
-            b = torch.empty((n, width), dtype=tdt, device=dev)
-            N.check(N.lib().ctb_pull_pack(
-                plan._h, C.c_void_p(x.ctypes.data), _NP2CTB[x.dtype], int(stride),
-                C.c_void_p(tix_d.data_ptr()) if tix_d is not None else None, int(t0), int(n),
-                C.c_void_p(b.data_ptr()), _stream_ptr(dev)))
-            bufs.append(b)
-        TRANSFER_BYTES["h2d"] += len(xs) * n * plan.info["n_pieces_distinct"] * 4 * itemsize
+        bufs = [torch.empty((n, width), dtype=tdt, device=dev) for _ in range(n_planes)]
+        pack(t0, n, bufs)
         if groups is None:
             aggregate_device(plan, bufs[0], bufs[1] if len(bufs) > 1 else None, N.LAYOUT_TIME_MAJOR, width, None,
                              n, kind, params, n_out, variant, out=_OffsetOut(out, t0), out_ld=T, workspace=ws,
@@ -545,6 +537,199 @@ def _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, grou
         main.wait_stream(back)
         return out, True
     return out, False
+
+
+def _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, groups, out, host_out=None,
+                    chunk_bytes=4 << 30, doy=None):
+    """Pinned host arrays + compact plan: the GPU packs for itself (``ctb_pull_pack`` reads the
+    referenced pieces over PCIe into a packed device buffer), then the kernel aggregates the packed
+    planes.  No host core touches the data (:func:`_aggregate_packed`)."""
+    dev = plan.device
+    itemsize = xs[0].dtype.itemsize
+    tix_d = plan.time_index_device(tix)
+
+    def pack(t0, n, bufs):
+        for x, b in zip(xs, bufs):
+            N.check(N.lib().ctb_pull_pack(
+                plan._h, C.c_void_p(x.ctypes.data), _NP2CTB[x.dtype], int(stride),
+                C.c_void_p(tix_d.data_ptr()) if tix_d is not None else None, int(t0), int(n),
+                C.c_void_p(b.data_ptr()), _stream_ptr(dev)))
+        TRANSFER_BYTES["h2d"] += len(xs) * n * plan.info["n_pieces_distinct"] * 4 * itemsize
+
+    return _aggregate_packed(plan, pack, len(xs), itemsize, T, kind, params, n_out, variant, groups, out, host_out,
+                             chunk_bytes, doy)
+
+
+# ---------------------------------------------------------------------------
+# sub-daily sources: daily mean / min / max reduced while the referenced pieces are packed
+# ---------------------------------------------------------------------------
+_DAILY_OP = {"mean": N.DAILY_MEAN, "min": N.DAILY_MIN, "max": N.DAILY_MAX}
+DAILY_STAGE_BYTES = 256 << 20    # pinned staging slot of a pageable sub-daily source
+
+
+class DailySource:
+    """What ``ctb_pull_pack_daily`` reads for one deferred daily variable (``utils.resample_daily``): the
+    sub-daily source as 2-D [t_phys, ncell], its steps per day, its first step and the physical day of
+    every day."""
+
+    def __init__(self, var):
+        d = var.deferred
+        self.how, self.S, self.t0, self.day = d.params
+        src = d.sources[0]
+        self.phys = x = src.physical
+        if isinstance(x, torch.Tensor) and not x.is_cuda:
+            x = x.numpy()
+        if isinstance(x, torch.Tensor):
+            x = (x if x.dtype in _T2CTB else x.to(torch.float64)).contiguous()
+            self.dtype = _T2CTB[x.dtype]
+            self.pinned = False
+        else:
+            x = np.ascontiguousarray(x if x.dtype in _NP2CTB else x.astype(np.float64))
+            self.dtype = _NP2CTB[x.dtype]
+            self.pinned = _all_pinned([x])
+        self.on_device = isinstance(x, torch.Tensor)
+        self.nlat_phys, self.nlon_phys = int(x.shape[1]), int(x.shape[2])
+        self.stride = self.nlat_phys * self.nlon_phys
+        self.x = x.reshape(x.shape[0], self.stride)
+        self.itemsize = 4 if self.dtype == N.F32 else 8
+        self.lat_phys, self.lon_phys = src.takes.get("lat"), src.takes.get("lon")
+        self.T = len(self.day)
+
+    def ptr(self):
+        base = self.x.data_ptr() if self.on_device else self.x.ctypes.data
+        return base + self.t0 * self.stride * self.itemsize
+
+    def same_read(self, other):
+        """Both read the same steps of the same buffer."""
+        return (self.phys is other.phys and (self.S, self.t0) == (other.S, other.t0) and
+                np.array_equal(self.day, other.day))
+
+
+def _day_arg(plan, day):
+    """Device day index for the kernel, or None when day d is physical day d."""
+    if np.array_equal(day, np.arange(len(day))):
+        return None
+    return plan.time_index_device(np.asarray(day))
+
+
+def _pull_daily(plan, src, dsts, d0, n):
+    """Queue ``ctb_pull_pack_daily`` for days d0 .. d0 + n - 1 of ``src`` into ``dsts`` ({how: device tensor
+    [>= n, n_packed_cells]}, all from one read).  A pageable host source is staged first: whole days are
+    copied into pinned buffers (those of the host path, two in turn) that the kernel then reads."""
+    dev = plan.device
+    L = N.lib()
+    ops = 0
+    for how in dsts:
+        ops |= _DAILY_OP[how]
+
+    def call(x_ptr, day, t_begin, k, m):
+        day_d = _day_arg(plan, day) if day is not None else None
+        ptrs = {h: C.c_void_p(t.data_ptr() + k * t.shape[1] * t.element_size()) for h, t in dsts.items()}
+        N.check(L.ctb_pull_pack_daily(
+            plan._h, C.c_void_p(x_ptr), src.dtype, int(src.stride), int(src.S),
+            C.c_void_p(day_d.data_ptr()) if day_d is not None else None, int(t_begin), int(m), ops,
+            ptrs.get("mean"), ptrs.get("min"), ptrs.get("max"), _stream_ptr(dev)))
+        if not src.on_device:
+            TRANSFER_BYTES["h2d"] += m * src.S * plan.info["n_pieces_distinct"] * 4 * src.itemsize
+
+    if n == 0:
+        return
+    if src.on_device or src.pinned:
+        call(src.ptr(), src.day, d0, 0, n)
+        return
+    day = src.day[d0: d0 + n]
+    per_day = src.S * src.stride * src.itemsize
+    cap = max(1, DAILY_STAGE_BYTES // per_day)
+    np_dt = np.float32 if src.itemsize == 4 else np.float64
+    main = torch.cuda.current_stream(dev)
+    k, slot = 0, 0
+    with _HOST_LOCK:
+        while k < n:
+            lo = hi = int(day[k])
+            m = 1
+            while k + m < n and lo <= day[k + m] < lo + cap:
+                hi = max(hi, int(day[k + m]))
+                m += 1
+            ent = _pinned_buffer((dev.index or 0, "daily", slot), cap * per_day)   # waits for its last reader
+            stage = ent[0][: (hi + 1 - lo) * per_day].numpy().view(np_dt).reshape(-1, src.stride)
+            first = src.t0 + lo * src.S
+            np.copyto(stage, src.x[first: first + (hi + 1 - lo) * src.S])
+            call(ent[0].data_ptr(), day[k: k + m] - lo, 0, k, m)
+            ev = torch.cuda.Event()
+            ev.record(main)
+            ent[1] = ev
+            k += m
+            slot ^= 1
+
+
+def aggregate_daily(plan, srcs, kind="identity", params=(), n_out=1, variant=N.VARIANT_AUTO, groups=None,
+                    host_out=None, doy=None):
+    """Deferred daily reductions of sub-daily data -> CUDA tensor [n_out, R, T] (with ``groups``:
+    [n_out, R, n_groups]).  ``srcs``: 1 or 2 (:class:`DailySource`, how).  Each chunk of days is
+    reduce-packed by ``ctb_pull_pack_daily`` into packed daily planes (float64 for the mean, the source
+    dtype for min / max; the plan is built for that element size) and aggregated by the compact-plan
+    launch; sources that read the same steps -- the daily minimum and maximum of one variable -- come from
+    one call.  ``host_out``: as :func:`aggregate_host`."""
+    dev = plan.device
+    T = srcs[0][0].T
+    out = torch.empty((n_out, plan.R, T if groups is None else groups.n_groups), dtype=torch.float64, device=dev)
+    if T == 0 or plan.R == 0:
+        return out.zero_() if groups is not None else out
+    calls = []          # [(DailySource, {how: plane index})]
+    for i, (src, how) in enumerate(srcs):
+        for c in calls:
+            if c[0].same_read(src) and how not in c[1]:
+                c[1][how] = i
+                break
+        else:
+            calls.append((src, {how: i}))
+
+    def pack(t0, n, bufs):
+        for src, planes in calls:
+            _pull_daily(plan, src, {h: bufs[i] for h, i in planes.items()}, t0, n)
+
+    itemsize = 8 if srcs[0][1] == "mean" else srcs[0][0].itemsize
+    out, filled = _aggregate_packed(plan, pack, len(srcs), itemsize, T, kind, params, n_out, variant, groups, out,
+                                    host_out[0] if host_out is not None else None, doy=doy)
+    if host_out is not None:
+        host_out[1] = filled
+    return out
+
+
+_FULL_GRID = {}
+
+
+def _full_grid_plan(nlat, nlon, elem_bytes, dev):
+    """Compact plan that references every gridcell of an nlat x nlon grid once: its packed planes are the
+    physical planes (one run from piece 0)."""
+    hit = _FULL_GRID.get((nlat, nlon))
+    if hit is None:
+        ii, jj = np.meshgrid(np.arange(nlat, dtype=np.float64), np.arange(nlon, dtype=np.float64), indexing="ij")
+        df = pd.DataFrame({"lat": ii.ravel(), "lon": jj.ravel(), "_r": np.zeros(ii.size, dtype=np.int32),
+                           "_w": np.ones(ii.size)})
+        grid = GridSpec(np.arange(nlat, dtype=np.float64), np.arange(nlon, dtype=np.float64))
+        if len(_FULL_GRID) > 8:
+            _FULL_GRID.clear()
+        hit = _FULL_GRID[(nlat, nlon)] = (grid, df)
+    grid, df = hit
+    return get_plan(grid, df, "_w", "_r", "_w", stage_bytes=elem_bytes, device=dev, compact=True,
+                    elem_bytes=elem_bytes, trusted=True)
+
+
+def daily_device(var, dev):
+    """A deferred daily variable evaluated for the whole grid by ``ctb_pull_pack_daily``: CUDA tensor
+    [days, lat, lon] with the variable's lat / lon takes applied."""
+    src = DailySource(var)
+    es = 8 if src.how == "mean" else src.itemsize
+    plan = _full_grid_plan(src.nlat_phys, src.nlon_phys, es, dev)
+    o = torch.empty((src.T, plan.info["n_packed_cells"]), dtype=torch.float32 if es == 4 else torch.float64,
+                    device=dev)
+    _pull_daily(plan, src, {src.how: o}, 0, src.T)
+    t = o[:, : src.stride].reshape(src.T, src.nlat_phys, src.nlon_phys)
+    for ax, pos in ((1, src.lat_phys), (2, src.lon_phys)):
+        if pos is not None:
+            t = t.index_select(ax, torch.as_tensor(pos, device=dev))
+    return t.contiguous()
 
 
 def aggregate_host(plan, xs, layout, stride, tix, T, kind="identity", params=(), n_out=1,
@@ -692,7 +877,9 @@ class _OffsetOut:
 # deferred variables (`.values` of a transformed / reindexed variable)
 # ---------------------------------------------------------------------------
 def _to_device(v, dev):
-    """Materialise a (non-deferred) Variable on the device with its lazy takes applied."""
+    """Materialise a (non-deferred or daily) Variable on the device with its lazy takes applied."""
+    if v.deferred is not None and v.deferred.kind == "daily":
+        return daily_device(v, dev)
     a = v.physical
     t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a))
     t = t.to(dev)
@@ -708,6 +895,8 @@ def materialize_deferred(var):
     dev = default_device()
     if d.kind == "reindex":
         return d.params[0]()  # closure built by aggregations._pointwise_reindex
+    if d.kind == "daily":
+        return daily_device(var, dev).cpu().numpy()
     srcs = [_to_device(s, dev) for s in d.sources]
     if srcs[0].dtype not in _T2CTB:
         srcs = [s.to(torch.float64) for s in srcs]

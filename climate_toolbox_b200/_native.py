@@ -18,13 +18,14 @@ LAYOUT_TIME_MAJOR, LAYOUT_CELL_MAJOR = 0, 1
 TR_IDENTITY, TR_POLY, TR_EDD, TR_GDD, TR_BINS, TR_RCSPLINE = range(6)
 MAX_OUT = 4
 VARIANT_AUTO, VARIANT_STAGED, VARIANT_DIRECT = 0, 1, 2
+DAILY_MEAN, DAILY_MIN, DAILY_MAX = 1, 2, 4
 
 # every symbol include/ctb.h declares (tests check the .so exports each one)
 SYMBOLS = (
     "ctb_version", "ctb_last_error", "ctb_launch_count", "ctb_plan_build", "ctb_plan_free",
     "ctb_plan_get_info", "ctb_plan_row_cells", "ctb_plan_den", "ctb_plan_row_weights", "ctb_plan_region_order",
     "ctb_aggregate_workspace_bytes", "ctb_aggregate", "ctb_transform", "ctb_gather_rows",
-    "ctb_host_pack", "ctb_pull_pack", "ctb_copy_rows_to_host", "ctb_time_groups_create", "ctb_time_groups_free", "ctb_time_groups_count",
+    "ctb_host_pack", "ctb_pull_pack", "ctb_pull_pack_daily", "ctb_copy_rows_to_host", "ctb_time_groups_create", "ctb_time_groups_free", "ctb_time_groups_count",
     "ctb_aggregate_grouped_workspace_bytes", "ctb_aggregate_grouped", "ctb_aggregate_ex",
     "ctb_ipc_alloc", "ctb_ipc_open", "ctb_ipc_close", "ctb_ipc_free", "ctb_push_rows", "ctb_fingerprint",
 )
@@ -127,6 +128,8 @@ def lib():
     L.ctb_gather_rows.argtypes = [p, vp, C.c_int, C.c_int, i64, vp, i64, vp, vp]
     L.ctb_pull_pack.restype = C.c_int
     L.ctb_pull_pack.argtypes = [p, vp, C.c_int, i64, vp, i64, i64, vp, vp]
+    L.ctb_pull_pack_daily.restype = C.c_int
+    L.ctb_pull_pack_daily.argtypes = [p, vp, C.c_int, i64, C.c_int, vp, i64, i64, C.c_int, vp, vp, vp, vp]
     L.ctb_copy_rows_to_host.restype = C.c_int
     L.ctb_copy_rows_to_host.argtypes = [vp, C.c_size_t, vp, C.c_size_t, C.c_size_t, C.c_size_t, vp]
     L.ctb_time_groups_create.restype = C.c_int

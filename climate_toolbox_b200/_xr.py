@@ -50,7 +50,8 @@ class Deferred:
     """A pointwise gridcell transform that has not been evaluated yet.
 
     kind   : "poly" | "bins" | "rcspline" | "edd" | "gdd" | "reindex" (pointwise lat/lon gather,
-             params = (materialise closure, origin Dataset))
+             params = (materialise closure, origin Dataset)) | "daily" (daily reduction of a sub-daily
+             (time, lat, lon) source, params = (how, steps per day, first step, physical day of every day))
     params : tuple of floats (poly: (offset, power); bins: (offset, lo, hi); rcspline: (offset, term,
              k_1, ..., k_n); edd: (threshold,); gdd: (threshold_low, threshold_high))
     sources: tuple of :class:`Variable` (poly / bins / rcspline: (tas,); edd/gdd: (tasmin, tasmax))
@@ -88,7 +89,10 @@ class Variable:
     @property
     def shape(self):
         if self.deferred is not None:
-            return self.deferred.shape or self.deferred.sources[0].shape
+            d = self.deferred
+            if d.kind == "daily":
+                return (len(d.params[3]),) + d.sources[0].shape[1:]
+            return d.shape or d.sources[0].shape
         phys = tuple(self._data.shape)
         return tuple(len(self.takes[d]) if d in self.takes else phys[i]
                      for i, d in enumerate(self.dims))
@@ -100,7 +104,8 @@ class Variable:
     @property
     def dtype(self):
         if self.deferred is not None:
-            return np.dtype("float64")
+            d = self.deferred
+            return d.sources[0].dtype if d.kind == "daily" and d.params[0] != "mean" else np.dtype("float64")
         d = self._data.dtype
         return np.dtype(str(d).replace("torch.", "")) if _is_torch(self._data) else d
 
@@ -116,6 +121,13 @@ class Variable:
         pos = pos.astype(np.int64)
         if self.deferred is not None and self.deferred.kind == "reindex":
             return Variable(self.dims, self.values, self.attrs).with_take(dim, pos)
+        if self.deferred is not None and self.deferred.kind == "daily":
+            d = self.deferred
+            if dim == self.dims[0]:     # a take of days: the physical day of every kept day
+                new = Deferred(d.kind, d.params[:3] + (d.params[3][pos],), d.sources)
+            else:
+                new = Deferred(d.kind, d.params, tuple(s.with_take(dim, pos) for s in d.sources))
+            return Variable(self.dims, None, self.attrs, None, new)
         if self.deferred is not None:
             d = self.deferred
             new = Deferred(d.kind, d.params, tuple(s.with_take(dim, pos) for s in d.sources))

@@ -99,6 +99,55 @@ class _GridView:
                 and self.on_device == other.on_device)
 
 
+class _DailyView:
+    """A deferred daily reduction of sub-daily data (``utils.resample_daily``) as the kernels see it: packed
+    planes of days, written by the reduce-pack kernel for a compact plan of the daily planes' element size."""
+
+    layout = N.LAYOUT_TIME_MAJOR
+    tix = None
+
+    def __init__(self, var):
+        self.src = E.DailySource(var)
+        self.how = self.src.how
+        self.dims = self.out_dims_template = var.dims
+        self.other_dims = (var.dims[0],)
+        self.T = self.src.T
+        self.other_shape = (self.T,)
+        self.lat_phys, self.lon_phys = self.src.lat_phys, self.src.lon_phys
+        self.nlat_phys, self.nlon_phys = self.src.nlat_phys, self.src.nlon_phys
+        self.stride = self.src.stride
+        self.data2d = self.src.x
+        self.on_device = self.src.on_device
+        self.elem_bytes = 8 if self.how == "mean" else self.src.itemsize
+
+    def same_geometry(self, other):
+        return (isinstance(other, _DailyView) and self.T == other.T and self.elem_bytes == other.elem_bytes
+                and (self.nlat_phys, self.nlon_phys) == (other.nlat_phys, other.nlon_phys)
+                and _eq(self.lat_phys, other.lat_phys) and _eq(self.lon_phys, other.lon_phys)
+                and self.on_device == other.on_device)
+
+
+def _is_daily(var):
+    return var.deferred is not None and var.deferred.kind == "daily"
+
+
+def _view(var):
+    return _DailyView(var) if _is_daily(var) else _GridView(var)
+
+
+def _same_source(a, b):
+    """Two transform sources read the same data: the same buffer and takes, and for daily reductions also
+    the same ``how``, steps and days."""
+    if _is_daily(a) or _is_daily(b):
+        if not (_is_daily(a) and _is_daily(b)):
+            return False
+        pa, pb = a.deferred.params, b.deferred.params
+        return (pa[:3] == pb[:3] and np.array_equal(pa[3], pb[3]) and
+                _same_source(a.deferred.sources[0], b.deferred.sources[0]))
+    return (a.physical is b.physical and a.dims == b.dims and
+            all(_eq(a.takes.get(d), b.takes.get(d)) for d in a.dims))
+
+
 def _eq(a, b):
     if a is None or b is None:
         return a is None and b is None
@@ -107,7 +156,7 @@ def _eq(a, b):
 
 def _resolve(var):
     """Variable -> (kind, params, [source Variables])."""
-    if var.deferred is None:
+    if var.deferred is None or _is_daily(var):
         return "identity", (), [var]
     d = var.deferred
     if d.kind == "reindex":
@@ -124,7 +173,10 @@ def _coord_labels(ds, name):
 def _run_group(plan, views, kind, params, n_out, variant, groups=None, ingest=None, host_out=None, doy=None):
     """One fused launch for `n_out` outputs sharing the same sources."""
     v0 = views[0]
-    if v0.on_device:
+    if isinstance(v0, _DailyView):
+        out = E.aggregate_daily(plan, [(v.src, v.how) for v in views], kind, params, n_out, variant, groups,
+                                host_out, doy)
+    elif v0.on_device:
         out = E.aggregate_device(plan, views[0].data2d, views[1].data2d if len(views) > 1 else None,
                                  v0.layout, v0.stride, v0.tix, v0.T, kind, params, n_out, variant,
                                  groups=groups, doy=doy)
@@ -205,10 +257,7 @@ def _group_requests(reqs):
     for name, kind, params, srcs in reqs:
         placed = False
         for g in groups:
-            same_src = len(g["srcs"]) == len(srcs) and all(
-                a.physical is b.physical and a.dims == b.dims and
-                all(_eq(a.takes.get(d), b.takes.get(d)) for d in a.dims)
-                for a, b in zip(g["srcs"], srcs))
+            same_src = len(g["srcs"]) == len(srcs) and all(_same_source(a, b) for a, b in zip(g["srcs"], srcs))
             if not same_src or g["kind"] != kind or len(g["names"]) >= N.MAX_OUT:
                 continue
             if kind == "identity" or (kind in ("poly", "bins") and g["params"][0] != params[0]):
@@ -241,8 +290,12 @@ def _aggregate_core(ds, variables, aggwt, agglev, weights, backup_aggwt, variant
 
     out_ds = Dataset()
     for g in _group_requests(reqs):
-        views = [_GridView(s) for s in g["srcs"]]
+        views = [_view(s) for s in g["srcs"]]
         v0 = views[0]
+        daily = isinstance(v0, _DailyView)
+        if any(isinstance(v, _DailyView) != daily for v in views):
+            raise ValueError("inputs of a two-input transform must both be daily reductions of sub-daily data, "
+                             "or neither")
         for v in views[1:]:
             if not v0.same_geometry(v):
                 raise ValueError("inputs of a two-input transform must share shape, dtype and layout")
@@ -250,7 +303,8 @@ def _aggregate_core(ds, variables, aggwt, agglev, weights, backup_aggwt, variant
         dev = device or (v0.data2d.device if v0.on_device else E.default_device())
         # host-resident (time, lat, lon) inputs go through a compact plan: only the referenced
         # gridcells are packed on the host and cross PCIe
-        compact = (not v0.on_device) and v0.layout == N.LAYOUT_TIME_MAJOR and pack_host
+        # daily reductions of sub-daily data are packed by the reduce-pack kernel wherever the data lives
+        compact = daily or ((not v0.on_device) and v0.layout == N.LAYOUT_TIME_MAJOR and pack_host)
         cell_gate = doy = None
         if season_mask is not None:
             # growing-season gate (SURVEY 8-f3): per-gridcell (first, last, wrap) into the plan, day of

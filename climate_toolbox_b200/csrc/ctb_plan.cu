@@ -888,6 +888,160 @@ extern "C" int ctb_pull_pack(const ctb_plan* P, const void* x, int dtype, int64_
   return CTB_OK;
 }
 
+// ---------------------------------------------------------------- sub-daily ingest ---
+// Packing and the daily reduction in one read: day d of the packed planes reduces the steps
+// s = day[t_begin + d] * S + h, h = 0..S-1, of a TIME_MAJOR source in device or pinned host memory.
+// Mean: every step widened to fp64 and added in step order (plain adds), NaN steps skipped, the sum
+// divided by the count (0/0: NaN for a day without values).  Min / max: NaN steps skipped, exact, in
+// the source dtype; both come from the same loads.  Thread = one 16-byte unit of a packed piece x one
+// day with 8 step loads in flight; a warp's loads are contiguous along a run of referenced pieces.
+namespace {
+__device__ __forceinline__ float ext_min(float a, float b) { return fminf(a, b); }
+__device__ __forceinline__ float ext_max(float a, float b) { return fmaxf(a, b); }
+__device__ __forceinline__ double ext_min(double a, double b) { return fmin(a, b); }
+__device__ __forceinline__ double ext_max(double a, double b) { return fmax(a, b); }
+__device__ __forceinline__ void unit_get(const uint4& v, float (&e)[4]) {
+  e[0] = __uint_as_float(v.x); e[1] = __uint_as_float(v.y); e[2] = __uint_as_float(v.z); e[3] = __uint_as_float(v.w);
+}
+__device__ __forceinline__ void unit_get(const uint4& v, double (&e)[2]) {
+  e[0] = __hiloint2double((int)v.y, (int)v.x); e[1] = __hiloint2double((int)v.w, (int)v.z);
+}
+__device__ __forceinline__ uint4 unit_put(const float (&e)[4]) {
+  return make_uint4(__float_as_uint(e[0]), __float_as_uint(e[1]), __float_as_uint(e[2]), __float_as_uint(e[3]));
+}
+__device__ __forceinline__ uint4 unit_put(const double (&e)[2]) {
+  return make_uint4((unsigned)__double2loint(e[0]), (unsigned)__double2hiint(e[0]), (unsigned)__double2loint(e[1]),
+                    (unsigned)__double2hiint(e[1]));
+}
+
+template <typename T, bool MEAN, bool EXT>
+__global__ void __launch_bounds__(256) subdaily_pack_kernel(
+    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
+    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, double2* __restrict__ dst_mean,
+    uint4* __restrict__ dst_min, uint4* __restrict__ dst_max) {
+  constexpr int C = 16 / sizeof(T);   // cells per 16-byte unit
+  constexpr int U = 8;                // step loads in flight
+  const int64_t n_work = (int64_t)n_units * n_days;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_work; i += (int64_t)gridDim.x * blockDim.x) {
+    const int u = (int)(i % n_units);
+    const int d = (int)(i / n_units);
+    const int p = __ldg(pack_src + u / halves);
+    if (p < 0) continue;                       // alignment padding of the packed plane: never read
+    const int64_t step0 = (int64_t)(day ? __ldg(day + t_begin + d) : t_begin + d) * S;
+    const uint4* s = src + step0 * stride16 + (int64_t)p * halves + (u % halves);
+    double sum[C];
+    int cnt[C];
+    T mn[C], mx[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+      sum[c] = 0.0;
+      cnt[c] = 0;
+      mn[c] = mx[c] = (T)NAN;
+    }
+    for (int h0 = 0; h0 < S; h0 += U) {
+      uint4 v[U];
+#pragma unroll
+      for (int k = 0; k < U; ++k)
+        if (h0 + k < S)
+          asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
+                       : "=r"(v[k].x), "=r"(v[k].y), "=r"(v[k].z), "=r"(v[k].w)
+                       : "l"(s + (int64_t)(h0 + k) * stride16));
+#pragma unroll
+      for (int k = 0; k < U; ++k)
+        if (h0 + k < S) {
+          T e[C];
+          unit_get(v[k], e);
+#pragma unroll
+          for (int c = 0; c < C; ++c) {
+            if (MEAN && e[c] == e[c]) { sum[c] = __dadd_rn(sum[c], (double)e[c]); ++cnt[c]; }
+            if (EXT) { mn[c] = ext_min(mn[c], e[c]); mx[c] = ext_max(mx[c], e[c]); }
+          }
+        }
+    }
+    if (MEAN) {
+#pragma unroll
+      for (int c = 0; c < C; c += 2)
+        dst_mean[((int64_t)d * n_units + u) * (C / 2) + c / 2] =
+            make_double2(__ddiv_rn(sum[c], (double)cnt[c]), __ddiv_rn(sum[c + 1], (double)cnt[c + 1]));
+    }
+    if (EXT) {
+      if (dst_min) dst_min[(int64_t)d * n_units + u] = unit_put(mn);
+      if (dst_max) dst_max[(int64_t)d * n_units + u] = unit_put(mx);
+    }
+  }
+}
+
+template <typename T, bool MEAN, bool EXT>
+void launch_subdaily(unsigned grid, cudaStream_t st, const void* x, int64_t stride16, int S, const int32_t* day,
+                     int64_t t_begin, int n_days, const int32_t* pack_src, int n_units, int halves, void* dmean,
+                     void* dmin, void* dmax) {
+  subdaily_pack_kernel<T, MEAN, EXT><<<grid, 256, 0, st>>>(
+      static_cast<const uint4*>(x), stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
+      static_cast<double2*>(dmean), static_cast<uint4*>(dmin), static_cast<uint4*>(dmax));
+}
+}  // namespace
+
+extern "C" int ctb_pull_pack_daily(const ctb_plan* P, const void* x, int dtype, int64_t stride, int steps_per_day,
+                                   const int32_t* day_index, int64_t t_begin, int64_t n_days, int ops,
+                                   void* dst_mean, void* dst_min, void* dst_max, void* stream) {
+  if (!P || !x || n_days < 0 || n_days >= (1ll << 31) || t_begin < 0 || !P->compact) {
+    ctb_set_error("ctb_pull_pack_daily: needs a compact plan, a non-null source and 0 <= n_days < 2^31");
+    return CTB_ERR_INVALID;
+  }
+  if (dtype != CTB_F32 && dtype != CTB_F64) { ctb_set_error("dtype=%d unsupported", dtype); return CTB_ERR_INVALID; }
+  if (steps_per_day < 1) {
+    ctb_set_error("ctb_pull_pack_daily: steps_per_day=%d, needs >= 1", steps_per_day);
+    return CTB_ERR_INVALID;
+  }
+  if (ops == 0 || (ops & ~(CTB_DAILY_MEAN | CTB_DAILY_MIN | CTB_DAILY_MAX))) {
+    ctb_set_error("ctb_pull_pack_daily: ops=%d, needs a non-empty subset of CTB_DAILY_MEAN|MIN|MAX", ops);
+    return CTB_ERR_INVALID;
+  }
+  if (((ops & CTB_DAILY_MEAN) && !dst_mean) || ((ops & CTB_DAILY_MIN) && !dst_min) ||
+      ((ops & CTB_DAILY_MAX) && !dst_max)) {
+    ctb_set_error("ctb_pull_pack_daily: every requested op needs a destination");
+    return CTB_ERR_INVALID;
+  }
+  const int64_t es = dtype == CTB_F32 ? 4 : 8;
+  if ((ops & CTB_DAILY_MEAN) && P->elem_bytes != 8) {
+    ctb_set_error("ctb_pull_pack_daily: the mean plane is float64, the plan was built for %d-byte elements",
+                  P->elem_bytes);
+    return CTB_ERR_INVALID;
+  }
+  if ((ops & (CTB_DAILY_MIN | CTB_DAILY_MAX)) && P->elem_bytes != es) {
+    ctb_set_error("ctb_pull_pack_daily: min/max planes have the source's %d-byte elements, the plan was built "
+                  "for %d-byte elements", (int)es, P->elem_bytes);
+    return CTB_ERR_INVALID;
+  }
+  const int64_t phys_ncell = (int64_t)P->nlat_phys * P->nlon_phys;
+  if ((stride * es) % 16 != 0 || (uintptr_t)x % 16 != 0 || phys_ncell % CTB_PIECE != 0 ||
+      (uintptr_t)dst_mean % 16 != 0 || (uintptr_t)dst_min % 16 != 0 || (uintptr_t)dst_max % 16 != 0) {
+    ctb_set_error("ctb_pull_pack_daily: planes must be 16-byte aligned and hold a multiple of 4 gridcells");
+    return CTB_ERR_UNSUPPORTED;
+  }
+  if (n_days == 0) return CTB_OK;
+  CtbDeviceGuard guard(P->device);
+  if (guard.err != cudaSuccess) { ctb_set_error("cudaSetDevice(%d) failed: %s", P->device, cudaGetErrorString(guard.err)); return CTB_ERR_CUDA; }
+  const int halves = (int)(es / 4);
+  const int n_units = (int)(P->ncell / CTB_PIECE) * halves;
+  const int64_t n_work = (int64_t)n_units * n_days;
+  const unsigned grid = (unsigned)std::min<int64_t>((n_work + 255) / 256, 148 * 32);
+  const cudaStream_t st = (cudaStream_t)stream;
+  const bool mean = ops & CTB_DAILY_MEAN, ext = ops & (CTB_DAILY_MIN | CTB_DAILY_MAX);
+  void* dmin = (ops & CTB_DAILY_MIN) ? dst_min : nullptr;
+  void* dmax = (ops & CTB_DAILY_MAX) ? dst_max : nullptr;
+  auto go = [&](auto tag) {
+    using T = decltype(tag);
+    auto f = mean ? (ext ? launch_subdaily<T, true, true> : launch_subdaily<T, true, false>)
+                  : launch_subdaily<T, false, true>;
+    f(grid, st, x, stride * es / 16, steps_per_day, day_index, t_begin, (int)n_days, P->d_pack_src, n_units,
+      halves, dst_mean, dmin, dmax);
+  };
+  if (dtype == CTB_F32) go(float{}); else go(double{});
+  CTB_LAUNCH_CHECK();
+  return CTB_OK;
+}
+
 // ---------------------------------------------------------------------------
 // Fingerprint of a host buffer for the plan cache's fast path: 8 independent polynomial lanes
 // h_j = h_j * P + word (mod 2^64, P odd) over the 64-bit words j, j+8, ..., folded with a second

@@ -19,12 +19,26 @@ __all__ = ["snyder_edd", "snyder_gdd", "validate_edd_snyder_agriculture", "tas_p
 
 
 def _source(da):
+    """The stored data a transform reads: daily reductions of sub-daily data stay deferred (they are
+    reduced while the aggregation packs its inputs), other deferred variables are evaluated."""
     v = da.variable
-    return v if v.deferred is None else Variable(v.dims, v.values, v.attrs)
+    return v if v.deferred is None or v.deferred.kind == "daily" else Variable(v.dims, v.values, v.attrs)
+
+
+def _min_max_of_one_source(a, b):
+    """``a`` and ``b`` are the daily minimum and maximum of the same sub-daily data and days."""
+    da, db = a.deferred, b.deferred
+    return (da is not None and db is not None and da.kind == db.kind == "daily" and
+            (da.params[0], db.params[0]) == ("min", "max") and da.params[1:3] == db.params[1:3] and
+            np.array_equal(da.params[3], db.params[3]) and da.sources[0].physical is db.sources[0].physical and
+            da.sources[0].takes.keys() == db.sources[0].takes.keys() and
+            all(np.array_equal(da.sources[0].takes[k], db.sources[0].takes[k]) for k in da.sources[0].takes))
 
 
 def _any_less(a, b):
     """``(a < b).any()`` on the data's own device (precondition check only)."""
+    if _min_max_of_one_source(b, a):
+        return False          # a daily maximum is never below the minimum of the same steps
     pa, pb = a.physical, b.physical
     if isinstance(pa, torch.Tensor) and isinstance(pb, torch.Tensor) and not a.takes and not b.takes:
         return bool((pa < pb).any().item())

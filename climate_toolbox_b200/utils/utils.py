@@ -16,7 +16,7 @@ from .._xr import Dataset, DataArray, Deferred, Variable, from_any, to_like
 
 __all__ = ["convert_kelvin_to_celsius", "convert_lons_mono", "convert_lons_split",
            "rename_coords_to_lon_and_lat", "rename_coords_to_longitude_and_latitude",
-           "remove_leap_days", "season_boundaries", "get_daily_growing_season_mask", "GrowingSeasonMask"]
+           "remove_leap_days", "resample_daily", "season_boundaries", "get_daily_growing_season_mask", "GrowingSeasonMask"]
 
 
 def convert_kelvin_to_celsius(df, temp_name):
@@ -86,6 +86,104 @@ def remove_leap_days(ds):
     ds = from_any(ds)
     keep = ~((ds["time.month"].values == 2) & (ds["time.day"].values == 29))
     return to_like(ds.loc[{"time": keep}], like)
+
+
+_DAILY_HOW = ("mean", "min", "max")
+
+
+def _steps_per_day(time):
+    """Steps per day of a datetime64 time axis made of whole, consecutive calendar days that all hold the
+    same steps in the same order; ``ValueError`` otherwise.  Returns ``(S, days)``."""
+    t = np.asarray(time)
+    if not np.issubdtype(t.dtype, np.datetime64):
+        raise ValueError("resample_daily needs a datetime64 'time' coordinate, got {}".format(t.dtype))
+    if t.size == 0:
+        raise ValueError("resample_daily: the time axis is empty")
+    if np.isnat(t).any():
+        raise ValueError("resample_daily: the time axis holds NaT")
+    days = t.astype("datetime64[D]")
+    starts = np.flatnonzero(np.r_[True, days[1:] != days[:-1]])
+    uniq = days[starts]
+    if (np.diff(uniq) != np.timedelta64(1, "D")).any():
+        raise ValueError("resample_daily: every calendar day from {} to {} must be present once, as one run of "
+                         "steps".format(uniq.min(), uniq.max()))
+    counts = np.diff(np.r_[starts, t.size])
+    S = int(counts[0])
+    if (counts != S).any():
+        bad = int(np.flatnonzero(counts != S)[0])
+        raise ValueError("resample_daily: day {} has {} steps, day {} has {}".format(uniq[0], S, uniq[bad], counts[bad]))
+    offs = (t - days).reshape(-1, S)
+    if S > 1 and (np.diff(offs[0]) <= np.timedelta64(0)).any():
+        raise ValueError("resample_daily: the steps of day {} are not in increasing order".format(uniq[0]))
+    if (offs != offs[0]).any():
+        bad = int(np.flatnonzero((offs != offs[0]).any(axis=1))[0])
+        raise ValueError("resample_daily: day {} holds other steps than day {}".format(uniq[bad], uniq[0]))
+    return S, uniq
+
+
+def resample_daily(ds, how="mean"):
+    """Daily mean, minimum or maximum of sub-daily (hourly, 3- or 6-hourly) data, as xarray's
+    ``ds.resample(time="1D").mean()`` / ``.min()`` / ``.max()`` with ``skipna=True``.
+
+    ``ds``: a Dataset or DataArray whose ``time`` coordinate is datetime64 and consists of complete,
+    consecutive calendar days that hold the same S steps in the same order (``ValueError`` otherwise).
+    Variables over ``(time, lat, lon)`` become deferred daily variables over ``(time, lat, lon)`` with
+    ``time`` as the day (``datetime64[D]``); other variables without ``time`` are kept.  The reduction runs
+    on the GPU per gridcell while the referenced gridcells are packed for aggregation, so the daily grid is
+    never built: the result feeds ``tas_poly``, ``tas_bins``, ``tas_rcspline``, ``snyder_edd`` /
+    ``snyder_gdd``, ``remove_leap_days`` and ``weighted_aggregate_grid_to_regions`` directly, and
+    ``.values`` computes it for the whole grid.
+
+    * ``"mean"``: each step widened to float64 and summed in step order, NaN steps skipped, divided by the
+      number of non-NaN steps (NaN for a day without one); float64.
+    * ``"min"`` / ``"max"``: NaN steps skipped (NaN for a day without a value); exact, in the source dtype.
+
+    Attributes carry over, plus ``cell_methods = "time: <how>"``.  Sources over ``(lat, lon, time)`` raise
+    ``NotImplementedError``."""
+    if how not in _DAILY_HOW:
+        raise ValueError("how={!r}: expected one of {}".format(how, _DAILY_HOW))
+    like = ds
+    ds = from_any(ds)
+    single = isinstance(ds, DataArray)
+    if single:
+        ds = Dataset({ds.name or "_da": ds.variable}, coords=ds._coords)
+    if "time" not in ds._coords:
+        raise ValueError("resample_daily needs a 'time' coordinate")
+    S, days = _steps_per_day(ds._coords["time"].values)
+    out = Dataset()
+    for k, c in ds._coords.items():
+        if "time" not in c.dims:
+            out._coords[k] = c
+    out._coords["time"] = Variable(("time",), days, ds._coords["time"].attrs)
+    for name, var in ds._vars.items():
+        if "time" not in var.dims:
+            out._vars[name] = var
+            continue
+        if var.dims == ("lat", "lon", "time") or var.dims == ("lon", "lat", "time"):
+            raise NotImplementedError("resample_daily: {!r} is over {}; sub-daily sources must be over "
+                                      "(time, lat, lon)".format(name, var.dims))
+        if var.dims != ("time", "lat", "lon"):
+            raise ValueError("resample_daily: {!r} is over {}, expected (time, lat, lon)".format(name, var.dims))
+        if var.deferred is not None:
+            raise ValueError("resample_daily: {!r} is a deferred variable, not stored data".format(name))
+        # the kernel reads whole days from the first step on: a time take must be one run of steps
+        t0 = 0
+        takes = dict(var.takes)
+        pos = takes.pop("time", None)
+        if pos is not None:
+            if len(pos) and not np.array_equal(pos, np.arange(pos[0], pos[0] + len(pos))):
+                raise NotImplementedError("resample_daily: {!r} selects time steps out of physical order".format(name))
+            t0 = int(pos[0]) if len(pos) else 0
+        src = Variable(var.dims, var.physical, var.attrs, takes)
+        attrs = dict(var.attrs)
+        attrs["cell_methods"] = "time: {}".format(how)
+        out._vars[name] = Variable(var.dims, None, attrs, None,
+                                   Deferred("daily", (how, S, t0, np.arange(len(days), dtype=np.int64)), (src,)))
+    if single:
+        name = next(iter(out._vars))
+        res = DataArray._wrap(out._vars[name], out._coords_for(out._vars[name].dims), like.name)
+        return res
+    return to_like(out, like)
 
 
 # ---------------------------------------------------------------------------

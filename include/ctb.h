@@ -264,6 +264,21 @@ int ctb_host_pack(const ctb_plan* plan, const void* x, int dtype, int64_t stride
 int ctb_pull_pack(const ctb_plan* plan, const void* x, int dtype, int64_t stride, const int32_t* time_index,
                   int64_t t_begin, int64_t T, void* dst, void* stream);
 
+/* Sub-daily sources: the same pull, reducing steps_per_day (S >= 1) steps to one day while the referenced
+ * pieces are packed.  x[t_phys][stride] is TIME_MAJOR, in DEVICE or pinned HOST memory; day d < n_days
+ * reduces steps day_index[t_begin + d] * S + h, h = 0..S-1 (day_index: DEVICE int32, nullable = t_begin + d).
+ * ops is a non-empty mask of CTB_DAILY_*, each with its DEVICE destination [n_days][n_packed_cells]:
+ *   MEAN -> dst_mean, float64: steps widened to float64, added in step order with NaN steps skipped,
+ *           divided by the count of non-NaN steps (NaN for a day without one); needs plan elem_bytes 8;
+ *   MIN / MAX -> dst_min / dst_max, in the source dtype: NaN steps skipped (NaN for a day without a value),
+ *           exact; needs plan elem_bytes = the source's.  MIN and MAX together read the source once.
+ * Errors as ctb_pull_pack: a non-compact plan or a bad argument is CTB_ERR_INVALID, planes or
+ * destinations that are not 16-byte aligned CTB_ERR_UNSUPPORTED. */
+enum { CTB_DAILY_MEAN = 1, CTB_DAILY_MIN = 2, CTB_DAILY_MAX = 4 };
+int ctb_pull_pack_daily(const ctb_plan* plan, const void* x, int dtype, int64_t stride, int steps_per_day,
+                        const int32_t* day_index, int64_t t_begin, int64_t n_days, int ops, void* dst_mean,
+                        void* dst_min, void* dst_max, void* stream);
+
 /* rows of a pitched DEVICE array -> pitched HOST (pinned) array, one asynchronous 2-D copy on `stream`:
  * the host path returns out[:, :, t0:t1] of a finished time chunk while the next chunk is in flight */
 int ctb_copy_rows_to_host(void* dst, size_t dst_pitch, const void* src, size_t src_pitch, size_t width_bytes,
