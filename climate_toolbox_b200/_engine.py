@@ -110,7 +110,8 @@ class Plan:
     def time_index_device(self, tix):
         if tix is None:
             return None
-        key = hashlib.sha1(tix.tobytes()).hexdigest()
+        # arrays of another dtype or shape can hold the same bytes ([5, 0] int32 and [5] int64)
+        key = (tix.dtype.str, tix.shape, hashlib.sha1(tix.tobytes()).hexdigest())
         if key not in self._tix_cache:
             if len(self._tix_cache) > 16:
                 self._tix_cache.clear()
