@@ -495,49 +495,73 @@ def pack_threads():
     return max(1, (3 * ncpu) // 4)
 
 
-def _aggregate_packed(plan, pack, n_planes, itemsize, T, kind, params, n_out, variant, groups, out, host_out=None,
-                      chunk_bytes=4 << 30, doy=None):
-    """Compact plan whose inputs the GPU packs itself: ``pack(t0, n, bufs)`` queues on the current stream
-    what fills ``bufs`` (``n_planes`` device tensors [n, n_packed_cells] of ``itemsize``-byte elements) with
-    days t0 .. t0 + n - 1, then the kernel aggregates the packed planes.  Packs and kernels queue on one
-    stream.  With ``host_out`` (a pinned [n_out, R, T] tensor) the result goes back in time chunks on a
-    second stream while the next chunk is packed (PCIe is full duplex); the caller then only has to
-    synchronise.  Returns ``(out, host_out filled)``."""
+def _chunk_days(chunk_bytes, day_bytes):
+    """Days per time chunk: as many as ``chunk_bytes`` holds, in multiples of 32, at least 32."""
+    return max(32, int(chunk_bytes // max(day_bytes, 1)) // 32 * 32)
+
+
+def _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, out, doy, host_out=None,
+                layout=N.LAYOUT_TIME_MAJOR):
+    """Aggregate T days in time chunks of ``days``, one launch each -> ``(out, host_out filled)``; ``out`` is
+    allocated when None.
+    ``stage(ci, t0, n, done)`` queues on the current stream what makes days t0 .. t0 + n - 1 readable and returns
+    ``(bufs, stride, tix)``: 1 or 2 input tensors (on the device, or CPU tensors over mapped pinned memory), kept
+    referenced until their launch is queued; ``done[k]`` is the event recorded after the launch of chunk k.
+    With ``host_out`` (a pinned [n_out, R, T] tensor) and no time groups, each chunk's columns go back on a second
+    stream while the next chunk is staged (PCIe is full duplex); the caller then only has to synchronise."""
     dev = plan.device
-    width = plan.info["n_packed_cells"]
-    tdt = torch.float32 if itemsize == 4 else torch.float64
-    days = max(32, int(chunk_bytes // max(width * itemsize * n_planes, 1)) // 32 * 32)
-    if host_out is not None and groups is None:
-        days = min(days, max(32, (-(-T // 4) + 31) // 32 * 32))      # about four chunks: the last D2H is exposed
-    ws = _workspace(plan, min(days, T), n_out, N.LAYOUT_TIME_MAJOR, variant, groups, None)
-    starts = list(range(0, T, days))
+    if out is None:
+        out = torch.empty((n_out, plan.R, T if groups is None else groups.n_groups), dtype=torch.float64, device=dev)
+    if T == 0 or plan.R == 0:
+        return (out.zero_() if groups is not None else out), False
+    # one workspace for the whole call: split-region rows of a chunk, or -- with time groups -- of the whole
+    # time axis plus the per-tile partial sums
+    ws = _workspace(plan, min(days, T), n_out, layout, variant, groups, None)
     main = torch.cuda.current_stream(dev)
     back = torch.cuda.Stream(dev) if host_out is not None and groups is None else None
-    for t0 in starts:
+    done = []
+    for ci, t0 in enumerate(range(0, T, days)):
         n = min(T, t0 + days) - t0
-        bufs = [torch.empty((n, width), dtype=tdt, device=dev) for _ in range(n_planes)]
-        pack(t0, n, bufs)
-        if groups is None:
-            aggregate_device(plan, bufs[0], bufs[1] if len(bufs) > 1 else None, N.LAYOUT_TIME_MAJOR, width, None,
-                             n, kind, params, n_out, variant, out=_OffsetOut(out, t0), out_ld=T, workspace=ws,
-                             doy=None if doy is None else doy[t0: t0 + n])
-            if back is not None:
-                ev = torch.cuda.Event()
-                ev.record(main)
-                back.wait_event(ev)
-                N.check(N.lib().ctb_copy_rows_to_host(
-                    C.c_void_p(host_out.data_ptr() + 8 * t0), 8 * T, C.c_void_p(out.data_ptr() + 8 * t0), 8 * T,
-                    8 * n, n_out * plan.R, C.c_void_p(back.cuda_stream)))
-                TRANSFER_BYTES["d2h"] += 8 * n * n_out * plan.R
-        else:
-            aggregate_device(plan, bufs[0], bufs[1] if len(bufs) > 1 else None, N.LAYOUT_TIME_MAJOR, width, None,
-                             n, kind, params, n_out, variant, out=out, workspace=ws, groups=groups, t_begin=t0,
-                             flush=(t0 == starts[-1]), doy=doy)
+        bufs, stride, tix = stage(ci, t0, n, done)
+        if groups is None:      # columns t0 .. t0 + n - 1 of out, and those days of the day-of-year axis
+            o, ld, d = _OffsetOut(out, t0), T, None if doy is None else doy[t0: t0 + n]
+        else:                   # a window of the time groups; the last chunk flushes them
+            o, ld, d = out, 0, doy
+        _launch(plan, bufs[0].data_ptr(), bufs[1].data_ptr() if len(bufs) > 1 else 0, _T2CTB[bufs[0].dtype], layout,
+                stride, tix, n, kind, params, n_out, variant, o, ld, ws, None, groups, t0, t0 + n == T, d)
+        ev = torch.cuda.Event()
+        ev.record(main)
+        done.append(ev)
+        if back is not None:
+            back.wait_event(ev)
+            N.check(N.lib().ctb_copy_rows_to_host(
+                C.c_void_p(host_out.data_ptr() + 8 * t0), 8 * T, C.c_void_p(out.data_ptr() + 8 * t0), 8 * T,
+                8 * n, n_out * plan.R, C.c_void_p(back.cuda_stream)))
+            TRANSFER_BYTES["d2h"] += 8 * n * n_out * plan.R
     if back is not None:
         out.record_stream(back)
         main.wait_stream(back)
-        return out, True
-    return out, False
+    return out, back is not None
+
+
+def _aggregate_packed(plan, pack, n_planes, itemsize, T, kind, params, n_out, variant, groups, out, host_out=None,
+                      chunk_bytes=4 << 30, doy=None):
+    """Compact plan whose inputs the GPU packs itself: ``pack(t0, n, bufs)`` queues on the current stream
+    what fills ``bufs`` (``n_planes`` fresh device tensors [n, n_packed_cells] of ``itemsize``-byte elements)
+    with days t0 .. t0 + n - 1, then the kernel aggregates the packed planes.  Packs and kernels queue on one
+    stream; ``out`` and ``host_out`` as :func:`_run_chunks`."""
+    width = plan.info["n_packed_cells"]
+    tdt = torch.float32 if itemsize == 4 else torch.float64
+    days = _chunk_days(chunk_bytes, width * itemsize * n_planes)
+    if host_out is not None and groups is None:
+        days = min(days, max(32, (-(-T // 4) + 31) // 32 * 32))      # about four chunks: the last D2H is exposed
+
+    def stage(ci, t0, n, done):
+        bufs = [torch.empty((n, width), dtype=tdt, device=plan.device) for _ in range(n_planes)]
+        pack(t0, n, bufs)
+        return bufs, width, None
+
+    return _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, out, doy, host_out)
 
 
 def _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, groups, out, host_out=None,
@@ -671,11 +695,6 @@ def aggregate_daily(plan, srcs, kind="identity", params=(), n_out=1, variant=N.V
     dtype for min / max; the plan is built for that element size) and aggregated by the compact-plan
     launch; sources that read the same steps -- the daily minimum and maximum of one variable -- come from
     one call.  ``host_out``: as :func:`aggregate_host`."""
-    dev = plan.device
-    T = srcs[0][0].T
-    out = torch.empty((n_out, plan.R, T if groups is None else groups.n_groups), dtype=torch.float64, device=dev)
-    if T == 0 or plan.R == 0:
-        return out.zero_() if groups is not None else out
     calls = []          # [(DailySource, {how: plane index})]
     for i, (src, how) in enumerate(srcs):
         for c in calls:
@@ -690,8 +709,8 @@ def aggregate_daily(plan, srcs, kind="identity", params=(), n_out=1, variant=N.V
             _pull_daily(plan, src, {h: bufs[i] for h, i in planes.items()}, t0, n)
 
     itemsize = 8 if srcs[0][1] == "mean" else srcs[0][0].itemsize
-    out, filled = _aggregate_packed(plan, pack, len(srcs), itemsize, T, kind, params, n_out, variant, groups, out,
-                                    host_out[0] if host_out is not None else None, doy=doy)
+    out, filled = _aggregate_packed(plan, pack, len(srcs), itemsize, srcs[0][0].T, kind, params, n_out, variant,
+                                    groups, None, host_out[0] if host_out is not None else None, doy=doy)
     if host_out is not None:
         host_out[1] = filled
     return out
@@ -733,6 +752,27 @@ def daily_device(var, dev):
     return t.contiguous()
 
 
+def _ingest_route(layout, compact, variant, dtype_ok, aligned, pinned, zero_copy=None, ingest=None):
+    """Route of host inputs to the kernel: "cell_major", "zero_copy", "pull", "host_pack" or "full_copy" (see
+    :func:`aggregate_host`).  ``aligned``: 16-byte aligned inputs and planes, whole 4-cell pieces; ``zero_copy`` /
+    ``ingest`` None: ``CTB_ZERO_COPY`` / ``CTB_INGEST``."""
+    if layout == N.LAYOUT_CELL_MAJOR:
+        return "cell_major"
+    if zero_copy is None:
+        # opt-in: on the round-1 box the in-place read moved 2.5 GB at ~7 GB/s (16-byte requests
+        # over PCIe) and lost to copying all 6 GB at ~21 GB/s (profiles/r1_e2e_notes.md)
+        zero_copy = os.environ.get("CTB_ZERO_COPY", "0") == "1"
+    if zero_copy and not compact and (variant & 0xff) != N.VARIANT_DIRECT and dtype_ok and pinned:
+        return "zero_copy"
+    if ingest is None:
+        ingest = os.environ.get("CTB_INGEST", "auto")
+    if compact and ingest in ("auto", "pull") and dtype_ok and aligned and pinned:
+        return "pull"
+    if ingest == "pull":
+        raise ValueError("ingest='pull' needs a compact plan and 16-byte aligned inputs in pinned host memory")
+    return "host_pack" if compact else "full_copy"
+
+
 def aggregate_host(plan, xs, layout, stride, tix, T, kind="identity", params=(), n_out=1,
                    variant=N.VARIANT_AUTO, chunk_bytes=192 << 20, zero_copy=None, threads=0, groups=None,
                    ingest=None, host_out=None, doy=None):
@@ -755,112 +795,88 @@ def aggregate_host(plan, xs, layout, stride, tix, T, kind="identity", params=(),
     caller synchronises the stream); otherwise the flag stays False and the caller copies ``out``.
     """
     dev = plan.device
-    n_cols = T if groups is None else groups.n_groups
-    out = torch.empty((n_out, plan.R, n_cols), dtype=torch.float64, device=dev)
-    if T == 0 or plan.R == 0:
-        return out.zero_() if groups is not None else out
-    if layout == N.LAYOUT_CELL_MAJOR:
-        d = [torch.from_numpy(x).to(dev, non_blocking=True) for x in xs]
-        TRANSFER_BYTES["h2d"] += sum(x.nbytes for x in xs)
-        return aggregate_device(plan, d[0], d[1] if len(d) > 1 else None, layout, stride, tix, T,
-                                kind, params, n_out, variant, out=out, groups=groups, doy=doy)
-    if zero_copy is None:
-        # opt-in: on the round-1 box the in-place read moved 2.5 GB at ~7 GB/s (16-byte requests
-        # over PCIe) and lost to copying all 6 GB at ~21 GB/s (profiles/r1_e2e_notes.md)
-        zero_copy = os.environ.get("CTB_ZERO_COPY", "0") == "1"
-    if zero_copy and not plan.compact and (variant & 0xff) != N.VARIANT_DIRECT \
-            and xs[0].dtype in _NP2CTB and _all_pinned(xs):
-        # pinned (mapped) host arrays: the kernel reads them in place over PCIe, so only the
-        # referenced gridcells (~30 % of a global land/ocean grid) cross the bus
-        return _launch(plan, xs[0].ctypes.data, xs[1].ctypes.data if len(xs) > 1 else 0,
-                       _NP2CTB[xs[0].dtype], layout, stride, tix, T, kind, params, n_out,
-                       N.VARIANT_STAGED | 0x100, out, 0, None, None, groups, 0, True, doy)
-
-    if ingest is None:
-        ingest = os.environ.get("CTB_INGEST", "auto")
-    if plan.compact and ingest in ("auto", "pull") and xs[0].dtype in _NP2CTB and \
-            (stride * xs[0].dtype.itemsize) % 16 == 0 and (plan.info["n_cells_grid"] % 4 == 0) and \
-            all(x.ctypes.data % 16 == 0 for x in xs) and _all_pinned(xs):
-        # pinned (device-accessible) source: the GPU pulls the referenced pieces itself
-        out, filled = _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, groups, out,
+    if len(xs) > 1 and (xs[1].dtype != xs[0].dtype or xs[1].shape != xs[0].shape):
+        raise ValueError("the two inputs must agree in dtype and shape")
+    itemsize = xs[0].dtype.itemsize
+    aligned = ((stride * itemsize) % 16 == 0 and plan.info["n_cells_grid"] % 4 == 0 and
+               all(x.ctypes.data % 16 == 0 for x in xs))
+    route = _ingest_route(layout, plan.compact, variant, xs[0].dtype in _NP2CTB, aligned, _all_pinned(xs),
+                          zero_copy, ingest)
+    if route == "pull":
+        out, filled = _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, groups, None,
                                       host_out[0] if host_out is not None else None, doy=doy)
         if host_out is not None:
             host_out[1] = filled
         return out
-    if ingest == "pull":
-        raise ValueError("ingest='pull' needs a compact plan and 16-byte aligned inputs in pinned host memory")
+    if route in ("cell_major", "zero_copy"):
+        if route == "zero_copy":
+            # pinned (mapped) host arrays: the kernel reads them in place over PCIe, so only the
+            # referenced gridcells (~30 % of a global land/ocean grid) cross the bus
+            variant = N.VARIANT_STAGED | N.VARIANT_MAPPED_HOST
 
+        def stage(ci, t0, n, done):
+            if route == "zero_copy":
+                return [torch.from_numpy(x) for x in xs], stride, tix
+            TRANSFER_BYTES["h2d"] += sum(x.nbytes for x in xs)
+            return [torch.from_numpy(x).to(dev, non_blocking=True) for x in xs], stride, tix
+
+        return _run_chunks(plan, T, T, stage, kind, params, n_out, variant, groups, None, doy, layout=layout)[0]
+
+    # host_pack / full_copy: two staging slots in turn, copied on a second stream
     threads = threads or pack_threads()
     main = torch.cuda.current_stream(dev)
     copy_stream = torch.cuda.Stream(dev)
     copy_stream.wait_stream(main)
     tix_full = None if tix is None else np.ascontiguousarray(tix, dtype=np.int64)
-    itemsize = xs[0].dtype.itemsize
     width = plan.info["n_packed_cells"] if plan.compact else xs[0].shape[1]
-    days = max(32, int(chunk_bytes // max(width * itemsize * len(xs), 1)) // 32 * 32)
-    # one workspace for the whole call: split-region rows of a chunk, or -- with time groups -- of
-    # the whole time axis plus the per-tile partial sums
-    ws = _workspace(plan, min(days, T), n_out, layout, variant, groups, None)
+    days = _chunk_days(chunk_bytes, width * itemsize * len(xs))
     tdt = torch.float32 if itemsize == 4 else torch.float64
-    dbuf, free_ev = {}, {}
-    ts = None if plan.compact else [torch.from_numpy(x) for x in xs]
+    dbuf = {}
     di = dev.index or 0
-    starts = list(range(0, T, days))
+
+    def stage(ci, t0, n, done):
+        slot = ci % 2
+        rel = None
+        pin_ents = []
+        if plan.compact:
+            # pack on the host (GIL released) while the previous chunk is in flight
+            srcs = []
+            for k, x in enumerate(xs):
+                ent = _pinned_buffer((di, slot, k), days * width * itemsize)   # waits for its last H2D
+                pin_ents.append(ent)
+                N.check(N.lib().ctb_host_pack(
+                    plan._h, C.c_void_p(x.ctypes.data), _NP2CTB[x.dtype], int(stride),
+                    tix_full.ctypes.data_as(C.POINTER(C.c_int64)) if tix_full is not None else None,
+                    int(t0), int(n), C.c_void_p(ent[0].data_ptr()), int(threads)))
+                srcs.append(ent[0][: n * width * itemsize].view(tdt).view(n, width))
+        else:
+            sub = np.arange(t0, t0 + n) if tix_full is None else tix_full[t0: t0 + n]
+            lo, hi = int(sub.min()), int(sub.max()) + 1
+            srcs = [torch.from_numpy(x)[lo:hi] for x in xs]
+            if tix_full is not None and not np.array_equal(sub - lo, np.arange(n)):
+                rel = sub - lo
+        with torch.cuda.stream(copy_stream):
+            if ci >= 2:
+                copy_stream.wait_event(done[ci - 2])     # the last launch that read this slot
+            cur = []
+            for k, src in enumerate(srcs):
+                b = dbuf.get((slot, k))
+                if b is None or b.shape[0] < src.shape[0]:
+                    b = torch.empty((max(src.shape[0], days + 8), src.shape[1]), dtype=tdt, device=dev)
+                    b.record_stream(main)
+                    dbuf[(slot, k)] = b
+                b[: src.shape[0]].copy_(src, non_blocking=True)
+                TRANSFER_BYTES["h2d"] += src.numel() * src.element_size()
+                cur.append(b)
+            ready = torch.cuda.Event()
+            ready.record(copy_stream)
+            for ent in pin_ents:
+                ent[1] = ready      # outlives this call: the next packer of the buffer waits for it
+        main.wait_event(ready)
+        return cur, width, rel
+
     with _HOST_LOCK:
-        for ci, t0 in enumerate(starts):
-            t1 = min(T, t0 + days)
-            n = t1 - t0
-            slot = ci % 2
-            rel = None
-            pin_ents = []
-            if plan.compact:
-                # pack on the host (GIL released) while the previous chunk is in flight
-                pins = []
-                for k, x in enumerate(xs):
-                    ent = _pinned_buffer((di, slot, k), days * width * itemsize)   # waits for its last H2D
-                    pin_ents.append(ent)
-                    N.check(N.lib().ctb_host_pack(
-                        plan._h, C.c_void_p(x.ctypes.data), _NP2CTB[x.dtype], int(stride),
-                        tix_full.ctypes.data_as(C.POINTER(C.c_int64)) if tix_full is not None else None,
-                        int(t0), int(n), C.c_void_p(ent[0].data_ptr()), int(threads)))
-                    pins.append(ent[0][: n * width * itemsize].view(tdt).view(n, width))
-                srcs = pins
-            else:
-                sub = np.arange(t0, t1) if tix_full is None else tix_full[t0:t1]
-                lo, hi = int(sub.min()), int(sub.max()) + 1
-                srcs = [t[lo:hi] for t in ts]
-                if tix_full is not None and not np.array_equal(sub - lo, np.arange(n)):
-                    rel = sub - lo
-            with torch.cuda.stream(copy_stream):
-                if slot in free_ev:
-                    copy_stream.wait_event(free_ev[slot])
-                cur = []
-                for k, src in enumerate(srcs):
-                    b = dbuf.get((slot, k))
-                    if b is None or b.shape[0] < src.shape[0]:
-                        b = torch.empty((max(src.shape[0], days + 8), src.shape[1]), dtype=tdt, device=dev)
-                        b.record_stream(main)
-                        dbuf[(slot, k)] = b
-                    b[: src.shape[0]].copy_(src, non_blocking=True)
-                    TRANSFER_BYTES["h2d"] += src.numel() * src.element_size()
-                    cur.append(b)
-                ready = torch.cuda.Event()
-                ready.record(copy_stream)
-                for ent in pin_ents:
-                    ent[1] = ready      # outlives this call: the next packer of the buffer waits for it
-            main.wait_event(ready)
-            if groups is None:
-                aggregate_device(plan, cur[0], cur[1] if len(cur) > 1 else None, layout, width, rel, n, kind,
-                                 params, n_out, variant, out=_OffsetOut(out, t0), out_ld=T, workspace=ws,
-                                 doy=None if doy is None else doy[t0: t1])
-            else:
-                aggregate_device(plan, cur[0], cur[1] if len(cur) > 1 else None, layout, width, rel, n, kind,
-                                 params, n_out, variant, out=out, workspace=ws, groups=groups, t_begin=t0,
-                                 flush=(t0 == starts[-1]), doy=doy)
-            ev = torch.cuda.Event()
-            ev.record(main)
-            free_ev[slot] = ev
-    return out
+        return _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, None, doy, layout=layout)[0]
 
 
 class _OffsetOut:

@@ -18,6 +18,7 @@ LAYOUT_TIME_MAJOR, LAYOUT_CELL_MAJOR = 0, 1
 TR_IDENTITY, TR_POLY, TR_EDD, TR_GDD, TR_BINS, TR_RCSPLINE = range(6)
 MAX_OUT = 4
 VARIANT_AUTO, VARIANT_STAGED, VARIANT_DIRECT = 0, 1, 2
+VARIANT_MAPPED_HOST = 0x100   # or-ed into a variant: x0 / x1 are mapped pinned host memory, read in place
 DAILY_MEAN, DAILY_MIN, DAILY_MAX = 1, 2, 4
 
 # every symbol include/ctb.h declares (tests check the .so exports each one)
