@@ -557,16 +557,19 @@ __global__ void __launch_bounds__(THREADS, 1) agg_stream_kernel(const AggArgs a)
 #pragma unroll
             for (int dd = 0; dd < CTB_TB / 4; ++dd, dst += 4 * CTB_ROWB) {
               if (dd * 4 + l4 < n_days) {
-                // byte addressing here: row pointer (64-bit, one multiply per row) + the unit's 32-bit byte
-                // offset.  (Measured: 0.69 -> 0.63 ms in this branch; the SAME form in the branch above
-                // costs it 2 %, 0.60 -> 0.61 ms, so that one keeps the element arithmetic.)
+                // byte addressing here: row pointer (64-bit, one multiply per row) + the unit's byte offset,
+                // a 32 x 32 -> 64-bit product (one IMAD.WIDE.U32): a float64 cell at or past 2^29 lies 4 GiB
+                // or more into its plane.  (Measured: 0.69 -> 0.63 ms in this branch; the SAME form in the
+                // branch above costs it 2 %, 0.60 -> 0.61 ms, so that one keeps the element arithmetic.  The
+                // 64-bit product against the 32-bit one it replaced, bench_micro/tix_cost.py on a B200 at 1,000 W:
+                // 0.640 / 0.648 ms with a time index.)
                 const int64_t ro = (int64_t)plane[dd] * stride_b;
                 const unsigned char* const r0 = reinterpret_cast<const unsigned char*>(X0) + ro;
                 const unsigned char* const r1 = reinterpret_cast<const unsigned char*>(X1) + ro;
 #pragma unroll
                 for (int gi = 0; gi < UPW; ++gi)
                   if (ok[gi])
-                    cp_async16(dst + dst_of[gi], (NIN == 2 && second[gi] ? r1 : r0) + (uint32_t)off[gi] * (uint32_t)sizeof(TIN));
+                    cp_async16(dst + dst_of[gi], (NIN == 2 && second[gi] ? r1 : r0) + (uint64_t)(uint32_t)off[gi] * sizeof(TIN));
               }
 #if CTB_PACE_NS > 0
               __nanosleep(CTB_PACE_NS);
