@@ -335,6 +335,32 @@ def aggregate_shard_p2p(plan, x0, x1, stride, T, peer_out, kind="identity", para
     return peer_out.gathered() if gathered else peer_out.raw
 
 
+def _shard_groups(gid, T, world):
+    """First global time group and number of groups of every rank's days, from the group id of every
+    day of the full axis.  A group that spans a shard boundary is counted by every rank it touches."""
+    firsts, counts = [], []
+    for r in range(world):
+        t0, t1 = shard_range(T, world, r)
+        firsts.append(int(gid[t0]) if t1 > t0 else 0)
+        counts.append(int(gid[t1 - 1]) - int(gid[t0]) + 1 if t1 > t0 else 0)
+    return firsts, counts
+
+
+def _sum_group_blocks(full2d, recv, firsts, counts):
+    """full2d[:, f_r : f_r + n_r] from recv[r, :, :n_r] of every rank r, in rank order.  A group's first
+    contribution is copied and a later one (the group continues from the previous shard) is added to it,
+    so a group that lies inside one shard keeps the exact bits its rank computed."""
+    done = 0                                       # groups [0, done) hold a contribution
+    for r, (f, n) in enumerate(zip(firsts, counts)):
+        if n == 0:
+            continue
+        k = min(n, max(0, done - f))              # leading groups continued from an earlier shard
+        if k:
+            full2d[:, f: f + k] += recv[r, :, :k]
+        full2d[:, f + k: f + n].copy_(recv[r, :, k:n])
+        done = max(done, f + n)
+
+
 def aggregate_time_sharded(ds, variable, aggwt, agglev, weights, backup_aggwt="areawt", gather=True,
                            group=None, time_dim="time", aggregate_fn=None, **engine_opts):
     """``weighted_aggregate_grid_to_regions`` over a process group: every rank aggregates its own
@@ -345,24 +371,38 @@ def aggregate_time_sharded(ds, variable, aggwt, agglev, weights, backup_aggwt="a
     year-block would otherwise cross NVLink for nothing).  Variables may carry leading dims
     (ensemble member, model): everything but ``time_dim`` rides along.
 
+    ``time_groups=`` (``"year"``, a block length or one label per step) is resolved once on the full
+    time axis, so groups are the ones the single-process call forms; each rank sums the groups its days
+    touch, and the gather adds the parts of a group that spans a shard boundary, in rank order.  With
+    ``gather=False`` a rank returns the sums over its own days, labelled with the global group labels:
+    its first and last group may then be partial, and the sum of every rank's part is the full group.
+
     ``aggregate_fn`` (tests) replaces the single-GPU aggregation; it must have the signature of
     ``weighted_aggregate_grid_to_regions``.
     """
     from ._xr import Dataset, Variable, from_any
+    from .aggregations.aggregations import _time_group_ids
     if aggregate_fn is None:
         from .aggregations.aggregations import weighted_aggregate_grid_to_regions as aggregate_fn
     ds = from_any(ds)
     if not (dist.is_available() and dist.is_initialized()):
         return aggregate_fn(ds, variable, aggwt, agglev, weights=weights, backup_aggwt=backup_aggwt,
-                            **engine_opts)
+                            time_dim=time_dim, **engine_opts)
     world, rank = dist.get_world_size(group), dist.get_rank(group)
     T = ds.dims[time_dim]
     t0, t1 = shard_range(T, world, rank)
+    spec = engine_opts.pop("time_groups", None)
+    if spec is not None:
+        # every rank resolves the same groups (or raises the same error) without communicating
+        gid, glabels = _time_group_ids(ds, time_dim, T, spec)
+        engine_opts["time_groups"] = glabels[gid[t0:t1]]              # one global label per step of the shard
     local = aggregate_fn(ds.isel(**{time_dim: np.arange(t0, t1)}), variable, aggwt, agglev,
-                         weights=weights, backup_aggwt=backup_aggwt, **engine_opts)
+                         weights=weights, backup_aggwt=backup_aggwt, time_dim=time_dim, **engine_opts)
     local = from_any(local)
     if not gather:
         return local
+    if spec is not None:
+        firsts, counts = _shard_groups(gid, T, world)
     names = [variable] if isinstance(variable, str) else list(variable)
     backend = dist.get_backend(group)
     out = Dataset()
@@ -373,10 +413,24 @@ def aggregate_time_sharded(ds, variable, aggwt, agglev, weights, backup_aggwt="a
         if backend == "nccl" and not a.is_cuda:
             a = a.cuda()
         blk = a.movedim(ax_t, -1).contiguous()                            # [..., T_local]
-        full = all_gather_time(blk, T, group).movedim(-1, ax_t)           # back to the variable's dim order
+        if spec is None:
+            full = all_gather_time(blk, T, group)
+        else:
+            lead = tuple(blk.shape[:-1])
+            M = int(np.prod(lead)) if lead else 1
+            recv = _gather_padded(blk.reshape(M, blk.shape[-1]), max(counts), group)
+            full = torch.empty((M, len(glabels)), dtype=blk.dtype, device=blk.device)
+            _sum_group_blocks(full, recv, firsts, counts)
+            full = full.reshape(lead + (len(glabels),))
+        full = full.movedim(-1, ax_t)                                     # back to the variable's dim order
         out[name] = Variable(v.dims, full if full.is_cuda else full.numpy(), v.attrs)
     out._coords[agglev] = local._coords[agglev]
     for d, c in ds._coords.items():
-        if d not in ("lat", "lon") and "lat" not in c.dims and "lon" not in c.dims:
-            out._coords[d] = Variable(c.dims, c.values, c.attrs)
+        if d in ("lat", "lon") or "lat" in c.dims or "lon" in c.dims:
+            continue
+        if spec is not None and time_dim in c.dims:      # the time axis is now one step per group
+            if d == time_dim:
+                out._coords[d] = Variable((d,), np.asarray(glabels))
+            continue
+        out._coords[d] = Variable(c.dims, c.values, c.attrs)
     return out
