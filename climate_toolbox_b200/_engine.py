@@ -501,9 +501,10 @@ def _chunk_days(chunk_bytes, day_bytes):
 
 
 def _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, out, doy, host_out=None,
-                layout=N.LAYOUT_TIME_MAJOR):
+                layout=N.LAYOUT_TIME_MAJOR, per_plane=False):
     """Aggregate T days in time chunks of ``days``, one launch each -> ``(out, host_out filled)``; ``out`` is
-    allocated when None.
+    allocated when None.  ``per_plane``: the chunk's n_out input planes are aggregated one launch each, plane j
+    into out[j] (single-input ``kind``, n_out = 1 per launch).
     ``stage(ci, t0, n, done)`` queues on the current stream what makes days t0 .. t0 + n - 1 readable and returns
     ``(bufs, stride, tix)``: 1 or 2 input tensors (on the device, or CPU tensors over mapped pinned memory), kept
     referenced until their launch is queued; ``done[k]`` is the event recorded after the launch of chunk k.
@@ -516,19 +517,24 @@ def _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, out,
         return (out.zero_() if groups is not None else out), False
     # one workspace for the whole call: split-region rows of a chunk, or -- with time groups -- of the whole
     # time axis plus the per-tile partial sums
-    ws = _workspace(plan, min(days, T), n_out, layout, variant, groups, None)
+    # (per plane: one each, since with time groups a workspace carries a plane's partial sums across chunks)
+    ws = [_workspace(plan, min(days, T), 1 if per_plane else n_out, layout, variant, groups, None)
+          for _ in range(n_out if per_plane else 1)]
     main = torch.cuda.current_stream(dev)
     back = torch.cuda.Stream(dev) if host_out is not None and groups is None else None
     done = []
     for ci, t0 in enumerate(range(0, T, days)):
         n = min(T, t0 + days) - t0
         bufs, stride, tix = stage(ci, t0, n, done)
-        if groups is None:      # columns t0 .. t0 + n - 1 of out, and those days of the day-of-year axis
-            o, ld, d = _OffsetOut(out, t0), T, None if doy is None else doy[t0: t0 + n]
-        else:                   # a window of the time groups; the last chunk flushes them
-            o, ld, d = out, 0, doy
-        _launch(plan, bufs[0].data_ptr(), bufs[1].data_ptr() if len(bufs) > 1 else 0, _T2CTB[bufs[0].dtype], layout,
-                stride, tix, n, kind, params, n_out, variant, o, ld, ws, None, groups, t0, t0 + n == T, d)
+        for j, ins in enumerate([bufs[j: j + 1] for j in range(n_out)] if per_plane else [bufs]):
+            oj = out[j: j + 1] if per_plane else out
+            if groups is None:      # columns t0 .. t0 + n - 1 of out, and those days of the day-of-year axis
+                o, ld, d = _OffsetOut(oj, t0), T, None if doy is None else doy[t0: t0 + n]
+            else:                   # a window of the time groups; the last chunk flushes them
+                o, ld, d = oj, 0, doy
+            _launch(plan, ins[0].data_ptr(), ins[1].data_ptr() if len(ins) > 1 else 0, _T2CTB[ins[0].dtype], layout,
+                    stride, tix, n, kind, params, 1 if per_plane else n_out, variant, o, ld, ws[j], None, groups, t0,
+                    t0 + n == T, d)
         ev = torch.cuda.Event()
         ev.record(main)
         done.append(ev)
@@ -545,11 +551,11 @@ def _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, out,
 
 
 def _aggregate_packed(plan, pack, n_planes, itemsize, T, kind, params, n_out, variant, groups, out, host_out=None,
-                      chunk_bytes=4 << 30, doy=None):
+                      chunk_bytes=4 << 30, doy=None, per_plane=False):
     """Compact plan whose inputs the GPU packs itself: ``pack(t0, n, bufs)`` queues on the current stream
     what fills ``bufs`` (``n_planes`` fresh device tensors [n, n_packed_cells] of ``itemsize``-byte elements)
     with days t0 .. t0 + n - 1, then the kernel aggregates the packed planes.  Packs and kernels queue on one
-    stream; ``out`` and ``host_out`` as :func:`_run_chunks`."""
+    stream; ``out``, ``host_out`` and ``per_plane`` as :func:`_run_chunks`."""
     width = plan.info["n_packed_cells"]
     tdt = torch.float32 if itemsize == 4 else torch.float64
     days = _chunk_days(chunk_bytes, width * itemsize * n_planes)
@@ -561,7 +567,8 @@ def _aggregate_packed(plan, pack, n_planes, itemsize, T, kind, params, n_out, va
         pack(t0, n, bufs)
         return bufs, width, None
 
-    return _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, out, doy, host_out)
+    return _run_chunks(plan, T, days, stage, kind, params, n_out, variant, groups, out, doy, host_out,
+                       per_plane=per_plane)
 
 
 def _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, groups, out, host_out=None,
@@ -586,9 +593,11 @@ def _aggregate_pull(plan, xs, stride, tix, T, kind, params, n_out, variant, grou
 
 
 # ---------------------------------------------------------------------------
-# sub-daily sources: daily mean / min / max reduced while the referenced pieces are packed
+# sub-daily sources: daily mean / min / max, or the daily mean of a per-step transform, reduced while the
+# referenced pieces are packed
 # ---------------------------------------------------------------------------
 _DAILY_OP = {"mean": N.DAILY_MEAN, "min": N.DAILY_MIN, "max": N.DAILY_MAX}
+_STEP_OP = {"edd": N.STEP_EDD, "gdd": N.STEP_GDD, "bins": N.STEP_BINS}
 DAILY_STAGE_BYTES = 256 << 20    # pinned staging slot of a pageable sub-daily source
 
 
@@ -617,6 +626,7 @@ class DailySource:
         self.stride = self.nlat_phys * self.nlon_phys
         self.x = x.reshape(x.shape[0], self.stride)
         self.itemsize = 4 if self.dtype == N.F32 else 8
+        self.out_bytes = self.itemsize if self.how in ("min", "max") else 8     # element size of its daily planes
         self.lat_phys, self.lon_phys = src.takes.get("lat"), src.takes.get("lon")
         self.T = len(self.day)
 
@@ -637,23 +647,52 @@ def _day_arg(plan, day):
     return plan.time_index_device(np.asarray(day))
 
 
+def _joins(hows, how):
+    """``how`` comes from the same reduce-pack call as ``hows``: mean, min and max together, or up to MAX_OUT
+    per-step transforms of one family, bins contiguous (each starts where the previous one ends)."""
+    last = hows[-1]
+    if how in hows or isinstance(how, tuple) != isinstance(last, tuple):
+        return False
+    return not isinstance(how, tuple) or (how[0] == last[0] and len(hows) < N.MAX_OUT and
+                                          (how[0] != "bins" or last[2] == how[1]))
+
+
+def _step_params(hows):
+    """``ctb_pull_pack_daily_steps`` parameters of per-step transforms of one family, in plane order."""
+    if hows[0][0] == "bins":
+        return [h[1] for h in hows] + [hows[-1][2]]
+    return [p for h in hows for p in h[1:]]
+
+
 def _pull_daily(plan, src, dsts, d0, n):
-    """Queue ``ctb_pull_pack_daily`` for days d0 .. d0 + n - 1 of ``src`` into ``dsts`` ({how: device tensor
-    [>= n, n_packed_cells]}, all from one read).  A pageable host source is staged first: whole days are
-    copied into pinned buffers (those of the host path, two in turn) that the kernel then reads."""
+    """Queue ``ctb_pull_pack_daily`` (or ``ctb_pull_pack_daily_steps`` for per-step transforms) for days
+    d0 .. d0 + n - 1 of ``src`` into ``dsts`` ({how: device tensor [>= n, n_packed_cells]}, all from one read, hows
+    that :func:`_joins` accepts).  A pageable host source is staged first: whole days are copied into pinned
+    buffers (those of the host path, two in turn) that the kernel then reads."""
     dev = plan.device
     L = N.lib()
-    ops = 0
-    for how in dsts:
-        ops |= _DAILY_OP[how]
+    hows = list(dsts)
+    steps = isinstance(hows[0], tuple)
+    if steps:
+        pa, pp = _params_array("daily_steps", _step_params(hows))
+    else:
+        ops = 0
+        for how in hows:
+            ops |= _DAILY_OP[how]
 
     def call(x_ptr, day, t_begin, k, m):
         day_d = _day_arg(plan, day) if day is not None else None
-        ptrs = {h: C.c_void_p(t.data_ptr() + k * t.shape[1] * t.element_size()) for h, t in dsts.items()}
-        N.check(L.ctb_pull_pack_daily(
-            plan._h, C.c_void_p(x_ptr), src.dtype, int(src.stride), int(src.S),
-            C.c_void_p(day_d.data_ptr()) if day_d is not None else None, int(t_begin), int(m), ops,
-            ptrs.get("mean"), ptrs.get("min"), ptrs.get("max"), _stream_ptr(dev)))
+        day_p = C.c_void_p(day_d.data_ptr()) if day_d is not None else None
+        ptrs = {h: t.data_ptr() + k * t.shape[1] * t.element_size() for h, t in dsts.items()}
+        if steps:
+            N.check(L.ctb_pull_pack_daily_steps(
+                plan._h, C.c_void_p(x_ptr), src.dtype, int(src.stride), int(src.S), day_p, int(t_begin), int(m),
+                _STEP_OP[hows[0][0]], pp, int(pa.size), len(hows), (C.c_void_p * len(hows))(*ptrs.values()),
+                _stream_ptr(dev)))
+        else:
+            N.check(L.ctb_pull_pack_daily(
+                plan._h, C.c_void_p(x_ptr), src.dtype, int(src.stride), int(src.S), day_p, int(t_begin), int(m), ops,
+                *[C.c_void_p(ptrs[h]) if h in ptrs else None for h in ("mean", "min", "max")], _stream_ptr(dev)))
         if not src.on_device:
             TRANSFER_BYTES["h2d"] += m * src.S * plan.info["n_pieces_distinct"] * 4 * src.itemsize
 
@@ -690,15 +729,17 @@ def _pull_daily(plan, src, dsts, d0, n):
 def aggregate_daily(plan, srcs, kind="identity", params=(), n_out=1, variant=N.VARIANT_AUTO, groups=None,
                     host_out=None, doy=None):
     """Deferred daily reductions of sub-daily data -> CUDA tensor [n_out, R, T] (with ``groups``:
-    [n_out, R, n_groups]).  ``srcs``: 1 or 2 (:class:`DailySource`, how).  Each chunk of days is
-    reduce-packed by ``ctb_pull_pack_daily`` into packed daily planes (float64 for the mean, the source
-    dtype for min / max; the plan is built for that element size) and aggregated by the compact-plan
-    launch; sources that read the same steps -- the daily minimum and maximum of one variable -- come from
-    one call.  ``host_out``: as :func:`aggregate_host`."""
+    [n_out, R, n_groups]).  ``srcs``: 1 or 2 (:class:`DailySource`, how), or -- ``kind="identity"`` with
+    n_out > 1 -- the n_out per-step transforms of one fused request.  Each chunk of days is reduce-packed by
+    ``ctb_pull_pack_daily`` / ``ctb_pull_pack_daily_steps`` into packed daily planes (the source dtype for
+    min / max, float64 otherwise; the plan is built for that element size) and aggregated by the compact-plan
+    launch, or by one identity launch per plane into out[j]; sources that read the same steps -- the daily
+    minimum and maximum of one variable, the thresholds or bins of one fused request -- come from one call.
+    ``host_out``: as :func:`aggregate_host`."""
     calls = []          # [(DailySource, {how: plane index})]
     for i, (src, how) in enumerate(srcs):
         for c in calls:
-            if c[0].same_read(src) and how not in c[1]:
+            if c[0].same_read(src) and _joins(list(c[1]), how):
                 c[1][how] = i
                 break
         else:
@@ -708,9 +749,9 @@ def aggregate_daily(plan, srcs, kind="identity", params=(), n_out=1, variant=N.V
         for src, planes in calls:
             _pull_daily(plan, src, {h: bufs[i] for h, i in planes.items()}, t0, n)
 
-    itemsize = 8 if srcs[0][1] == "mean" else srcs[0][0].itemsize
-    out, filled = _aggregate_packed(plan, pack, len(srcs), itemsize, srcs[0][0].T, kind, params, n_out, variant,
-                                    groups, None, host_out[0] if host_out is not None else None, doy=doy)
+    out, filled = _aggregate_packed(plan, pack, len(srcs), srcs[0][0].out_bytes, srcs[0][0].T, kind, params, n_out,
+                                    variant, groups, None, host_out[0] if host_out is not None else None, doy=doy,
+                                    per_plane=kind == "identity" and n_out > 1)
     if host_out is not None:
         host_out[1] = filled
     return out
@@ -740,7 +781,7 @@ def daily_device(var, dev):
     """A deferred daily variable evaluated for the whole grid by ``ctb_pull_pack_daily``: CUDA tensor
     [days, lat, lon] with the variable's lat / lon takes applied."""
     src = DailySource(var)
-    es = 8 if src.how == "mean" else src.itemsize
+    es = src.out_bytes
     plan = _full_grid_plan(src.nlat_phys, src.nlon_phys, es, dev)
     o = torch.empty((src.T, plan.info["n_packed_cells"]), dtype=torch.float32 if es == 4 else torch.float64,
                     device=dev)

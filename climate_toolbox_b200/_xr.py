@@ -51,7 +51,9 @@ class Deferred:
 
     kind   : "poly" | "bins" | "rcspline" | "edd" | "gdd" | "reindex" (pointwise lat/lon gather,
              params = (materialise closure, origin Dataset)) | "daily" (daily reduction of a sub-daily
-             (time, lat, lon) source, params = (how, steps per day, first step, physical day of every day))
+             (time, lat, lon) source, params = (how, steps per day, first step, physical day of every day);
+             how = "mean" | "min" | "max", or the daily mean of a per-step transform: ("edd", e) |
+             ("gdd", lo, hi) | ("bins", lo, hi))
     params : tuple of floats (poly: (offset, power); bins: (offset, lo, hi); rcspline: (offset, term,
              k_1, ..., k_n); edd: (threshold,); gdd: (threshold_low, threshold_high))
     sources: tuple of :class:`Variable` (poly / bins / rcspline: (tas,); edd/gdd: (tasmin, tasmax))
@@ -105,7 +107,7 @@ class Variable:
     def dtype(self):
         if self.deferred is not None:
             d = self.deferred
-            return d.sources[0].dtype if d.kind == "daily" and d.params[0] != "mean" else np.dtype("float64")
+            return d.sources[0].dtype if d.kind == "daily" and d.params[0] in ("min", "max") else np.dtype("float64")
         d = self._data.dtype
         return np.dtype(str(d).replace("torch.", "")) if _is_torch(self._data) else d
 

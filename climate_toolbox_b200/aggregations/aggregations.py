@@ -118,7 +118,7 @@ class _DailyView:
         self.stride = self.src.stride
         self.data2d = self.src.x
         self.on_device = self.src.on_device
-        self.elem_bytes = 8 if self.how == "mean" else self.src.itemsize
+        self.elem_bytes = self.src.out_bytes
 
     def same_geometry(self, other):
         return (isinstance(other, _DailyView) and self.T == other.T and self.elem_bytes == other.elem_bytes
@@ -135,15 +135,24 @@ def _view(var):
     return _DailyView(var) if _is_daily(var) else _GridView(var)
 
 
+def _step_family(var):
+    """"edd" / "gdd" / "bins" for the daily mean of a per-step transform of sub-daily data
+    (``transformations.subdaily_*``), else None."""
+    return var.deferred.params[0][0] if _is_daily(var) and isinstance(var.deferred.params[0], tuple) else None
+
+
+def _same_steps(a, b):
+    """Two deferred daily variables read the same steps of the same buffer."""
+    pa, pb = a.deferred.params, b.deferred.params
+    return (pa[1:3] == pb[1:3] and np.array_equal(pa[3], pb[3]) and
+            _same_source(a.deferred.sources[0], b.deferred.sources[0]))
+
+
 def _same_source(a, b):
     """Two transform sources read the same data: the same buffer and takes, and for daily reductions also
     the same ``how``, steps and days."""
     if _is_daily(a) or _is_daily(b):
-        if not (_is_daily(a) and _is_daily(b)):
-            return False
-        pa, pb = a.deferred.params, b.deferred.params
-        return (pa[:3] == pb[:3] and np.array_equal(pa[3], pb[3]) and
-                _same_source(a.deferred.sources[0], b.deferred.sources[0]))
+        return _is_daily(a) and _is_daily(b) and a.deferred.params[0] == b.deferred.params[0] and _same_steps(a, b)
     return (a.physical is b.physical and a.dims == b.dims and
             all(_eq(a.takes.get(d), b.takes.get(d)) for d in a.dims))
 
@@ -252,11 +261,24 @@ def _group_requests(reqs):
     the data (config 3/4).  A bin (offset, lo, hi) joins a group of bins whose
     last edge is lo: the group's params are (offset, e_0, ..., e_n).  A spline term
     (offset, i, k_1, ..., k_n) joins a group of the same offset and knots whose
-    terms run first .. i - 1: the group keeps the params (offset, first, k_1, ..., k_n)."""
+    terms run first .. i - 1: the group keeps the params (offset, first, k_1, ..., k_n).
+    Per-step transforms of sub-daily data (identity requests of one ``_step_family``) that read the same steps
+    fuse too, bins when contiguous: up to MAX_OUT planes from one reduce-pack call, each aggregated on its own
+    (the group's "step" names the family, its "srcs" hold every member)."""
     groups = []
     for name, kind, params, srcs in reqs:
         placed = False
+        step = _step_family(srcs[0]) if kind == "identity" else None
         for g in groups:
+            if step is not None or g["step"] is not None:
+                last = g["srcs"][-1]
+                if (step == g["step"] and len(g["names"]) < N.MAX_OUT and _same_steps(last, srcs[0]) and
+                        (step != "bins" or last.deferred.params[0][2] == srcs[0].deferred.params[0][1])):
+                    g["names"].append(name)
+                    g["srcs"].append(srcs[0])
+                    placed = True
+                    break
+                continue
             same_src = len(g["srcs"]) == len(srcs) and all(_same_source(a, b) for a, b in zip(g["srcs"], srcs))
             if not same_src or g["kind"] != kind or len(g["names"]) >= N.MAX_OUT:
                 continue
@@ -273,7 +295,7 @@ def _group_requests(reqs):
             placed = True
             break
         if not placed:
-            groups.append({"names": [name], "kind": kind, "params": tuple(params), "srcs": srcs})
+            groups.append({"names": [name], "kind": kind, "params": tuple(params), "srcs": list(srcs), "step": step})
     return groups
 
 
@@ -314,7 +336,7 @@ def _aggregate_core(ds, variables, aggwt, agglev, weights, backup_aggwt, variant
                     time_dim, v0.out_dims_template))
             cell_gate, doy = _season_gate(season_mask, ds, lat, lon, v0, time_dim)
         plan = E.get_plan(grid, weights, aggwt, agglev, backup_aggwt,
-                          stage_bytes=len(views) * v0.elem_bytes, device=dev,
+                          stage_bytes=(1 if g["step"] else len(views)) * v0.elem_bytes, device=dev,
                           smem_budget=smem_budget, compact=compact, elem_bytes=v0.elem_bytes,
                           trusted=trusted_weights, cell_gate=cell_gate)
         n_out = len(g["names"])

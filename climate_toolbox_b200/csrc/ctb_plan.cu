@@ -1042,6 +1042,201 @@ extern "C" int ctb_pull_pack_daily(const ctb_plan* P, const void* x, int dtype, 
   return CTB_OK;
 }
 
+// Per-step transforms of sub-daily sources, reduced to daily means in the same read: the addressing, the loads
+// in flight and the plane layout of subdaily_pack_kernel, with NOUT float64 planes of f_j averaged over the
+// day's non-NaN steps.  The threshold and edge decisions are those of the aggregation kernels (CtbTr packed by
+// ctb_pack_transform): fp64 comparisons for double sources; for float sources the fp32 comparisons against
+// up / dn, which decide every float -- infinities included -- as the fp64 rule does (NaN steps never get here).
+//   EDD:  f = x > e ? x - e : 0                                    (= max(x - e, 0): x - e > 0 <=> x > e)
+//   GDD:  f = x > lo ? (x >= hi ? hi - lo : x - lo) : 0           (= min(max(x - lo, 0), hi - lo): rounding
+//         is monotone, so x < hi gives fl(x - lo) <= fl(hi - lo) and x >= hi the reverse; +inf gives hi - lo)
+//   BINS: a count per bin (ctb_bins_in), divided by the count of valid steps
+namespace {
+struct StepDst {
+  double2* p[CTB_MAX_OUT];
+};
+
+// (256, 2): at most 128 registers, which every instantiation fits (the largest uses 127); without the bound
+// ptxas spills 8 bytes around the division's slow path in one of them
+template <typename T, int OP, int NOUT>
+__global__ void __launch_bounds__(256, 2) subdaily_steps_kernel(
+    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
+    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, const CtbTr tr, StepDst dst) {
+  constexpr int C = 16 / sizeof(T);   // cells per 16-byte unit
+  constexpr int U = 8;                // step loads in flight
+  constexpr bool F32 = sizeof(T) == 4;
+  double w[NOUT];                     // GDD: hi - lo of every pair
+#pragma unroll
+  for (int j = 0; j < NOUT; ++j) w[j] = OP == CTB_STEP_GDD ? tr.a[2 * j + 1] - tr.a[2 * j] : 0.0;
+  const int64_t n_work = (int64_t)n_units * n_days;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_work; i += (int64_t)gridDim.x * blockDim.x) {
+    const int u = (int)(i % n_units);
+    const int d = (int)(i / n_units);
+    const int p = __ldg(pack_src + u / halves);
+    if (p < 0) continue;                       // alignment padding of the packed plane: never read
+    const int64_t step0 = (int64_t)(day ? __ldg(day + t_begin + d) : t_begin + d) * S;
+    const uint4* s = src + step0 * stride16 + (int64_t)p * halves + (u % halves);
+    double sum[C][NOUT];
+    int hits[C][NOUT];
+    int cnt[C];
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+      cnt[c] = 0;
+#pragma unroll
+      for (int j = 0; j < NOUT; ++j) {
+        sum[c][j] = 0.0;
+        hits[c][j] = 0;
+      }
+    }
+    for (int h0 = 0; h0 < S; h0 += U) {
+      uint4 v[U];
+#pragma unroll
+      for (int k = 0; k < U; ++k)
+        if (h0 + k < S)
+          asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
+                       : "=r"(v[k].x), "=r"(v[k].y), "=r"(v[k].z), "=r"(v[k].w)
+                       : "l"(s + (int64_t)(h0 + k) * stride16));
+#pragma unroll
+      for (int k = 0; k < U; ++k)
+        if (h0 + k < S) {
+          T e[C];
+          unit_get(v[k], e);
+#pragma unroll
+          for (int c = 0; c < C; ++c) {
+            if (!(e[c] == e[c])) continue;   // NaN step: skipped
+            ++cnt[c];
+            const double x = (double)e[c];
+            if constexpr (OP == CTB_STEP_BINS) {
+              bool in[NOUT];
+              if constexpr (F32) ctb_bins_in_f32<NOUT>(tr, e[c], in); else ctb_bins_in<NOUT>(tr, x, in);
+#pragma unroll
+              for (int j = 0; j < NOUT; ++j) hits[c][j] += in[j];
+            } else if constexpr (OP == CTB_STEP_EDD) {
+#pragma unroll
+              for (int j = 0; j < NOUT; ++j) {
+                const bool above = F32 ? (float)e[c] > tr.dn[j] : x > tr.a[j];
+                sum[c][j] = __dadd_rn(sum[c][j], above ? __dsub_rn(x, tr.a[j]) : 0.0);
+              }
+            } else {
+#pragma unroll
+              for (int j = 0; j < NOUT; ++j) {
+                const bool above = F32 ? (float)e[c] > tr.dn[2 * j] : x > tr.a[2 * j];
+                const bool top = F32 ? (float)e[c] >= tr.up[2 * j + 1] : x >= tr.a[2 * j + 1];
+                const double f = top ? w[j] : __dsub_rn(x, tr.a[2 * j]);
+                sum[c][j] = __dadd_rn(sum[c][j], above ? f : 0.0);
+              }
+            }
+          }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < NOUT; ++j) {
+#pragma unroll
+      for (int c = 0; c < C; c += 2) {
+        const double s0 = OP == CTB_STEP_BINS ? (double)hits[c][j] : sum[c][j];
+        const double s1 = OP == CTB_STEP_BINS ? (double)hits[c + 1][j] : sum[c + 1][j];
+        dst.p[j][((int64_t)d * n_units + u) * (C / 2) + c / 2] =
+            make_double2(__ddiv_rn(s0, (double)cnt[c]), __ddiv_rn(s1, (double)cnt[c + 1]));
+      }
+    }
+  }
+}
+}  // namespace
+
+extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int dtype, int64_t stride,
+                                         int steps_per_day, const int32_t* day_index, int64_t t_begin,
+                                         int64_t n_days, int step_op, const double* params, int n_params, int n_out,
+                                         double* const* dst, void* stream) {
+  if (!P || !x || n_days < 0 || n_days >= (1ll << 31) || t_begin < 0 || !P->compact) {
+    ctb_set_error("ctb_pull_pack_daily_steps: needs a compact plan, a non-null source and 0 <= n_days < 2^31");
+    return CTB_ERR_INVALID;
+  }
+  if (dtype != CTB_F32 && dtype != CTB_F64) { ctb_set_error("dtype=%d unsupported", dtype); return CTB_ERR_INVALID; }
+  if (steps_per_day < 1) {
+    ctb_set_error("ctb_pull_pack_daily_steps: steps_per_day=%d, needs >= 1", steps_per_day);
+    return CTB_ERR_INVALID;
+  }
+  if (step_op != CTB_STEP_EDD && step_op != CTB_STEP_GDD && step_op != CTB_STEP_BINS) {
+    ctb_set_error("ctb_pull_pack_daily_steps: step_op=%d, needs CTB_STEP_EDD, GDD or BINS", step_op);
+    return CTB_ERR_INVALID;
+  }
+  if (n_out < 1 || n_out > CTB_MAX_OUT) {
+    ctb_set_error("ctb_pull_pack_daily_steps: n_out=%d out of range 1..%d", n_out, CTB_MAX_OUT);
+    return CTB_ERR_INVALID;
+  }
+  const int need = step_op == CTB_STEP_EDD ? n_out : step_op == CTB_STEP_GDD ? 2 * n_out : n_out + 1;
+  if (n_params != need || !params) {
+    ctb_set_error("ctb_pull_pack_daily_steps: step_op %d with n_out=%d needs %d params, got %d", step_op, n_out,
+                  need, n_params);
+    return CTB_ERR_INVALID;
+  }
+  for (int j = 0; j < n_params && step_op != CTB_STEP_BINS; ++j) {
+    if (!std::isfinite(params[j]) || (step_op == CTB_STEP_GDD && j % 2 == 1 && !(params[j - 1] < params[j]))) {
+      ctb_set_error("ctb_pull_pack_daily_steps: thresholds must be finite, with lo < hi in every GDD pair: "
+                    "param %d is %g", j, params[j]);
+      return CTB_ERR_INVALID;
+    }
+  }
+  CtbTr tr;
+  int rc;
+  if (step_op == CTB_STEP_BINS) {
+    double b[CTB_MAX_OUT + 2] = {0.0};   // offset 0, then the edges
+    std::copy(params, params + n_params, b + 1);
+    rc = ctb_pack_transform(CTB_TR_BINS, b, n_params + 1, n_out, &tr);
+  } else {
+    rc = ctb_pack_transform(step_op == CTB_STEP_EDD ? CTB_TR_EDD : CTB_TR_GDD, params, n_params, n_out, &tr);
+  }
+  if (rc != CTB_OK) return rc;
+  if (!dst) { ctb_set_error("ctb_pull_pack_daily_steps: dst is null"); return CTB_ERR_INVALID; }
+  StepDst planes{};
+  for (int j = 0; j < n_out; ++j) {
+    if (!dst[j]) { ctb_set_error("ctb_pull_pack_daily_steps: dst[%d] is null", j); return CTB_ERR_INVALID; }
+    planes.p[j] = reinterpret_cast<double2*>(dst[j]);
+  }
+  if (P->elem_bytes != 8) {
+    ctb_set_error("ctb_pull_pack_daily_steps: the planes are float64, the plan was built for %d-byte elements",
+                  P->elem_bytes);
+    return CTB_ERR_INVALID;
+  }
+  const int64_t es = dtype == CTB_F32 ? 4 : 8;
+  const int64_t phys_ncell = (int64_t)P->nlat_phys * P->nlon_phys;
+  bool aligned = (stride * es) % 16 == 0 && (uintptr_t)x % 16 == 0 && phys_ncell % CTB_PIECE == 0;
+  for (int j = 0; j < n_out; ++j) aligned = aligned && (uintptr_t)dst[j] % 16 == 0;
+  if (!aligned) {
+    ctb_set_error("ctb_pull_pack_daily_steps: planes must be 16-byte aligned and hold a multiple of 4 gridcells");
+    return CTB_ERR_UNSUPPORTED;
+  }
+  if (n_days == 0) return CTB_OK;
+  CtbDeviceGuard guard(P->device);
+  if (guard.err != cudaSuccess) { ctb_set_error("cudaSetDevice(%d) failed: %s", P->device, cudaGetErrorString(guard.err)); return CTB_ERR_CUDA; }
+  const int halves = (int)(es / 4);
+  const int n_units = (int)(P->ncell / CTB_PIECE) * halves;
+  const int64_t n_work = (int64_t)n_units * n_days;
+  const unsigned grid = (unsigned)std::min<int64_t>((n_work + 255) / 256, 148 * 32);
+  const cudaStream_t st = (cudaStream_t)stream;
+  auto go = [&](auto tag, auto op, auto nout) {
+    subdaily_steps_kernel<decltype(tag), decltype(op)::value, decltype(nout)::value><<<grid, 256, 0, st>>>(
+        static_cast<const uint4*>(x), stride * es / 16, steps_per_day, day_index, t_begin, (int)n_days,
+        P->d_pack_src, n_units, halves, tr, planes);
+  };
+  auto by_nout = [&](auto tag, auto op) {
+    switch (n_out) {
+      case 1: go(tag, op, std::integral_constant<int, 1>{}); break;
+      case 2: go(tag, op, std::integral_constant<int, 2>{}); break;
+      case 3: go(tag, op, std::integral_constant<int, 3>{}); break;
+      default: go(tag, op, std::integral_constant<int, 4>{}); break;
+    }
+  };
+  auto by_op = [&](auto tag) {
+    if (step_op == CTB_STEP_EDD) by_nout(tag, std::integral_constant<int, CTB_STEP_EDD>{});
+    else if (step_op == CTB_STEP_GDD) by_nout(tag, std::integral_constant<int, CTB_STEP_GDD>{});
+    else by_nout(tag, std::integral_constant<int, CTB_STEP_BINS>{});
+  };
+  if (dtype == CTB_F32) by_op(float{}); else by_op(double{});
+  CTB_LAUNCH_CHECK();
+  return CTB_OK;
+}
+
 // ---------------------------------------------------------------------------
 // Fingerprint of a host buffer for the plan cache's fast path: 8 independent polynomial lanes
 // h_j = h_j * P + word (mod 2^64, P odd) over the 64-bit words j, j+8, ..., folded with a second

@@ -12,10 +12,10 @@ import numpy as np
 import torch
 
 from .._xr import DataArray, Dataset, Deferred, Variable, from_any, to_like
-from ..utils.utils import remove_leap_days, convert_kelvin_to_celsius  # noqa: F401
+from ..utils.utils import _resample, remove_leap_days, convert_kelvin_to_celsius  # noqa: F401
 
-__all__ = ["snyder_edd", "snyder_gdd", "validate_edd_snyder_agriculture", "tas_poly", "tas_bins", "tas_rcspline",
-           "ordinal"]
+__all__ = ["snyder_edd", "snyder_gdd", "subdaily_edd", "subdaily_gdd", "subdaily_bins",
+           "validate_edd_snyder_agriculture", "tas_poly", "tas_bins", "tas_rcspline", "ordinal"]
 
 
 def _source(da):
@@ -87,6 +87,77 @@ def snyder_gdd(tasmin, tasmax, threshold_low, threshold_high, check=True):
     var = Variable(smin.dims, None, attrs, None,
                    Deferred("gdd", (float(threshold_low), float(threshold_high)), (smin, smax)))
     return DataArray._wrap(var, tasmax._coords, tasmax.name)
+
+
+_SUBDAILY_RULES = """
+    ``tas``: a sub-daily DataArray over ``(time, lat, lon)`` whose time axis meets the rules of
+    ``utils.resample_daily`` (``ValueError`` otherwise), with a ``units`` attribute (``AttributeError``
+    otherwise); thresholds and edges are in those units.  Each step is widened to float64 first; NaN steps are
+    skipped, and the daily value is the sum of ``f`` over the day's other steps, in step order with float64
+    adds, divided by their count (NaN for a day without one) -- ``f(tas).resample(time="1D").mean()``.  The
+    result is deferred and daily (``time`` as ``datetime64[D]``): the transform runs on the GPU while the
+    referenced gridcells are packed for aggregation, so the sub-daily grid of ``f`` is never built.  It
+    composes with ``remove_leap_days``, ``time_groups=``, ``season_mask=`` and
+    ``weighted_aggregate_grid_to_regions_multi``; ``.values`` computes it for the whole grid.  Up to 4
+    thresholds (pairs, bins) of one ``tas`` aggregated together come from one read of the source."""
+
+
+def _finite(*values):
+    v = [float(x) for x in values]
+    if not np.isfinite(v).all():
+        raise ValueError("thresholds must be finite, got {}".format(values))
+    return v
+
+
+def subdaily_edd(tas, threshold):
+    """Exceedance degree days from sub-daily data: the daily mean of ``max(tas - threshold, 0)`` per step, in
+    degree days (``units = "degreedays_{threshold}{units}"``, as :func:`snyder_edd`).
+    """
+    tas = from_any(tas)
+    e, = _finite(threshold)
+    return _resample(tas, ("edd", e), {"units": "degreedays_{}{}".format(threshold, tas.units)})
+
+
+def subdaily_gdd(tas, threshold_low, threshold_high):
+    """Growing degree days from sub-daily data: the daily mean of ``min(max(tas - lo, 0), hi - lo)`` per step,
+    ``hi - lo`` one float64 value (so ``+inf`` gives ``hi - lo``); in real arithmetic ``EDD(lo) - EDD(hi)``.
+    ``lo < hi``, both finite (``ValueError`` otherwise); units as :func:`snyder_gdd`.
+    """
+    tas = from_any(tas)
+    lo, hi = _finite(threshold_low, threshold_high)
+    if not lo < hi:
+        raise ValueError("threshold_low {} must be below threshold_high {}".format(threshold_low, threshold_high))
+    return _resample(tas, ("gdd", lo, hi),
+                     {"units": "degreedays_{}-{}{}".format(threshold_low, threshold_high, tas.units)})
+
+
+def subdaily_bins(tas, edges, varname="tas_bin"):
+    """Time per temperature bin from sub-daily data: one variable per bin ``[lo, hi)``, the fraction of the
+    day's valid steps with ``lo <= tas < hi`` (times 24 for hourly data: hours), ``units = "days"``, so that
+    annual sums are days in the bin.  ``edges``: K+1 strictly increasing values for K bins, ``-inf`` allowed
+    first and ``+inf`` last (as :func:`tas_bins`: ``+inf`` lies in no bin, ``-inf`` in a first bin open to
+    ``-inf``).  ``varname``: a prefix (variables ``"{varname}_{k}"``) or a list of K names.  Returns a Dataset.
+    """
+    e = _bin_edges(edges)
+    K = e.size - 1
+    names = ["{}_{}".format(varname, k) for k in range(K)] if isinstance(varname, str) else list(varname)
+    if len(names) != K:
+        raise ValueError("{} edges give {} bins, but {} names were given".format(e.size, K, len(names)))
+    tas = from_any(tas)
+    units = tas.units
+    out = Dataset()
+    for lo, hi, name in zip(e[:-1], e[1:], names):
+        attrs = {"units": "days", "bin_lower": float(lo), "bin_upper": float(hi),
+                 "long_title": "Fraction of the day's steps with {} in [{:g}, {:g}) {}".format(
+                     tas.name or "tas", lo, hi, units)}
+        da = _resample(tas, ("bins", float(lo), float(hi)), attrs)
+        out._vars[name] = da.variable
+        out._coords.update(da._coords)
+    return out
+
+
+for _f in (subdaily_edd, subdaily_gdd, subdaily_bins):
+    _f.__doc__ += _SUBDAILY_RULES
 
 
 def validate_edd_snyder_agriculture(ds, thresholds):

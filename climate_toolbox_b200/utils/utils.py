@@ -131,8 +131,11 @@ def resample_daily(ds, how="mean"):
     ``time`` as the day (``datetime64[D]``); other variables without ``time`` are kept.  The reduction runs
     on the GPU per gridcell while the referenced gridcells are packed for aggregation, so the daily grid is
     never built: the result feeds ``tas_poly``, ``tas_bins``, ``tas_rcspline``, ``snyder_edd`` /
-    ``snyder_gdd``, ``remove_leap_days`` and ``weighted_aggregate_grid_to_regions`` directly, and
-    ``.values`` computes it for the whole grid.
+    ``snyder_gdd``, ``remove_leap_days`` and ``weighted_aggregate_grid_to_regions`` (with ``time_groups=``,
+    ``season_mask=``) and ``weighted_aggregate_grid_to_regions_multi`` directly, and ``.values`` computes it
+    for the whole grid.  Transforms that are nonlinear in each step -- degree days and time per temperature
+    bin from the steps themselves -- are ``transformations.subdaily_edd`` / ``subdaily_gdd`` /
+    ``subdaily_bins``, reduced in the same way.
 
     * ``"mean"``: each step widened to float64 and summed in step order, NaN steps skipped, divided by the
       number of non-NaN steps (NaN for a day without one); float64.
@@ -142,6 +145,12 @@ def resample_daily(ds, how="mean"):
     ``NotImplementedError``."""
     if how not in _DAILY_HOW:
         raise ValueError("how={!r}: expected one of {}".format(how, _DAILY_HOW))
+    return _resample(ds, how)
+
+
+def _resample(ds, how, attrs=None):
+    """:func:`resample_daily` for any ``how`` of the deferred daily record (``_xr.Deferred``); ``attrs``: the
+    attributes of every daily variable (default: the source's plus ``cell_methods``)."""
     like = ds
     ds = from_any(ds)
     single = isinstance(ds, DataArray)
@@ -175,9 +184,12 @@ def resample_daily(ds, how="mean"):
                 raise NotImplementedError("resample_daily: {!r} selects time steps out of physical order".format(name))
             t0 = int(pos[0]) if len(pos) else 0
         src = Variable(var.dims, var.physical, var.attrs, takes)
-        attrs = dict(var.attrs)
-        attrs["cell_methods"] = "time: {}".format(how)
-        out._vars[name] = Variable(var.dims, None, attrs, None,
+        if attrs is None:
+            a = dict(var.attrs)
+            a["cell_methods"] = "time: {}".format(how)
+        else:
+            a = dict(attrs)
+        out._vars[name] = Variable(var.dims, None, a, None,
                                    Deferred("daily", (how, S, t0, np.arange(len(days), dtype=np.int64)), (src,)))
     if single:
         name = next(iter(out._vars))

@@ -279,6 +279,23 @@ int ctb_pull_pack_daily(const ctb_plan* plan, const void* x, int dtype, int64_t 
                         const int32_t* day_index, int64_t t_begin, int64_t n_days, int ops, void* dst_mean,
                         void* dst_min, void* dst_max, void* stream);
 
+/* Per-step transforms of sub-daily sources: the same read as ctb_pull_pack_daily, with a function f_j applied to
+ * every step before the day's mean.  Each step is widened to float64; NaN steps are skipped; output j of day d is
+ * the sum of f_j over the day's non-NaN steps, in step order with plain float64 adds, divided by their count
+ * (NaN for a day without one).  step_op and params (n_out = 1..4 outputs, all from one read):
+ *   EDD  {e_1..e_n}, n_params = n_out:          f = max(x - e, 0)                     (e finite)
+ *   GDD  {lo_1, hi_1, ...}, n_params = 2 n_out: f = min(max(x - lo, 0), hi - lo)      (lo < hi, both finite;
+ *                                               hi - lo is one float64 value, so x = +inf gives hi - lo)
+ *   BINS {e_0..e_n}, n_params = n_out + 1:      f = 1 if e_j <= x < e_{j+1}, else 0   (edges strictly
+ *                                               increasing, -inf only first, +inf only last; +inf in no bin)
+ * dst: HOST array of n_out DEVICE float64 planes [n_days][n_packed_cells]; the plan needs elem_bytes 8.
+ * Errors as ctb_pull_pack_daily: a non-compact plan, an unknown step_op, an n_out or n_params out of range, bad
+ * thresholds or edges, or a null destination is CTB_ERR_INVALID; misaligned planes CTB_ERR_UNSUPPORTED. */
+enum { CTB_STEP_EDD = 1, CTB_STEP_GDD = 2, CTB_STEP_BINS = 3 };
+int ctb_pull_pack_daily_steps(const ctb_plan* plan, const void* x, int dtype, int64_t stride, int steps_per_day,
+                              const int32_t* day_index, int64_t t_begin, int64_t n_days, int step_op,
+                              const double* params, int n_params, int n_out, double* const* dst, void* stream);
+
 /* rows of a pitched DEVICE array -> pitched HOST (pinned) array, one asynchronous 2-D copy on `stream`:
  * the host path returns out[:, :, t0:t1] of a finished time chunk while the next chunk is in flight */
 int ctb_copy_rows_to_host(void* dst, size_t dst_pitch, const void* src, size_t src_pitch, size_t width_bytes,
