@@ -859,33 +859,67 @@ __global__ void __launch_bounds__(256) pull_pack_kernel(const uint4* __restrict_
       if (d0 + k < T) dst[(int64_t)(d0 + k) * n_units + u] = v[k];
   }
 }
+
+// The launch shape of the pull kernels: one thread per 16-byte unit of a packed plane and work row.
+struct PullShape {
+  int64_t es;        // bytes per source element
+  int64_t stride16;  // the source's plane stride in 16-byte units
+  int halves;        // 16-byte units per 4-cell piece
+  int n_units;       // 16-byte units per packed plane
+  unsigned grid;
+};
+
+// The checks the three pull entry points share, in this order: a compact plan, a source, 0 <= n_days < 2^31
+// and t_begin >= 0, a float32 or float64 dtype, and 16-byte aligned source planes on a grid of whole 4-cell
+// pieces (a ragged last piece would be read past the plane).  Each entry checks its destinations itself.
+int pull_check(const char* fn, const ctb_plan* P, const void* x, int dtype, int64_t stride, int64_t t_begin,
+               int64_t n_days, int64_t rows, PullShape* sh) {
+  if (!P || !P->compact) { ctb_set_error("%s: needs a compact plan", fn); return CTB_ERR_INVALID; }
+  if (!x) { ctb_set_error("%s: the source is null", fn); return CTB_ERR_INVALID; }
+  if (n_days < 0 || n_days >= (1ll << 31) || t_begin < 0) {
+    ctb_set_error("%s: needs 0 <= T < 2^31 and t_begin >= 0, got T=%lld, t_begin=%lld", fn, (long long)n_days,
+                  (long long)t_begin);
+    return CTB_ERR_INVALID;
+  }
+  if (dtype != CTB_F32 && dtype != CTB_F64) {
+    ctb_set_error("%s: dtype=%d unsupported", fn, dtype);
+    return CTB_ERR_INVALID;
+  }
+  sh->es = dtype == CTB_F32 ? 4 : 8;
+  if ((stride * sh->es) % 16 != 0 || (uintptr_t)x % 16 != 0 || (int64_t)P->nlat_phys * P->nlon_phys % CTB_PIECE != 0) {
+    ctb_set_error("%s: planes must be 16-byte aligned and hold a multiple of 4 gridcells", fn);
+    return CTB_ERR_UNSUPPORTED;
+  }
+  sh->stride16 = stride * sh->es / 16;
+  sh->halves = (int)(sh->es / 4);
+  sh->n_units = (int)(P->ncell / CTB_PIECE) * sh->halves;
+  sh->grid = (unsigned)std::min<int64_t>(((int64_t)sh->n_units * rows + 255) / 256, 148 * 32);
+  return CTB_OK;
+}
+
+// launch() enqueues the kernel on the plan's device; nothing is launched for zero days
+template <typename F>
+int pull_launch(const ctb_plan* P, int64_t n_days, F&& launch) {
+  if (n_days == 0) return CTB_OK;
+  CtbDeviceGuard guard(P->device);
+  if (guard.err != cudaSuccess) { ctb_set_error("cudaSetDevice(%d) failed: %s", P->device, cudaGetErrorString(guard.err)); return CTB_ERR_CUDA; }
+  if (int rc = launch()) return rc;
+  CTB_LAUNCH_CHECK();
+  return CTB_OK;
+}
 }  // namespace
 
 extern "C" int ctb_pull_pack(const ctb_plan* P, const void* x, int dtype, int64_t stride,
                              const int32_t* time_index, int64_t t_begin, int64_t T, void* dst, void* stream) {
-  if (!P || !x || (!dst && T > 0) || T < 0 || T >= (1ll << 31) || !P->compact) {
-    ctb_set_error("ctb_pull_pack: needs a compact plan and non-null buffers");
-    return CTB_ERR_INVALID;
-  }
-  if (dtype != CTB_F32 && dtype != CTB_F64) { ctb_set_error("dtype=%d unsupported", dtype); return CTB_ERR_INVALID; }
-  const int64_t es = dtype == CTB_F32 ? 4 : 8;
-  const int64_t phys_ncell = (int64_t)P->nlat_phys * P->nlon_phys;
-  if ((stride * es) % 16 != 0 || (uintptr_t)x % 16 != 0 || phys_ncell % CTB_PIECE != 0) {
-    ctb_set_error("ctb_pull_pack: planes must be 16-byte aligned and hold a multiple of 4 gridcells");
-    return CTB_ERR_UNSUPPORTED;
-  }
-  if (T == 0) return CTB_OK;
-  CtbDeviceGuard guard(P->device);
-  if (guard.err != cudaSuccess) { ctb_set_error("cudaSetDevice(%d) failed: %s", P->device, cudaGetErrorString(guard.err)); return CTB_ERR_CUDA; }
-  const int halves = (int)(es / 4);
-  const int n_units = (int)(P->ncell / CTB_PIECE) * halves;
-  const int64_t n_work = (int64_t)n_units * ((T + 3) / 4);
-  const unsigned grid = (unsigned)std::min<int64_t>((n_work + 255) / 256, 148 * 32);
-  pull_pack_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
-      static_cast<const uint4*>(x), stride * es / 16, time_index, t_begin, (int)T, P->d_pack_src, n_units,
-      halves, static_cast<uint4*>(dst));
-  CTB_LAUNCH_CHECK();
-  return CTB_OK;
+  PullShape sh;
+  if (int rc = pull_check("ctb_pull_pack", P, x, dtype, stride, t_begin, T, (T + 3) / 4, &sh)) return rc;
+  if (!dst && T > 0) { ctb_set_error("ctb_pull_pack: dst is null"); return CTB_ERR_INVALID; }
+  return pull_launch(P, T, [&] {
+    pull_pack_kernel<<<sh.grid, 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint4*>(x), sh.stride16, time_index, t_begin, (int)T, P->d_pack_src, sh.n_units,
+        sh.halves, static_cast<uint4*>(dst));
+    return CTB_OK;
+  });
 }
 
 // ---------------------------------------------------------------- sub-daily ingest ---
@@ -914,11 +948,13 @@ __device__ __forceinline__ uint4 unit_put(const double (&e)[2]) {
                     (unsigned)__double2hiint(e[1]));
 }
 
-template <typename T, bool MEAN, bool EXT>
-__global__ void __launch_bounds__(256) subdaily_pack_kernel(
-    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
-    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, double2* __restrict__ dst_mean,
-    uint4* __restrict__ dst_min, uint4* __restrict__ dst_max) {
+// The step loop of both sub-daily kernels.  Item = one 16-byte unit u of a packed plane x one day d: step(e) gets
+// the C = 16 / sizeof(T) elements of each of the day's S steps, in step order, then item(d, u) stores the item's
+// results and resets the kernel's accumulators for the next item.  Padding units call neither.
+template <typename T, typename Step, typename Item>
+__device__ __forceinline__ void subdaily_step_loop(const uint4* src, int64_t stride16, int S, const int32_t* day,
+                                                   int64_t t_begin, int n_days, const int32_t* pack_src, int n_units,
+                                                   int halves, Step&& step, Item&& item) {
   constexpr int C = 16 / sizeof(T);   // cells per 16-byte unit
   constexpr int U = 8;                // step loads in flight
   const int64_t n_work = (int64_t)n_units * n_days;
@@ -929,15 +965,6 @@ __global__ void __launch_bounds__(256) subdaily_pack_kernel(
     if (p < 0) continue;                       // alignment padding of the packed plane: never read
     const int64_t step0 = (int64_t)(day ? __ldg(day + t_begin + d) : t_begin + d) * S;
     const uint4* s = src + step0 * stride16 + (int64_t)p * halves + (u % halves);
-    double sum[C];
-    int cnt[C];
-    T mn[C], mx[C];
-#pragma unroll
-    for (int c = 0; c < C; ++c) {
-      sum[c] = 0.0;
-      cnt[c] = 0;
-      mn[c] = mx[c] = (T)NAN;
-    }
     for (int h0 = 0; h0 < S; h0 += U) {
       uint4 v[U];
 #pragma unroll
@@ -951,44 +978,61 @@ __global__ void __launch_bounds__(256) subdaily_pack_kernel(
         if (h0 + k < S) {
           T e[C];
           unit_get(v[k], e);
-#pragma unroll
-          for (int c = 0; c < C; ++c) {
-            if (MEAN && e[c] == e[c]) { sum[c] = __dadd_rn(sum[c], (double)e[c]); ++cnt[c]; }
-            if (EXT) { mn[c] = ext_min(mn[c], e[c]); mx[c] = ext_max(mx[c], e[c]); }
-          }
+          step(e);
         }
     }
-    if (MEAN) {
-#pragma unroll
-      for (int c = 0; c < C; c += 2)
-        dst_mean[((int64_t)d * n_units + u) * (C / 2) + c / 2] =
-            make_double2(__ddiv_rn(sum[c], (double)cnt[c]), __ddiv_rn(sum[c + 1], (double)cnt[c + 1]));
-    }
-    if (EXT) {
-      if (dst_min) dst_min[(int64_t)d * n_units + u] = unit_put(mn);
-      if (dst_max) dst_max[(int64_t)d * n_units + u] = unit_put(mx);
-    }
+    item(d, u);
   }
 }
 
 template <typename T, bool MEAN, bool EXT>
-void launch_subdaily(unsigned grid, cudaStream_t st, const void* x, int64_t stride16, int S, const int32_t* day,
-                     int64_t t_begin, int n_days, const int32_t* pack_src, int n_units, int halves, void* dmean,
-                     void* dmin, void* dmax) {
-  subdaily_pack_kernel<T, MEAN, EXT><<<grid, 256, 0, st>>>(
-      static_cast<const uint4*>(x), stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
-      static_cast<double2*>(dmean), static_cast<uint4*>(dmin), static_cast<uint4*>(dmax));
+__global__ void __launch_bounds__(256) subdaily_pack_kernel(
+    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
+    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, double2* __restrict__ dst_mean,
+    uint4* __restrict__ dst_min, uint4* __restrict__ dst_max) {
+  constexpr int C = 16 / sizeof(T);
+  double sum[C];
+  int cnt[C];
+  T mn[C], mx[C];
+  auto reset = [&] {
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+      sum[c] = 0.0;
+      cnt[c] = 0;
+      mn[c] = mx[c] = (T)NAN;
+    }
+  };
+  reset();
+  subdaily_step_loop<T>(
+      src, stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
+      [&](const T (&e)[C]) {
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+          if (MEAN && e[c] == e[c]) { sum[c] = __dadd_rn(sum[c], (double)e[c]); ++cnt[c]; }
+          if (EXT) { mn[c] = ext_min(mn[c], e[c]); mx[c] = ext_max(mx[c], e[c]); }
+        }
+      },
+      [&](int d, int u) {
+        if (MEAN) {
+#pragma unroll
+          for (int c = 0; c < C; c += 2)
+            dst_mean[((int64_t)d * n_units + u) * (C / 2) + c / 2] =
+                make_double2(__ddiv_rn(sum[c], (double)cnt[c]), __ddiv_rn(sum[c + 1], (double)cnt[c + 1]));
+        }
+        if (EXT) {
+          if (dst_min) dst_min[(int64_t)d * n_units + u] = unit_put(mn);
+          if (dst_max) dst_max[(int64_t)d * n_units + u] = unit_put(mx);
+        }
+        reset();
+      });
 }
 }  // namespace
 
 extern "C" int ctb_pull_pack_daily(const ctb_plan* P, const void* x, int dtype, int64_t stride, int steps_per_day,
                                    const int32_t* day_index, int64_t t_begin, int64_t n_days, int ops,
                                    void* dst_mean, void* dst_min, void* dst_max, void* stream) {
-  if (!P || !x || n_days < 0 || n_days >= (1ll << 31) || t_begin < 0 || !P->compact) {
-    ctb_set_error("ctb_pull_pack_daily: needs a compact plan, a non-null source and 0 <= n_days < 2^31");
-    return CTB_ERR_INVALID;
-  }
-  if (dtype != CTB_F32 && dtype != CTB_F64) { ctb_set_error("dtype=%d unsupported", dtype); return CTB_ERR_INVALID; }
+  PullShape sh;
+  if (int rc = pull_check("ctb_pull_pack_daily", P, x, dtype, stride, t_begin, n_days, n_days, &sh)) return rc;
   if (steps_per_day < 1) {
     ctb_set_error("ctb_pull_pack_daily: steps_per_day=%d, needs >= 1", steps_per_day);
     return CTB_ERR_INVALID;
@@ -1002,49 +1046,38 @@ extern "C" int ctb_pull_pack_daily(const ctb_plan* P, const void* x, int dtype, 
     ctb_set_error("ctb_pull_pack_daily: every requested op needs a destination");
     return CTB_ERR_INVALID;
   }
-  const int64_t es = dtype == CTB_F32 ? 4 : 8;
   if ((ops & CTB_DAILY_MEAN) && P->elem_bytes != 8) {
     ctb_set_error("ctb_pull_pack_daily: the mean plane is float64, the plan was built for %d-byte elements",
                   P->elem_bytes);
     return CTB_ERR_INVALID;
   }
-  if ((ops & (CTB_DAILY_MIN | CTB_DAILY_MAX)) && P->elem_bytes != es) {
+  if ((ops & (CTB_DAILY_MIN | CTB_DAILY_MAX)) && P->elem_bytes != sh.es) {
     ctb_set_error("ctb_pull_pack_daily: min/max planes have the source's %d-byte elements, the plan was built "
-                  "for %d-byte elements", (int)es, P->elem_bytes);
+                  "for %d-byte elements", (int)sh.es, P->elem_bytes);
     return CTB_ERR_INVALID;
   }
-  const int64_t phys_ncell = (int64_t)P->nlat_phys * P->nlon_phys;
-  if ((stride * es) % 16 != 0 || (uintptr_t)x % 16 != 0 || phys_ncell % CTB_PIECE != 0 ||
-      (uintptr_t)dst_mean % 16 != 0 || (uintptr_t)dst_min % 16 != 0 || (uintptr_t)dst_max % 16 != 0) {
-    ctb_set_error("ctb_pull_pack_daily: planes must be 16-byte aligned and hold a multiple of 4 gridcells");
+  if ((uintptr_t)dst_mean % 16 != 0 || (uintptr_t)dst_min % 16 != 0 || (uintptr_t)dst_max % 16 != 0) {
+    ctb_set_error("ctb_pull_pack_daily: destination planes must be 16-byte aligned");
     return CTB_ERR_UNSUPPORTED;
   }
-  if (n_days == 0) return CTB_OK;
-  CtbDeviceGuard guard(P->device);
-  if (guard.err != cudaSuccess) { ctb_set_error("cudaSetDevice(%d) failed: %s", P->device, cudaGetErrorString(guard.err)); return CTB_ERR_CUDA; }
-  const int halves = (int)(es / 4);
-  const int n_units = (int)(P->ncell / CTB_PIECE) * halves;
-  const int64_t n_work = (int64_t)n_units * n_days;
-  const unsigned grid = (unsigned)std::min<int64_t>((n_work + 255) / 256, 148 * 32);
-  const cudaStream_t st = (cudaStream_t)stream;
   const bool mean = ops & CTB_DAILY_MEAN, ext = ops & (CTB_DAILY_MIN | CTB_DAILY_MAX);
-  void* dmin = (ops & CTB_DAILY_MIN) ? dst_min : nullptr;
-  void* dmax = (ops & CTB_DAILY_MAX) ? dst_max : nullptr;
+  uint4* dmin = (ops & CTB_DAILY_MIN) ? static_cast<uint4*>(dst_min) : nullptr;
+  uint4* dmax = (ops & CTB_DAILY_MAX) ? static_cast<uint4*>(dst_max) : nullptr;
   auto go = [&](auto tag) {
     using T = decltype(tag);
-    auto f = mean ? (ext ? launch_subdaily<T, true, true> : launch_subdaily<T, true, false>)
-                  : launch_subdaily<T, false, true>;
-    f(grid, st, x, stride * es / 16, steps_per_day, day_index, t_begin, (int)n_days, P->d_pack_src, n_units,
-      halves, dst_mean, dmin, dmax);
+    auto k = mean ? (ext ? subdaily_pack_kernel<T, true, true> : subdaily_pack_kernel<T, true, false>)
+                  : subdaily_pack_kernel<T, false, true>;
+    k<<<sh.grid, 256, 0, (cudaStream_t)stream>>>(static_cast<const uint4*>(x), sh.stride16, steps_per_day, day_index,
+                                                  t_begin, (int)n_days, P->d_pack_src, sh.n_units, sh.halves,
+                                                  static_cast<double2*>(dst_mean), dmin, dmax);
+    return CTB_OK;
   };
-  if (dtype == CTB_F32) go(float{}); else go(double{});
-  CTB_LAUNCH_CHECK();
-  return CTB_OK;
+  return pull_launch(P, n_days, [&] { return dtype == CTB_F32 ? go(float{}) : go(double{}); });
 }
 
-// Per-step transforms of sub-daily sources, reduced to daily means in the same read: the addressing, the loads
-// in flight and the plane layout of subdaily_pack_kernel, with NOUT float64 planes of f_j averaged over the
-// day's non-NaN steps.  The threshold and edge decisions are those of the aggregation kernels (CtbTr packed by
+// Per-step transforms of sub-daily sources, reduced to daily means in the same read: the step loop and the plane
+// layout of subdaily_pack_kernel, with NOUT float64 planes of f_j averaged over the day's non-NaN steps.
+// The threshold and edge decisions are those of the aggregation kernels (CtbTr packed by
 // ctb_pack_transform): fp64 comparisons for double sources; for float sources the fp32 comparisons against
 // up / dn, which decide every float -- infinities included -- as the fp64 rule does (NaN steps never get here).
 //   EDD:  f = x > e ? x - e : 0                                    (= max(x - e, 0): x - e > 0 <=> x > e)
@@ -1062,23 +1095,15 @@ template <typename T, int OP, int NOUT>
 __global__ void __launch_bounds__(256, 2) subdaily_steps_kernel(
     const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
     int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, const CtbTr tr, StepDst dst) {
-  constexpr int C = 16 / sizeof(T);   // cells per 16-byte unit
-  constexpr int U = 8;                // step loads in flight
+  constexpr int C = 16 / sizeof(T);
   constexpr bool F32 = sizeof(T) == 4;
   double w[NOUT];                     // GDD: hi - lo of every pair
 #pragma unroll
   for (int j = 0; j < NOUT; ++j) w[j] = OP == CTB_STEP_GDD ? tr.a[2 * j + 1] - tr.a[2 * j] : 0.0;
-  const int64_t n_work = (int64_t)n_units * n_days;
-  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_work; i += (int64_t)gridDim.x * blockDim.x) {
-    const int u = (int)(i % n_units);
-    const int d = (int)(i / n_units);
-    const int p = __ldg(pack_src + u / halves);
-    if (p < 0) continue;                       // alignment padding of the packed plane: never read
-    const int64_t step0 = (int64_t)(day ? __ldg(day + t_begin + d) : t_begin + d) * S;
-    const uint4* s = src + step0 * stride16 + (int64_t)p * halves + (u % halves);
-    double sum[C][NOUT];
-    int hits[C][NOUT];
-    int cnt[C];
+  double sum[C][NOUT];
+  int hits[C][NOUT];
+  int cnt[C];
+  auto reset = [&] {
 #pragma unroll
     for (int c = 0; c < C; ++c) {
       cnt[c] = 0;
@@ -1088,58 +1113,51 @@ __global__ void __launch_bounds__(256, 2) subdaily_steps_kernel(
         hits[c][j] = 0;
       }
     }
-    for (int h0 = 0; h0 < S; h0 += U) {
-      uint4 v[U];
+  };
+  reset();
+  subdaily_step_loop<T>(
+      src, stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
+      [&](const T (&e)[C]) {
 #pragma unroll
-      for (int k = 0; k < U; ++k)
-        if (h0 + k < S)
-          asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                       : "=r"(v[k].x), "=r"(v[k].y), "=r"(v[k].z), "=r"(v[k].w)
-                       : "l"(s + (int64_t)(h0 + k) * stride16));
+        for (int c = 0; c < C; ++c) {
+          if (!(e[c] == e[c])) continue;   // NaN step: skipped
+          ++cnt[c];
+          const double x = (double)e[c];
+          if constexpr (OP == CTB_STEP_BINS) {
+            bool in[NOUT];
+            if constexpr (F32) ctb_bins_in_f32<NOUT>(tr, e[c], in); else ctb_bins_in<NOUT>(tr, x, in);
 #pragma unroll
-      for (int k = 0; k < U; ++k)
-        if (h0 + k < S) {
-          T e[C];
-          unit_get(v[k], e);
+            for (int j = 0; j < NOUT; ++j) hits[c][j] += in[j];
+          } else if constexpr (OP == CTB_STEP_EDD) {
 #pragma unroll
-          for (int c = 0; c < C; ++c) {
-            if (!(e[c] == e[c])) continue;   // NaN step: skipped
-            ++cnt[c];
-            const double x = (double)e[c];
-            if constexpr (OP == CTB_STEP_BINS) {
-              bool in[NOUT];
-              if constexpr (F32) ctb_bins_in_f32<NOUT>(tr, e[c], in); else ctb_bins_in<NOUT>(tr, x, in);
+            for (int j = 0; j < NOUT; ++j) {
+              const bool above = F32 ? (float)e[c] > tr.dn[j] : x > tr.a[j];
+              sum[c][j] = __dadd_rn(sum[c][j], above ? __dsub_rn(x, tr.a[j]) : 0.0);
+            }
+          } else {
 #pragma unroll
-              for (int j = 0; j < NOUT; ++j) hits[c][j] += in[j];
-            } else if constexpr (OP == CTB_STEP_EDD) {
-#pragma unroll
-              for (int j = 0; j < NOUT; ++j) {
-                const bool above = F32 ? (float)e[c] > tr.dn[j] : x > tr.a[j];
-                sum[c][j] = __dadd_rn(sum[c][j], above ? __dsub_rn(x, tr.a[j]) : 0.0);
-              }
-            } else {
-#pragma unroll
-              for (int j = 0; j < NOUT; ++j) {
-                const bool above = F32 ? (float)e[c] > tr.dn[2 * j] : x > tr.a[2 * j];
-                const bool top = F32 ? (float)e[c] >= tr.up[2 * j + 1] : x >= tr.a[2 * j + 1];
-                const double f = top ? w[j] : __dsub_rn(x, tr.a[2 * j]);
-                sum[c][j] = __dadd_rn(sum[c][j], above ? f : 0.0);
-              }
+            for (int j = 0; j < NOUT; ++j) {
+              const bool above = F32 ? (float)e[c] > tr.dn[2 * j] : x > tr.a[2 * j];
+              const bool top = F32 ? (float)e[c] >= tr.up[2 * j + 1] : x >= tr.a[2 * j + 1];
+              const double f = top ? w[j] : __dsub_rn(x, tr.a[2 * j]);
+              sum[c][j] = __dadd_rn(sum[c][j], above ? f : 0.0);
             }
           }
         }
-    }
+      },
+      [&](int d, int u) {
 #pragma unroll
-    for (int j = 0; j < NOUT; ++j) {
+        for (int j = 0; j < NOUT; ++j) {
 #pragma unroll
-      for (int c = 0; c < C; c += 2) {
-        const double s0 = OP == CTB_STEP_BINS ? (double)hits[c][j] : sum[c][j];
-        const double s1 = OP == CTB_STEP_BINS ? (double)hits[c + 1][j] : sum[c + 1][j];
-        dst.p[j][((int64_t)d * n_units + u) * (C / 2) + c / 2] =
-            make_double2(__ddiv_rn(s0, (double)cnt[c]), __ddiv_rn(s1, (double)cnt[c + 1]));
-      }
-    }
-  }
+          for (int c = 0; c < C; c += 2) {
+            const double s0 = OP == CTB_STEP_BINS ? (double)hits[c][j] : sum[c][j];
+            const double s1 = OP == CTB_STEP_BINS ? (double)hits[c + 1][j] : sum[c + 1][j];
+            dst.p[j][((int64_t)d * n_units + u) * (C / 2) + c / 2] =
+                make_double2(__ddiv_rn(s0, (double)cnt[c]), __ddiv_rn(s1, (double)cnt[c + 1]));
+          }
+        }
+        reset();
+      });
 }
 }  // namespace
 
@@ -1147,11 +1165,8 @@ extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int d
                                          int steps_per_day, const int32_t* day_index, int64_t t_begin,
                                          int64_t n_days, int step_op, const double* params, int n_params, int n_out,
                                          double* const* dst, void* stream) {
-  if (!P || !x || n_days < 0 || n_days >= (1ll << 31) || t_begin < 0 || !P->compact) {
-    ctb_set_error("ctb_pull_pack_daily_steps: needs a compact plan, a non-null source and 0 <= n_days < 2^31");
-    return CTB_ERR_INVALID;
-  }
-  if (dtype != CTB_F32 && dtype != CTB_F64) { ctb_set_error("dtype=%d unsupported", dtype); return CTB_ERR_INVALID; }
+  PullShape sh;
+  if (int rc = pull_check("ctb_pull_pack_daily_steps", P, x, dtype, stride, t_begin, n_days, n_days, &sh)) return rc;
   if (steps_per_day < 1) {
     ctb_set_error("ctb_pull_pack_daily_steps: steps_per_day=%d, needs >= 1", steps_per_day);
     return CTB_ERR_INVALID;
@@ -1191,6 +1206,10 @@ extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int d
   StepDst planes{};
   for (int j = 0; j < n_out; ++j) {
     if (!dst[j]) { ctb_set_error("ctb_pull_pack_daily_steps: dst[%d] is null", j); return CTB_ERR_INVALID; }
+    if ((uintptr_t)dst[j] % 16 != 0) {
+      ctb_set_error("ctb_pull_pack_daily_steps: dst[%d] is not 16-byte aligned", j);
+      return CTB_ERR_UNSUPPORTED;
+    }
     planes.p[j] = reinterpret_cast<double2*>(dst[j]);
   }
   if (P->elem_bytes != 8) {
@@ -1198,43 +1217,18 @@ extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int d
                   P->elem_bytes);
     return CTB_ERR_INVALID;
   }
-  const int64_t es = dtype == CTB_F32 ? 4 : 8;
-  const int64_t phys_ncell = (int64_t)P->nlat_phys * P->nlon_phys;
-  bool aligned = (stride * es) % 16 == 0 && (uintptr_t)x % 16 == 0 && phys_ncell % CTB_PIECE == 0;
-  for (int j = 0; j < n_out; ++j) aligned = aligned && (uintptr_t)dst[j] % 16 == 0;
-  if (!aligned) {
-    ctb_set_error("ctb_pull_pack_daily_steps: planes must be 16-byte aligned and hold a multiple of 4 gridcells");
-    return CTB_ERR_UNSUPPORTED;
-  }
-  if (n_days == 0) return CTB_OK;
-  CtbDeviceGuard guard(P->device);
-  if (guard.err != cudaSuccess) { ctb_set_error("cudaSetDevice(%d) failed: %s", P->device, cudaGetErrorString(guard.err)); return CTB_ERR_CUDA; }
-  const int halves = (int)(es / 4);
-  const int n_units = (int)(P->ncell / CTB_PIECE) * halves;
-  const int64_t n_work = (int64_t)n_units * n_days;
-  const unsigned grid = (unsigned)std::min<int64_t>((n_work + 255) / 256, 148 * 32);
-  const cudaStream_t st = (cudaStream_t)stream;
-  auto go = [&](auto tag, auto op, auto nout) {
-    subdaily_steps_kernel<decltype(tag), decltype(op)::value, decltype(nout)::value><<<grid, 256, 0, st>>>(
-        static_cast<const uint4*>(x), stride * es / 16, steps_per_day, day_index, t_begin, (int)n_days,
-        P->d_pack_src, n_units, halves, tr, planes);
+  auto go = [&](auto tag) {
+    auto launch = [&](auto op, auto nout) {
+      subdaily_steps_kernel<decltype(tag), op, nout><<<sh.grid, 256, 0, (cudaStream_t)stream>>>(
+          static_cast<const uint4*>(x), sh.stride16, steps_per_day, day_index, t_begin, (int)n_days, P->d_pack_src,
+          sh.n_units, sh.halves, tr, planes);
+      return CTB_OK;
+    };
+    if (step_op == CTB_STEP_EDD) return ctb_dispatch_nout<CTB_STEP_EDD>(n_out, launch);
+    if (step_op == CTB_STEP_GDD) return ctb_dispatch_nout<CTB_STEP_GDD>(n_out, launch);
+    return ctb_dispatch_nout<CTB_STEP_BINS>(n_out, launch);
   };
-  auto by_nout = [&](auto tag, auto op) {
-    switch (n_out) {
-      case 1: go(tag, op, std::integral_constant<int, 1>{}); break;
-      case 2: go(tag, op, std::integral_constant<int, 2>{}); break;
-      case 3: go(tag, op, std::integral_constant<int, 3>{}); break;
-      default: go(tag, op, std::integral_constant<int, 4>{}); break;
-    }
-  };
-  auto by_op = [&](auto tag) {
-    if (step_op == CTB_STEP_EDD) by_nout(tag, std::integral_constant<int, CTB_STEP_EDD>{});
-    else if (step_op == CTB_STEP_GDD) by_nout(tag, std::integral_constant<int, CTB_STEP_GDD>{});
-    else by_nout(tag, std::integral_constant<int, CTB_STEP_BINS>{});
-  };
-  if (dtype == CTB_F32) by_op(float{}); else by_op(double{});
-  CTB_LAUNCH_CHECK();
-  return CTB_OK;
+  return pull_launch(P, n_days, [&] { return dtype == CTB_F32 ? go(float{}) : go(double{}); });
 }
 
 // ---------------------------------------------------------------------------

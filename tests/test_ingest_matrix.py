@@ -575,6 +575,44 @@ def test_ragged_grid(dev, dtype, nlat, nlon):
     check(out.cpu().numpy(), ref, base, sny, "ragged {}".format(np.dtype(dtype).name))
 
 
+# one fault per call of ctb_pull_pack: (arguments changed, status, a word of the message)
+PULL_FAULTS = (
+    ("non-compact plan", {"plan": "full"}, N.ERR_INVALID, "compact"),
+    ("dtype 7", {"dtype": 7}, N.ERR_INVALID, "dtype=7"),
+    ("misaligned source", {"offset": 4}, N.ERR_UNSUPPORTED, "aligned"),
+    ("T < 0", {"T": -1}, N.ERR_INVALID, "T=-1"),
+    ("T >= 2^31", {"T": 2 ** 31}, N.ERR_INVALID, "T=2147483648"),
+    ("t_begin < 0", {"t_begin": -1}, N.ERR_INVALID, "t_begin=-1"),
+)
+
+
+@pytest.mark.gpu
+def test_pull_pack_refuses_single_faults(dev):
+    """``ctb_pull_pack`` refuses each fault of ``PULL_FAULTS`` alone, with its status and message, and writes
+    nothing; the same call without the fault succeeds.  The source starts one plane into its buffer, so that
+    even plane t_begin - 1 lies inside it."""
+    import torch
+    from climate_toolbox_b200 import _engine as E
+    full, comp = plans(4, 1, 0)
+    n_days = 8
+    buf = torch.zeros((n_days + 1, NCELL), dtype=torch.float32, device=dev)
+    width = 4 * len(layout_of(comp))
+    L = N.lib()
+
+    def call(plan="comp", dtype=N.F32, offset=0, t_begin=0, T=n_days):
+        dst = _filled_planes(n_days, width, F32, dev)
+        rc = L.ctb_pull_pack((full if plan == "full" else comp)._h, C.c_void_p(buf[1].data_ptr() + offset), dtype,
+                             NCELL, None, t_begin, T, _ptr(dst), E._stream_ptr(dev))
+        torch.cuda.synchronize(dev)
+        return rc, bool((dst.view(torch.int32) == int(SENT32)).all())
+
+    assert call() == (N.OK, False)
+    for label, change, status, word in PULL_FAULTS:
+        rc, untouched = call(**change)
+        assert rc == status and word in N.last_error(), (label, rc, N.last_error())
+        assert untouched, label
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("dtype", [F32, F64])
 def test_padding_is_never_read(dev, dtype):

@@ -27,8 +27,9 @@ agg_direct_kernel      ``tp * stride + c`` / ``c * stride + tp`` (int64)        
 transform_kernel       grid-stride ``i`` (int64), ``(size_t)j * n + i``              2,164,838,399 (case H)
 gather_rows_kernel     ``tp * stride + c`` / ``c * stride + tp``, ``out[i]``         2,164,838,399 (case I)
 pull_pack_kernel       ``src + tp * stride16 + so`` (16-byte units)                  8,659,353,596 bytes (case J)
-subdaily_pack_kernel   ``src + step0 * stride16 + p * halves + u % halves``          8,659,353,596 bytes (case J)
-                       ``+ (h0 + k) * stride16``
+subdaily_step_loop     ``src + step0 * stride16 + p * halves + u % halves``          8,659,353,596 bytes (case J, both
+  (both sub-daily      ``+ (h0 + k) * stride16``                                    kernels: subdaily_pack_kernel
+  kernels)                                                                          and subdaily_steps_kernel)
 =====================  ===========================================================  ===================================
 
 The float64 time-indexed byte offset (row C) wrapped at 2^32 before: ``(uint32_t)off * (uint32_t)sizeof(TIN)``
@@ -36,8 +37,8 @@ read the cell 2^29 positions earlier for every cell at or past 2^29.  Case C fai
 
 Audited and not reachable within 180 GB (limits the library checks, so no test): the plan refuses grids of 2^30
 cells or more and 2^31 weights rows (case D checks the first refusal), so unit offsets, row cells and CSR indices
-fit int32; ``T`` and every time index are below 2^31 (``ctb_aggregate``, ``ctb_pull_pack`` and
-``ctb_pull_pack_daily`` refuse more), so ``tb * 32 + lane`` and the day of a tile fit int32; the streaming
+fit int32; ``T`` and every time index are below 2^31 (``ctb_aggregate`` and the three ``ctb_pull_pack*`` entry
+points refuse more), so ``tb * 32 + lane`` and the day of a tile fit int32; the streaming
 scheduler refuses 2^31 work units; a packed plane has fewer than 2^30 cells, so ``n_units`` of the pull kernels
 fits int32.  The split-region scratch ``((size_t)j * n_scratch + slot) * scratch_ld + t`` and the time-group
 partial sums are size_t products reached only at small sizes here.
@@ -61,6 +62,7 @@ import pytest
 import oracle
 from test_kernel_matrix import NEEDED, U, check, reference
 from test_subdaily import resample_daily_ref
+from test_subdaily_steps import steps_ref
 from climate_toolbox_b200 import _native as N
 
 # ----------------------------------------------------------------------------
@@ -701,3 +703,37 @@ def test_j_pull_pack_daily_hourly_past_2_31_steps(q32):
             want = resample_daily_ref(hourly, S, h).astype(np.float64).T
             assert np.array_equal(got, want), h
         plan.close()
+
+
+# thresholds and edges that split both the kelvin values and the Celsius range
+J_STEPS = (("edd", N.STEP_EDD, (0.0, 290.0), (0.0, 290.0)),
+           ("gdd", N.STEP_GDD, (10.0, 30.0, 250.0, 300.0), ((10.0, 30.0), (250.0, 300.0))),
+           ("bins", N.STEP_BINS, (0.0, 260.0, 300.0), (0.0, 260.0, 300.0)))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("op,step_op,params,ref_params", J_STEPS, ids=[s[0] for s in J_STEPS])
+def test_j_pull_pack_daily_steps_hourly_past_2_31_steps(q32, op, step_op, params, ref_params):
+    """J: ctb_pull_pack_daily_steps on the same hourly view: day 86 reads steps past 2^31 elements through the step
+    loop that subdaily_pack_kernel shares.  Two outputs of EDD, GDD and bins, bit for bit against
+    ``test_subdaily_steps.steps_ref``."""
+    import torch
+    from climate_toolbox_b200 import _engine as E
+    S = 24
+    days = np.array([0, 86, 43, 86, 85, 1, 86])
+    dev = q32.device
+    day_t = torch.as_tensor(days.astype(np.int32), device=dev)
+    steps = (days[:, None] * S + np.arange(S)[None]).reshape(-1)
+    hourly = value_np(tm_index(steps, J_CELLS, QCELL), QCELL, Q_CELSIUS).astype(np.float32)
+    plan = _one_cell_plan(J_CELLS, 8, 12)
+    width = plan.info["n_packed_cells"]
+    dst = [torch.empty((len(days), width), dtype=torch.float64, device=dev) for _ in range(2)]
+    prm = (C.c_double * len(params))(*params)
+    ptrs = (C.c_void_p * 2)(*[d.data_ptr() for d in dst])
+    N.check(N.lib().ctb_pull_pack_daily_steps(plan._h, C.c_void_p(q32.data_ptr()), N.F32, QCELL, S,
+                                              C.c_void_p(day_t.data_ptr()), 0, len(days), step_op, prm, len(params),
+                                              2, ptrs, E._stream_ptr(dev)))
+    for j, want in enumerate(steps_ref(hourly, S, op, ref_params)):
+        got = _agg(plan, dst[j], None, width, None, len(days))[0].cpu().numpy()
+        assert np.array_equal(got, want.T), (op, j)
+    plan.close()
