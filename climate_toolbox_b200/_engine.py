@@ -604,16 +604,37 @@ DAILY_STAGE_BYTES = 256 << 20    # pinned staging slot of a pageable sub-daily s
 class DailySource:
     """What ``ctb_pull_pack_daily`` reads for one deferred daily variable (``utils.resample_daily``): the
     sub-daily source as 2-D [t_phys, ncell], its steps per day, its first step and the physical day of
-    every day."""
+    every day.  A decoded packed source (``io.decode_packed``) is read the same way: its own deferred record is
+    ``how = "decode"`` with one step per day and the raw source's time take as the days; as the source of a daily
+    reduction it is the raw int16 buffer with ``dec``, its decoding (None for float sources)."""
 
     def __init__(self, var):
         d = var.deferred
-        self.how, self.S, self.t0, self.day = d.params
-        src = d.sources[0]
+        self.dec = None
+        if d.kind == "decode":
+            src = d.sources[0]
+            self.how, self.S, self.t0, self.dec = "decode", 1, 0, d.params
+            self.day = src.takes.get(src.dims[0])
+            if self.day is None:
+                self.day = np.arange(src.physical.shape[0], dtype=np.int64)
+        else:
+            self.how, self.S, self.t0, self.day = d.params
+            src = d.sources[0]
+            if src.deferred is not None:      # a daily reduction of a decoded packed source
+                self.dec = src.deferred.params
+                src = src.deferred.sources[0]
         self.phys = x = src.physical
         if isinstance(x, torch.Tensor) and not x.is_cuda:
             x = x.numpy()
-        if isinstance(x, torch.Tensor):
+        if self.dec is not None:
+            x = x.contiguous() if isinstance(x, torch.Tensor) else np.ascontiguousarray(x)
+            self.dtype = None
+            self.pinned = not isinstance(x, torch.Tensor) and _all_pinned([x])
+            self.itemsize = 2
+            self.decoded_bytes = np.dtype(self.dec[3]).itemsize
+            self.ctb_dec = N.Decode(self.dec[0], self.dec[1], _NP2CTB[np.dtype(self.dec[3])], len(self.dec[2]),
+                                    (C.c_int16 * 4)(*self.dec[2]))
+        elif isinstance(x, torch.Tensor):
             x = (x if x.dtype in _T2CTB else x.to(torch.float64)).contiguous()
             self.dtype = _T2CTB[x.dtype]
             self.pinned = False
@@ -625,8 +646,10 @@ class DailySource:
         self.nlat_phys, self.nlon_phys = int(x.shape[1]), int(x.shape[2])
         self.stride = self.nlat_phys * self.nlon_phys
         self.x = x.reshape(x.shape[0], self.stride)
-        self.itemsize = 4 if self.dtype == N.F32 else 8
-        self.out_bytes = self.itemsize if self.how in ("min", "max") else 8     # element size of its daily planes
+        if self.dec is None:
+            self.itemsize = self.decoded_bytes = 4 if self.dtype == N.F32 else 8
+        # element size of its planes: the (decoded) source type for decoded values and min / max, else float64
+        self.out_bytes = self.decoded_bytes if self.how in ("decode", "min", "max") else 8
         self.lat_phys, self.lon_phys = src.takes.get("lat"), src.takes.get("lon")
         self.T = len(self.day)
 
@@ -635,9 +658,9 @@ class DailySource:
         return base + self.t0 * self.stride * self.itemsize
 
     def same_read(self, other):
-        """Both read the same steps of the same buffer."""
+        """Both read the same steps of the same buffer, decoded the same way."""
         return (self.phys is other.phys and (self.S, self.t0) == (other.S, other.t0) and
-                np.array_equal(self.day, other.day))
+                np.array_equal(self.day, other.day) and self.dec == other.dec)
 
 
 def _day_arg(plan, day):
@@ -665,7 +688,8 @@ def _step_params(hows):
 
 
 def _pull_daily(plan, src, dsts, d0, n):
-    """Queue ``ctb_pull_pack_daily`` (or ``ctb_pull_pack_daily_steps`` for per-step transforms) for days
+    """Queue ``ctb_pull_pack_daily`` (or ``ctb_pull_pack_daily_steps`` for per-step transforms; their ``_decode``
+    counterparts for a decoded source, and ``ctb_pull_pack_decode`` for its decoded values) for days
     d0 .. d0 + n - 1 of ``src`` into ``dsts`` ({how: device tensor [>= n, n_packed_cells]}, all from one read, hows
     that :func:`_joins` accepts).  A pageable host source is staged first: whole days are copied into pinned
     buffers (those of the host path, two in turn) that the kernel then reads."""
@@ -675,25 +699,33 @@ def _pull_daily(plan, src, dsts, d0, n):
     steps = isinstance(hows[0], tuple)
     if steps:
         pa, pp = _params_array("daily_steps", _step_params(hows))
-    else:
+    elif hows != ["decode"]:
         ops = 0
         for how in hows:
             ops |= _DAILY_OP[how]
+    dec = src.dec is not None
+    # the float entry points take the dtype, the decoding ones the ctb_decode record
+    kind = (C.byref(src.ctb_dec),) if dec else (src.dtype,)
 
     def call(x_ptr, day, t_begin, k, m):
         day_d = _day_arg(plan, day) if day is not None else None
         day_p = C.c_void_p(day_d.data_ptr()) if day_d is not None else None
         ptrs = {h: t.data_ptr() + k * t.shape[1] * t.element_size() for h, t in dsts.items()}
-        if steps:
-            N.check(L.ctb_pull_pack_daily_steps(
-                plan._h, C.c_void_p(x_ptr), src.dtype, int(src.stride), int(src.S), day_p, int(t_begin), int(m),
+        x, stride = C.c_void_p(x_ptr), int(src.stride)
+        args = (x, stride) + kind if dec else (x,) + kind + (stride,)
+        if hows == ["decode"]:
+            N.check(L.ctb_pull_pack_decode(plan._h, *args, day_p, int(t_begin), int(m), C.c_void_p(ptrs["decode"]),
+                                           _stream_ptr(dev)))
+        elif steps:
+            N.check((L.ctb_pull_pack_daily_steps_decode if dec else L.ctb_pull_pack_daily_steps)(
+                plan._h, *args, int(src.S), day_p, int(t_begin), int(m),
                 _STEP_OP[hows[0][0]], pp, int(pa.size), len(hows), (C.c_void_p * len(hows))(*ptrs.values()),
                 _stream_ptr(dev)))
         else:
-            N.check(L.ctb_pull_pack_daily(
-                plan._h, C.c_void_p(x_ptr), src.dtype, int(src.stride), int(src.S), day_p, int(t_begin), int(m), ops,
+            N.check((L.ctb_pull_pack_daily_decode if dec else L.ctb_pull_pack_daily)(
+                plan._h, *args, int(src.S), day_p, int(t_begin), int(m), ops,
                 *[C.c_void_p(ptrs[h]) if h in ptrs else None for h in ("mean", "min", "max")], _stream_ptr(dev)))
-        if not src.on_device:
+        if not src.on_device:      # 4 cells of the source per piece and step: 8 bytes of int16
             TRANSFER_BYTES["h2d"] += m * src.S * plan.info["n_pieces_distinct"] * 4 * src.itemsize
 
     if n == 0:
@@ -704,7 +736,7 @@ def _pull_daily(plan, src, dsts, d0, n):
     day = src.day[d0: d0 + n]
     per_day = src.S * src.stride * src.itemsize
     cap = max(1, DAILY_STAGE_BYTES // per_day)
-    np_dt = np.float32 if src.itemsize == 4 else np.float64
+    np_dt = src.x.dtype
     main = torch.cuda.current_stream(dev)
     k, slot = 0, 0
     with _HOST_LOCK:
@@ -778,8 +810,9 @@ def _full_grid_plan(nlat, nlon, elem_bytes, dev):
 
 
 def daily_device(var, dev):
-    """A deferred daily variable evaluated for the whole grid by ``ctb_pull_pack_daily``: CUDA tensor
-    [days, lat, lon] with the variable's lat / lon takes applied."""
+    """A deferred daily variable (or a decoded packed source) evaluated for the whole grid by
+    ``ctb_pull_pack_daily`` (``ctb_pull_pack_decode``): CUDA tensor [days, lat, lon] with the variable's lat / lon
+    takes applied."""
     src = DailySource(var)
     es = src.out_bytes
     plan = _full_grid_plan(src.nlat_phys, src.nlon_phys, es, dev)
@@ -935,8 +968,8 @@ class _OffsetOut:
 # deferred variables (`.values` of a transformed / reindexed variable)
 # ---------------------------------------------------------------------------
 def _to_device(v, dev):
-    """Materialise a (non-deferred or daily) Variable on the device with its lazy takes applied."""
-    if v.deferred is not None and v.deferred.kind == "daily":
+    """Materialise a (non-deferred, daily or decoded) Variable on the device with its lazy takes applied."""
+    if v.deferred is not None and v.deferred.kind in ("daily", "decode"):
         return daily_device(v, dev)
     a = v.physical
     t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a))
@@ -953,7 +986,7 @@ def materialize_deferred(var):
     dev = default_device()
     if d.kind == "reindex":
         return d.params[0]()  # closure built by aggregations._pointwise_reindex
-    if d.kind == "daily":
+    if d.kind in ("daily", "decode"):
         return daily_device(var, dev).cpu().numpy()
     srcs = [_to_device(s, dev) for s in d.sources]
     if srcs[0].dtype not in _T2CTB:

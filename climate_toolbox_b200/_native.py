@@ -28,6 +28,7 @@ SYMBOLS = (
     "ctb_plan_get_info", "ctb_plan_row_cells", "ctb_plan_den", "ctb_plan_row_weights", "ctb_plan_region_order",
     "ctb_aggregate_workspace_bytes", "ctb_aggregate", "ctb_transform", "ctb_gather_rows",
     "ctb_host_pack", "ctb_pull_pack", "ctb_pull_pack_daily", "ctb_pull_pack_daily_steps",
+    "ctb_pull_pack_decode", "ctb_pull_pack_daily_decode", "ctb_pull_pack_daily_steps_decode",
     "ctb_copy_rows_to_host", "ctb_time_groups_create", "ctb_time_groups_free", "ctb_time_groups_count",
     "ctb_aggregate_grouped_workspace_bytes", "ctb_aggregate_grouped", "ctb_aggregate_ex",
     "ctb_ipc_alloc", "ctb_ipc_open", "ctb_ipc_close", "ctb_ipc_free", "ctb_push_rows", "ctb_fingerprint",
@@ -43,6 +44,12 @@ class PlanOpts(C.Structure):
 class AggOpts(C.Structure):
     _fields_ = [("groups", C.c_void_p), ("t_begin", C.c_int64), ("flush", C.c_int32), ("n_peer_out", C.c_int32),
                 ("day_of_year", C.c_void_p), ("peer_out", C.POINTER(C.c_void_p)), ("peer_row", C.c_void_p)]
+
+
+class Decode(C.Structure):
+    """``ctb_decode``: CF packing of an int16 source (scale, offset, decoded dtype, fill values)."""
+    _fields_ = [("scale", C.c_double), ("offset", C.c_double), ("dtype", C.c_int32), ("n_fill", C.c_int32),
+                ("fill", C.c_int16 * 4)]
 
 
 PUSH_SM, PUSH_COPY_ENGINE = 0, 1
@@ -136,6 +143,14 @@ def lib():
     L.ctb_pull_pack_daily_steps.restype = C.c_int
     L.ctb_pull_pack_daily_steps.argtypes = [p, vp, C.c_int, i64, C.c_int, vp, i64, i64, C.c_int, vp, C.c_int, C.c_int,
                                             vp, vp]
+    dec = C.POINTER(Decode)
+    L.ctb_pull_pack_decode.restype = C.c_int
+    L.ctb_pull_pack_decode.argtypes = [p, vp, i64, dec, vp, i64, i64, vp, vp]
+    L.ctb_pull_pack_daily_decode.restype = C.c_int
+    L.ctb_pull_pack_daily_decode.argtypes = [p, vp, i64, dec, C.c_int, vp, i64, i64, C.c_int, vp, vp, vp, vp]
+    L.ctb_pull_pack_daily_steps_decode.restype = C.c_int
+    L.ctb_pull_pack_daily_steps_decode.argtypes = [p, vp, i64, dec, C.c_int, vp, i64, i64, C.c_int, vp, C.c_int,
+                                                   C.c_int, vp, vp]
     L.ctb_copy_rows_to_host.restype = C.c_int
     L.ctb_copy_rows_to_host.argtypes = [vp, C.c_size_t, vp, C.c_size_t, C.c_size_t, C.c_size_t, vp]
     L.ctb_time_groups_create.restype = C.c_int

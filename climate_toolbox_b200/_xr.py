@@ -53,7 +53,9 @@ class Deferred:
              params = (materialise closure, origin Dataset)) | "daily" (daily reduction of a sub-daily
              (time, lat, lon) source, params = (how, steps per day, first step, physical day of every day);
              how = "mean" | "min" | "max", or the daily mean of a per-step transform: ("edd", e) |
-             ("gdd", lo, hi) | ("bins", lo, hi))
+             ("gdd", lo, hi) | ("bins", lo, hi)) | "decode" (a CF-packed int16 (time, lat, lon) source decoded on
+             the GPU, ``io.decode_packed``; params = (scale, offset, fill values, D), D the decoded numpy dtype;
+             takes compose onto the raw source)
     params : tuple of floats (poly: (offset, power); bins: (offset, lo, hi); rcspline: (offset, term,
              k_1, ..., k_n); edd: (threshold,); gdd: (threshold_low, threshold_high))
     sources: tuple of :class:`Variable` (poly / bins / rcspline: (tas,); edd/gdd: (tasmin, tasmax))
@@ -107,6 +109,8 @@ class Variable:
     def dtype(self):
         if self.deferred is not None:
             d = self.deferred
+            if d.kind == "decode":
+                return np.dtype(d.params[3])
             return d.sources[0].dtype if d.kind == "daily" and d.params[0] in ("min", "max") else np.dtype("float64")
         d = self._data.dtype
         return np.dtype(str(d).replace("torch.", "")) if _is_torch(self._data) else d

@@ -100,14 +100,16 @@ class _GridView:
 
 
 class _DailyView:
-    """A deferred daily reduction of sub-daily data (``utils.resample_daily``) as the kernels see it: packed
-    planes of days, written by the reduce-pack kernel for a compact plan of the daily planes' element size."""
+    """A deferred daily reduction of sub-daily data (``utils.resample_daily``) or a decoded packed source
+    (``io.decode_packed``) as the kernels see it: packed planes of days, written by the reduce-pack or decode-pack
+    kernel for a compact plan of the planes' element size."""
 
     layout = N.LAYOUT_TIME_MAJOR
     tix = None
 
     def __init__(self, var):
         self.src = E.DailySource(var)
+        self.kind = var.deferred.kind
         self.how = self.src.how
         self.dims = self.out_dims_template = var.dims
         self.other_dims = (var.dims[0],)
@@ -128,7 +130,8 @@ class _DailyView:
 
 
 def _is_daily(var):
-    return var.deferred is not None and var.deferred.kind == "daily"
+    """A deferred variable that the GPU pack evaluates: a daily reduction or a decoded packed source."""
+    return var.deferred is not None and var.deferred.kind in ("daily", "decode")
 
 
 def _view(var):
@@ -138,7 +141,8 @@ def _view(var):
 def _step_family(var):
     """"edd" / "gdd" / "bins" for the daily mean of a per-step transform of sub-daily data
     (``transformations.subdaily_*``), else None."""
-    return var.deferred.params[0][0] if _is_daily(var) and isinstance(var.deferred.params[0], tuple) else None
+    d = var.deferred
+    return d.params[0][0] if _is_daily(var) and d.kind == "daily" and isinstance(d.params[0], tuple) else None
 
 
 def _same_steps(a, b):
@@ -149,12 +153,21 @@ def _same_steps(a, b):
 
 
 def _same_source(a, b):
-    """Two transform sources read the same data: the same buffer and takes, and for daily reductions also
-    the same ``how``, steps and days."""
+    """Two transform sources read the same data: the same buffer and takes, for daily reductions also the same
+    ``how``, steps and days, and for decoded sources the same decoding."""
     if _is_daily(a) or _is_daily(b):
-        return _is_daily(a) and _is_daily(b) and a.deferred.params[0] == b.deferred.params[0] and _same_steps(a, b)
+        if not (_is_daily(a) and _is_daily(b) and a.deferred.kind == b.deferred.kind):
+            return False
+        if a.deferred.kind == "decode":
+            return _same_decode(a.deferred.params, b.deferred.params) and \
+                _same_source(a.deferred.sources[0], b.deferred.sources[0])
+        return a.deferred.params[0] == b.deferred.params[0] and _same_steps(a, b)
     return (a.physical is b.physical and a.dims == b.dims and
             all(_eq(a.takes.get(d), b.takes.get(d)) for d in a.dims))
+
+
+def _same_decode(pa, pb):
+    return pa[:3] == pb[:3] and np.dtype(pa[3]) == np.dtype(pb[3])
 
 
 def _eq(a, b):
@@ -315,9 +328,9 @@ def _aggregate_core(ds, variables, aggwt, agglev, weights, backup_aggwt, variant
         views = [_view(s) for s in g["srcs"]]
         v0 = views[0]
         daily = isinstance(v0, _DailyView)
-        if any(isinstance(v, _DailyView) != daily for v in views):
-            raise ValueError("inputs of a two-input transform must both be daily reductions of sub-daily data, "
-                             "or neither")
+        if any(getattr(v, "kind", None) != getattr(v0, "kind", None) for v in views):
+            raise ValueError("inputs of a two-input transform must both be daily reductions of sub-daily data "
+                             "or decoded packed sources, or neither")
         for v in views[1:]:
             if not v0.same_geometry(v):
                 raise ValueError("inputs of a two-input transform must share shape, dtype and layout")
@@ -325,7 +338,8 @@ def _aggregate_core(ds, variables, aggwt, agglev, weights, backup_aggwt, variant
         dev = device or (v0.data2d.device if v0.on_device else E.default_device())
         # host-resident (time, lat, lon) inputs go through a compact plan: only the referenced
         # gridcells are packed on the host and cross PCIe
-        # daily reductions of sub-daily data are packed by the reduce-pack kernel wherever the data lives
+        # daily reductions of sub-daily data and decoded packed sources are packed by the reduce-pack or
+        # decode-pack kernel wherever the data lives
         compact = daily or ((not v0.on_device) and v0.layout == N.LAYOUT_TIME_MAJOR and pack_host)
         cell_gate = doy = None
         if season_mask is not None:

@@ -860,20 +860,25 @@ __global__ void __launch_bounds__(256) pull_pack_kernel(const uint4* __restrict_
   }
 }
 
-// The launch shape of the pull kernels: one thread per 16-byte unit of a packed plane and work row.
+// The launch shape of the pull kernels: one thread per unit of a packed plane and work row.  A unit is 16 bytes
+// of a float source; of an int16 source it is one 4-cell piece, 8 bytes.
 struct PullShape {
   int64_t es;        // bytes per source element
-  int64_t stride16;  // the source's plane stride in 16-byte units
-  int halves;        // 16-byte units per 4-cell piece
-  int n_units;       // 16-byte units per packed plane
+  int64_t stride16;  // the source's plane stride in units (16 bytes; 8 for int16)
+  int halves;        // units per 4-cell piece
+  int n_units;       // units per packed plane
   unsigned grid;
 };
 
-// The checks the three pull entry points share, in this order: a compact plan, a source, 0 <= n_days < 2^31
-// and t_begin >= 0, a float32 or float64 dtype, and 16-byte aligned source planes on a grid of whole 4-cell
-// pieces (a ragged last piece would be read past the plane).  Each entry checks its destinations itself.
-int pull_check(const char* fn, const ctb_plan* P, const void* x, int dtype, int64_t stride, int64_t t_begin,
-               int64_t n_days, int64_t rows, PullShape* sh) {
+// Bytes per element of a float dtype, 0 for any other value
+int64_t float_bytes(int dtype) { return dtype == CTB_F32 ? 4 : dtype == CTB_F64 ? 8 : 0; }
+
+// The checks the pull entry points share, in this order: a compact plan, a source, 0 <= n_days < 2^31 and
+// t_begin >= 0, a source element size es of 2, 4 or 8 (0: `dtype` is no float dtype), and source planes aligned
+// to one unit on a grid of whole 4-cell pieces (a ragged last piece would be read past the plane).  Each entry
+// checks its destinations itself.
+int pull_check(const char* fn, const ctb_plan* P, const void* x, int dtype, int64_t es, int64_t stride,
+               int64_t t_begin, int64_t n_days, int64_t rows, PullShape* sh) {
   if (!P || !P->compact) { ctb_set_error("%s: needs a compact plan", fn); return CTB_ERR_INVALID; }
   if (!x) { ctb_set_error("%s: the source is null", fn); return CTB_ERR_INVALID; }
   if (n_days < 0 || n_days >= (1ll << 31) || t_begin < 0) {
@@ -881,17 +886,19 @@ int pull_check(const char* fn, const ctb_plan* P, const void* x, int dtype, int6
                   (long long)t_begin);
     return CTB_ERR_INVALID;
   }
-  if (dtype != CTB_F32 && dtype != CTB_F64) {
+  if (es == 0) {
     ctb_set_error("%s: dtype=%d unsupported", fn, dtype);
     return CTB_ERR_INVALID;
   }
-  sh->es = dtype == CTB_F32 ? 4 : 8;
-  if ((stride * sh->es) % 16 != 0 || (uintptr_t)x % 16 != 0 || (int64_t)P->nlat_phys * P->nlon_phys % CTB_PIECE != 0) {
-    ctb_set_error("%s: planes must be 16-byte aligned and hold a multiple of 4 gridcells", fn);
+  sh->es = es;
+  const int64_t unit = es == 2 ? 8 : 16;
+  if ((stride * sh->es) % unit != 0 || (uintptr_t)x % unit != 0 ||
+      (int64_t)P->nlat_phys * P->nlon_phys % CTB_PIECE != 0) {
+    ctb_set_error("%s: planes must be %d-byte aligned and hold a multiple of 4 gridcells", fn, (int)unit);
     return CTB_ERR_UNSUPPORTED;
   }
-  sh->stride16 = stride * sh->es / 16;
-  sh->halves = (int)(sh->es / 4);
+  sh->stride16 = stride * sh->es / unit;
+  sh->halves = es == 2 ? 1 : (int)(sh->es / 4);
   sh->n_units = (int)(P->ncell / CTB_PIECE) * sh->halves;
   sh->grid = (unsigned)std::min<int64_t>(((int64_t)sh->n_units * rows + 255) / 256, 148 * 32);
   return CTB_OK;
@@ -912,7 +919,7 @@ int pull_launch(const ctb_plan* P, int64_t n_days, F&& launch) {
 extern "C" int ctb_pull_pack(const ctb_plan* P, const void* x, int dtype, int64_t stride,
                              const int32_t* time_index, int64_t t_begin, int64_t T, void* dst, void* stream) {
   PullShape sh;
-  if (int rc = pull_check("ctb_pull_pack", P, x, dtype, stride, t_begin, T, (T + 3) / 4, &sh)) return rc;
+  if (int rc = pull_check("ctb_pull_pack", P, x, dtype, float_bytes(dtype), stride, t_begin, T, (T + 3) / 4, &sh)) return rc;
   if (!dst && T > 0) { ctb_set_error("ctb_pull_pack: dst is null"); return CTB_ERR_INVALID; }
   return pull_launch(P, T, [&] {
     pull_pack_kernel<<<sh.grid, 256, 0, (cudaStream_t)stream>>>(
@@ -948,14 +955,60 @@ __device__ __forceinline__ uint4 unit_put(const double (&e)[2]) {
                     (unsigned)__double2hiint(e[1]));
 }
 
-// The step loop of both sub-daily kernels.  Item = one 16-byte unit u of a packed plane x one day d: step(e) gets
-// the C = 16 / sizeof(T) elements of each of the day's S steps, in step order, then item(d, u) stores the item's
-// results and resets the kernel's accumulators for the next item.  Padding units call neither.
-template <typename T, typename Step, typename Item>
-__device__ __forceinline__ void subdaily_step_loop(const uint4* src, int64_t stride16, int S, const int32_t* day,
-                                                   int64_t t_begin, int n_days, const int32_t* pack_src, int n_units,
-                                                   int halves, Step&& step, Item&& item) {
-  constexpr int C = 16 / sizeof(T);   // cells per 16-byte unit
+// Sources of the step loop: how one unit of a source piece is loaded and unpacked into C elements of type E.
+// A float source: a unit is 16 bytes, C = 16 / sizeof(T) elements as stored.
+template <typename T>
+struct FloatSrc {
+  using E = T;
+  using V = uint4;
+  static constexpr int C = 16 / sizeof(T);
+  __device__ __forceinline__ void load(V& v, const V* p) const {
+    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
+                 : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
+  }
+  __device__ __forceinline__ void get(const V& v, T (&e)[C]) const { unit_get(v, e); }
+};
+
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+
+// A CF-packed int16 source (netCDF short): a unit is one 4-cell piece, 8 bytes.  Raw value r decodes to NaN when
+// it is a fill value, else to fl(fl(D(r) * scale) + offset) in D: two rounded operations, no contraction, which
+// is numpy's r.astype(D) * D(scale) + D(offset) bit for bit.
+template <typename D>
+struct PackedI16Src {
+  using E = D;
+  using V = uint2;
+  static constexpr int C = 4;
+  D scale, offset;
+  int fill[4];   // raw fill values; unused slots hold 0x10000, which no int16 equals
+  __device__ __forceinline__ void load(V& v, const V* p) const {
+    asm volatile("ld.global.nc.L1::no_allocate.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p));
+  }
+  __device__ __forceinline__ void get(const V& v, D (&e)[4]) const {
+    const int r[4] = {(int)(short)(v.x & 0xffff), (int)(short)(v.x >> 16), (int)(short)(v.y & 0xffff),
+                      (int)(short)(v.y >> 16)};
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      const bool masked = r[c] == fill[0] || r[c] == fill[1] || r[c] == fill[2] || r[c] == fill[3];
+      e[c] = masked ? (D)NAN : add_rn(mul_rn((D)r[c], scale), offset);
+    }
+  }
+};
+
+// The step loop of the sub-daily kernels.  Item = one unit u of a packed plane x one day d: step(e) gets the
+// Src::C elements of each of the day's S steps, in step order, then item(d, u) stores the item's results and
+// resets the kernel's accumulators for the next item.  Padding units call neither.  stride16 is the source's
+// plane stride in units.
+template <typename Src, typename Step, typename Item>
+__device__ __forceinline__ void subdaily_step_loop(const Src& sp, const typename Src::V* src, int64_t stride16, int S,
+                                                   const int32_t* day, int64_t t_begin, int n_days,
+                                                   const int32_t* pack_src, int n_units, int halves, Step&& step,
+                                                   Item&& item) {
+  using T = typename Src::E;
+  constexpr int C = Src::C;           // cells per unit
   constexpr int U = 8;                // step loads in flight
   const int64_t n_work = (int64_t)n_units * n_days;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n_work; i += (int64_t)gridDim.x * blockDim.x) {
@@ -964,20 +1017,17 @@ __device__ __forceinline__ void subdaily_step_loop(const uint4* src, int64_t str
     const int p = __ldg(pack_src + u / halves);
     if (p < 0) continue;                       // alignment padding of the packed plane: never read
     const int64_t step0 = (int64_t)(day ? __ldg(day + t_begin + d) : t_begin + d) * S;
-    const uint4* s = src + step0 * stride16 + (int64_t)p * halves + (u % halves);
+    const typename Src::V* s = src + step0 * stride16 + (int64_t)p * halves + (u % halves);
     for (int h0 = 0; h0 < S; h0 += U) {
-      uint4 v[U];
+      typename Src::V v[U];
 #pragma unroll
       for (int k = 0; k < U; ++k)
-        if (h0 + k < S)
-          asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];"
-                       : "=r"(v[k].x), "=r"(v[k].y), "=r"(v[k].z), "=r"(v[k].w)
-                       : "l"(s + (int64_t)(h0 + k) * stride16));
+        if (h0 + k < S) sp.load(v[k], s + (int64_t)(h0 + k) * stride16);
 #pragma unroll
       for (int k = 0; k < U; ++k)
         if (h0 + k < S) {
           T e[C];
-          unit_get(v[k], e);
+          sp.get(v[k], e);
           step(e);
         }
     }
@@ -985,12 +1035,25 @@ __device__ __forceinline__ void subdaily_step_loop(const uint4* src, int64_t str
   }
 }
 
-template <typename T, bool MEAN, bool EXT>
-__global__ void __launch_bounds__(256) subdaily_pack_kernel(
-    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
-    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, double2* __restrict__ dst_mean,
-    uint4* __restrict__ dst_min, uint4* __restrict__ dst_max) {
-  constexpr int C = 16 / sizeof(T);
+// Stores the C elements of one item to a plane of T at item index i: one 16-byte unit, or two (4 float64 cells)
+template <typename T, int C>
+__device__ __forceinline__ void item_put(uint4* dst, int64_t i, const T (&e)[C]) {
+  if constexpr (C * sizeof(T) == 16) {
+    dst[i] = unit_put(e);
+  } else {
+    dst[2 * i] = unit_put({e[0], e[1]});
+    dst[2 * i + 1] = unit_put({e[2], e[3]});
+  }
+}
+
+// Daily mean / min / max of the steps of one item: the body of subdaily_pack_kernel for a source Src
+template <typename Src, bool MEAN, bool EXT>
+__device__ __forceinline__ void subdaily_pack(const Src& sp, const typename Src::V* src, int64_t stride16, int S,
+                                              const int32_t* day, int64_t t_begin, int n_days,
+                                              const int32_t* pack_src, int n_units, int halves, double2* dst_mean,
+                                              uint4* dst_min, uint4* dst_max) {
+  using T = typename Src::E;
+  constexpr int C = Src::C;
   double sum[C];
   int cnt[C];
   T mn[C], mx[C];
@@ -1003,8 +1066,8 @@ __global__ void __launch_bounds__(256) subdaily_pack_kernel(
     }
   };
   reset();
-  subdaily_step_loop<T>(
-      src, stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
+  subdaily_step_loop(
+      sp, src, stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
       [&](const T (&e)[C]) {
 #pragma unroll
         for (int c = 0; c < C; ++c) {
@@ -1020,44 +1083,109 @@ __global__ void __launch_bounds__(256) subdaily_pack_kernel(
                 make_double2(__ddiv_rn(sum[c], (double)cnt[c]), __ddiv_rn(sum[c + 1], (double)cnt[c + 1]));
         }
         if (EXT) {
-          if (dst_min) dst_min[(int64_t)d * n_units + u] = unit_put(mn);
-          if (dst_max) dst_max[(int64_t)d * n_units + u] = unit_put(mx);
+          if (dst_min) item_put(dst_min, (int64_t)d * n_units + u, mn);
+          if (dst_max) item_put(dst_max, (int64_t)d * n_units + u, mx);
         }
         reset();
       });
 }
+
+template <typename T, bool MEAN, bool EXT>
+__global__ void __launch_bounds__(256) subdaily_pack_kernel(
+    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
+    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, double2* __restrict__ dst_mean,
+    uint4* __restrict__ dst_min, uint4* __restrict__ dst_max) {
+  subdaily_pack<FloatSrc<T>, MEAN, EXT>(FloatSrc<T>{}, src, stride16, S, day, t_begin, n_days, pack_src, n_units,
+                                        halves, dst_mean, dst_min, dst_max);
+}
+
+// subdaily_pack_kernel of a CF-packed int16 source decoded to D; a unit of the source is a piece (halves = 1).
+// (256, 2): without the bound ptxas spills 8 bytes around the division's slow path in <double, mean only>
+template <typename D, bool MEAN, bool EXT>
+__global__ void __launch_bounds__(256, 2) subdaily_pack_decode_kernel(
+    const uint2* __restrict__ src, int64_t stride8, const PackedI16Src<D> dec, int S, const int32_t* __restrict__ day,
+    int64_t t_begin, int n_days, const int32_t* __restrict__ pack_src, int n_units, double2* __restrict__ dst_mean,
+    uint4* __restrict__ dst_min, uint4* __restrict__ dst_max) {
+  subdaily_pack<PackedI16Src<D>, MEAN, EXT>(dec, src, stride8, S, day, t_begin, n_days, pack_src, n_units, 1,
+                                            dst_mean, dst_min, dst_max);
+}
+
+// Decode-pack of daily int16 data: the step loop with one step per day, day_index as the time index, and the
+// decoded values stored to packed planes of D
+template <typename D>
+__global__ void __launch_bounds__(256) pull_pack_decode_kernel(
+    const uint2* __restrict__ src, int64_t stride8, const PackedI16Src<D> dec, const int32_t* __restrict__ tix,
+    int64_t t_begin, int T, const int32_t* __restrict__ pack_src, int n_units, uint4* __restrict__ dst) {
+  D y[4];
+  subdaily_step_loop(
+      dec, src, stride8, 1, tix, t_begin, T, pack_src, n_units, 1,
+      [&](const D (&e)[4]) {
+#pragma unroll
+        for (int c = 0; c < 4; ++c) y[c] = e[c];
+      },
+      [&](int d, int u) { item_put(dst, (int64_t)d * n_units + u, y); });
+}
 }  // namespace
 
-extern "C" int ctb_pull_pack_daily(const ctb_plan* P, const void* x, int dtype, int64_t stride, int steps_per_day,
-                                   const int32_t* day_index, int64_t t_begin, int64_t n_days, int ops,
-                                   void* dst_mean, void* dst_min, void* dst_max, void* stream) {
+namespace {
+// The CF decoding of an int16 source as the kernels take it.  CTB_ERR_INVALID for a null dec, a non-finite scale
+// or offset, n_fill outside 0..4 or a dtype other than F32 / F64.
+int decode_check(const char* fn, const ctb_decode* dec) {
+  if (!dec) { ctb_set_error("%s: dec is null", fn); return CTB_ERR_INVALID; }
+  if (!std::isfinite(dec->scale) || !std::isfinite(dec->offset) || dec->n_fill < 0 || dec->n_fill > 4 ||
+      (dec->dtype != CTB_F32 && dec->dtype != CTB_F64)) {
+    ctb_set_error("%s: dec needs a finite scale and offset, 0..4 fill values and dtype F32 or F64, got scale=%g, "
+                  "offset=%g, n_fill=%d, dtype=%d", fn, dec->scale, dec->offset, dec->n_fill, dec->dtype);
+    return CTB_ERR_INVALID;
+  }
+  return CTB_OK;
+}
+
+template <typename D>
+PackedI16Src<D> decode_src(const ctb_decode& dec) {
+  PackedI16Src<D> s;
+  s.scale = (D)dec.scale;
+  s.offset = (D)dec.offset;
+  for (int k = 0; k < 4; ++k) s.fill[k] = k < dec.n_fill ? (int)dec.fill[k] : 0x10000;
+  return s;
+}
+
+// Bytes per decoded element
+int decoded_bytes(const ctb_decode& dec) { return dec.dtype == CTB_F32 ? 4 : 8; }
+
+// ctb_pull_pack_daily (es = float_bytes(dtype)), and with es = 2 its CF-decoding counterpart for int16 sources
+int pull_pack_daily(const char* fn, const ctb_plan* P, const void* x, int dtype, int64_t es, const ctb_decode* dec,
+                    int64_t stride, int steps_per_day, const int32_t* day_index, int64_t t_begin, int64_t n_days,
+                    int ops, void* dst_mean, void* dst_min, void* dst_max, void* stream) {
   PullShape sh;
-  if (int rc = pull_check("ctb_pull_pack_daily", P, x, dtype, stride, t_begin, n_days, n_days, &sh)) return rc;
+  if (int rc = pull_check(fn, P, x, dtype, es, stride, t_begin, n_days, n_days, &sh)) return rc;
+  if (es != 2) dec = nullptr;
+  else if (int rc = decode_check(fn, dec)) return rc;
   if (steps_per_day < 1) {
-    ctb_set_error("ctb_pull_pack_daily: steps_per_day=%d, needs >= 1", steps_per_day);
+    ctb_set_error("%s: steps_per_day=%d, needs >= 1", fn, steps_per_day);
     return CTB_ERR_INVALID;
   }
   if (ops == 0 || (ops & ~(CTB_DAILY_MEAN | CTB_DAILY_MIN | CTB_DAILY_MAX))) {
-    ctb_set_error("ctb_pull_pack_daily: ops=%d, needs a non-empty subset of CTB_DAILY_MEAN|MIN|MAX", ops);
+    ctb_set_error("%s: ops=%d, needs a non-empty subset of CTB_DAILY_MEAN|MIN|MAX", fn, ops);
     return CTB_ERR_INVALID;
   }
   if (((ops & CTB_DAILY_MEAN) && !dst_mean) || ((ops & CTB_DAILY_MIN) && !dst_min) ||
       ((ops & CTB_DAILY_MAX) && !dst_max)) {
-    ctb_set_error("ctb_pull_pack_daily: every requested op needs a destination");
+    ctb_set_error("%s: every requested op needs a destination", fn);
     return CTB_ERR_INVALID;
   }
   if ((ops & CTB_DAILY_MEAN) && P->elem_bytes != 8) {
-    ctb_set_error("ctb_pull_pack_daily: the mean plane is float64, the plan was built for %d-byte elements",
-                  P->elem_bytes);
+    ctb_set_error("%s: the mean plane is float64, the plan was built for %d-byte elements", fn, P->elem_bytes);
     return CTB_ERR_INVALID;
   }
-  if ((ops & (CTB_DAILY_MIN | CTB_DAILY_MAX)) && P->elem_bytes != sh.es) {
-    ctb_set_error("ctb_pull_pack_daily: min/max planes have the source's %d-byte elements, the plan was built "
-                  "for %d-byte elements", (int)sh.es, P->elem_bytes);
+  const int ext_bytes = dec ? decoded_bytes(*dec) : (int)sh.es;   // min / max planes: the source's (decoded) type
+  if ((ops & (CTB_DAILY_MIN | CTB_DAILY_MAX)) && P->elem_bytes != ext_bytes) {
+    ctb_set_error("%s: min/max planes have the source's %d-byte elements, the plan was built for %d-byte elements",
+                  fn, ext_bytes, P->elem_bytes);
     return CTB_ERR_INVALID;
   }
   if ((uintptr_t)dst_mean % 16 != 0 || (uintptr_t)dst_min % 16 != 0 || (uintptr_t)dst_max % 16 != 0) {
-    ctb_set_error("ctb_pull_pack_daily: destination planes must be 16-byte aligned");
+    ctb_set_error("%s: destination planes must be 16-byte aligned", fn);
     return CTB_ERR_UNSUPPORTED;
   }
   const bool mean = ops & CTB_DAILY_MEAN, ext = ops & (CTB_DAILY_MIN | CTB_DAILY_MAX);
@@ -1072,7 +1200,58 @@ extern "C" int ctb_pull_pack_daily(const ctb_plan* P, const void* x, int dtype, 
                                                   static_cast<double2*>(dst_mean), dmin, dmax);
     return CTB_OK;
   };
-  return pull_launch(P, n_days, [&] { return dtype == CTB_F32 ? go(float{}) : go(double{}); });
+  auto go_decode = [&](auto tag) {
+    using D = decltype(tag);
+    auto k = mean ? (ext ? subdaily_pack_decode_kernel<D, true, true> : subdaily_pack_decode_kernel<D, true, false>)
+                  : subdaily_pack_decode_kernel<D, false, true>;
+    k<<<sh.grid, 256, 0, (cudaStream_t)stream>>>(static_cast<const uint2*>(x), sh.stride16, decode_src<D>(*dec),
+                                                  steps_per_day, day_index, t_begin, (int)n_days, P->d_pack_src,
+                                                  sh.n_units, static_cast<double2*>(dst_mean), dmin, dmax);
+    return CTB_OK;
+  };
+  return pull_launch(P, n_days, [&] {
+    if (dec) return dec->dtype == CTB_F32 ? go_decode(float{}) : go_decode(double{});
+    return dtype == CTB_F32 ? go(float{}) : go(double{});
+  });
+}
+}  // namespace
+
+extern "C" int ctb_pull_pack_daily(const ctb_plan* P, const void* x, int dtype, int64_t stride, int steps_per_day,
+                                   const int32_t* day_index, int64_t t_begin, int64_t n_days, int ops,
+                                   void* dst_mean, void* dst_min, void* dst_max, void* stream) {
+  return pull_pack_daily("ctb_pull_pack_daily", P, x, dtype, float_bytes(dtype), nullptr, stride, steps_per_day, day_index, t_begin,
+                         n_days, ops, dst_mean, dst_min, dst_max, stream);
+}
+
+extern "C" int ctb_pull_pack_daily_decode(const ctb_plan* P, const int16_t* x, int64_t stride, const ctb_decode* dec,
+                                          int steps_per_day, const int32_t* day_index, int64_t t_begin,
+                                          int64_t n_days, int ops, void* dst_mean, void* dst_min, void* dst_max,
+                                          void* stream) {
+  return pull_pack_daily("ctb_pull_pack_daily_decode", P, x, 0, 2, dec, stride, steps_per_day, day_index, t_begin,
+                         n_days, ops, dst_mean, dst_min, dst_max, stream);
+}
+
+extern "C" int ctb_pull_pack_decode(const ctb_plan* P, const int16_t* x, int64_t stride, const ctb_decode* dec,
+                                    const int32_t* time_index, int64_t t_begin, int64_t T, void* dst, void* stream) {
+  const char* fn = "ctb_pull_pack_decode";
+  PullShape sh;
+  if (int rc = pull_check(fn, P, x, 0, 2, stride, t_begin, T, T, &sh)) return rc;
+  if (int rc = decode_check(fn, dec)) return rc;
+  if (!dst && T > 0) { ctb_set_error("%s: dst is null", fn); return CTB_ERR_INVALID; }
+  if (P->elem_bytes != decoded_bytes(*dec)) {
+    ctb_set_error("%s: the planes have %d-byte elements, the plan was built for %d-byte elements", fn,
+                  decoded_bytes(*dec), P->elem_bytes);
+    return CTB_ERR_INVALID;
+  }
+  if ((uintptr_t)dst % 16 != 0) { ctb_set_error("%s: dst must be 16-byte aligned", fn); return CTB_ERR_UNSUPPORTED; }
+  auto go = [&](auto tag) {
+    using D = decltype(tag);
+    pull_pack_decode_kernel<D><<<sh.grid, 256, 0, (cudaStream_t)stream>>>(
+        static_cast<const uint2*>(static_cast<const void*>(x)), sh.stride16, decode_src<D>(*dec), time_index, t_begin,
+        (int)T, P->d_pack_src, sh.n_units, static_cast<uint4*>(dst));
+    return CTB_OK;
+  };
+  return pull_launch(P, T, [&] { return dec->dtype == CTB_F32 ? go(float{}) : go(double{}); });
 }
 
 // Per-step transforms of sub-daily sources, reduced to daily means in the same read: the step loop and the plane
@@ -1091,11 +1270,13 @@ struct StepDst {
 
 // (256, 2): at most 128 registers, which every instantiation fits (the largest uses 127); without the bound
 // ptxas spills 8 bytes around the division's slow path in one of them
-template <typename T, int OP, int NOUT>
-__global__ void __launch_bounds__(256, 2) subdaily_steps_kernel(
-    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
-    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, const CtbTr tr, StepDst dst) {
-  constexpr int C = 16 / sizeof(T);
+template <typename Src, int OP, int NOUT>
+__device__ __forceinline__ void subdaily_steps(const Src& sp, const typename Src::V* src, int64_t stride16, int S,
+                                               const int32_t* day, int64_t t_begin, int n_days,
+                                               const int32_t* pack_src, int n_units, int halves, const CtbTr& tr,
+                                               const StepDst& dst) {
+  using T = typename Src::E;
+  constexpr int C = Src::C;
   constexpr bool F32 = sizeof(T) == 4;
   double w[NOUT];                     // GDD: hi - lo of every pair
 #pragma unroll
@@ -1115,8 +1296,8 @@ __global__ void __launch_bounds__(256, 2) subdaily_steps_kernel(
     }
   };
   reset();
-  subdaily_step_loop<T>(
-      src, stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
+  subdaily_step_loop(
+      sp, src, stride16, S, day, t_begin, n_days, pack_src, n_units, halves,
       [&](const T (&e)[C]) {
 #pragma unroll
         for (int c = 0; c < C; ++c) {
@@ -1159,36 +1340,57 @@ __global__ void __launch_bounds__(256, 2) subdaily_steps_kernel(
         reset();
       });
 }
+
+template <typename T, int OP, int NOUT>
+__global__ void __launch_bounds__(256, 2) subdaily_steps_kernel(
+    const uint4* __restrict__ src, int64_t stride16, int S, const int32_t* __restrict__ day, int64_t t_begin,
+    int n_days, const int32_t* __restrict__ pack_src, int n_units, int halves, const CtbTr tr, StepDst dst) {
+  subdaily_steps<FloatSrc<T>, OP, NOUT>(FloatSrc<T>{}, src, stride16, S, day, t_begin, n_days, pack_src, n_units,
+                                        halves, tr, dst);
+}
+
+// subdaily_steps_kernel of a CF-packed int16 source decoded to D; a unit of the source is a piece (halves = 1)
+template <typename D, int OP, int NOUT>
+__global__ void __launch_bounds__(256, 2) subdaily_steps_decode_kernel(
+    const uint2* __restrict__ src, int64_t stride8, const PackedI16Src<D> dec, int S, const int32_t* __restrict__ day,
+    int64_t t_begin, int n_days, const int32_t* __restrict__ pack_src, int n_units, const CtbTr tr, StepDst dst) {
+  subdaily_steps<PackedI16Src<D>, OP, NOUT>(dec, src, stride8, S, day, t_begin, n_days, pack_src, n_units, 1, tr,
+                                            dst);
+}
 }  // namespace
 
-extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int dtype, int64_t stride,
-                                         int steps_per_day, const int32_t* day_index, int64_t t_begin,
-                                         int64_t n_days, int step_op, const double* params, int n_params, int n_out,
-                                         double* const* dst, void* stream) {
+namespace {
+// ctb_pull_pack_daily_steps (es = float_bytes(dtype)), and with es = 2 its CF-decoding counterpart for int16 sources
+int pull_pack_daily_steps(const char* fn, const ctb_plan* P, const void* x, int dtype, int64_t es,
+                          const ctb_decode* dec, int64_t stride, int steps_per_day, const int32_t* day_index,
+                          int64_t t_begin, int64_t n_days, int step_op, const double* params, int n_params, int n_out,
+                          double* const* dst, void* stream) {
   PullShape sh;
-  if (int rc = pull_check("ctb_pull_pack_daily_steps", P, x, dtype, stride, t_begin, n_days, n_days, &sh)) return rc;
+  if (int rc = pull_check(fn, P, x, dtype, es, stride, t_begin, n_days, n_days, &sh)) return rc;
+  if (es != 2) dec = nullptr;
+  else if (int rc = decode_check(fn, dec)) return rc;
   if (steps_per_day < 1) {
-    ctb_set_error("ctb_pull_pack_daily_steps: steps_per_day=%d, needs >= 1", steps_per_day);
+    ctb_set_error("%s: steps_per_day=%d, needs >= 1", fn, steps_per_day);
     return CTB_ERR_INVALID;
   }
   if (step_op != CTB_STEP_EDD && step_op != CTB_STEP_GDD && step_op != CTB_STEP_BINS) {
-    ctb_set_error("ctb_pull_pack_daily_steps: step_op=%d, needs CTB_STEP_EDD, GDD or BINS", step_op);
+    ctb_set_error("%s: step_op=%d, needs CTB_STEP_EDD, GDD or BINS", fn, step_op);
     return CTB_ERR_INVALID;
   }
   if (n_out < 1 || n_out > CTB_MAX_OUT) {
-    ctb_set_error("ctb_pull_pack_daily_steps: n_out=%d out of range 1..%d", n_out, CTB_MAX_OUT);
+    ctb_set_error("%s: n_out=%d out of range 1..%d", fn, n_out, CTB_MAX_OUT);
     return CTB_ERR_INVALID;
   }
   const int need = step_op == CTB_STEP_EDD ? n_out : step_op == CTB_STEP_GDD ? 2 * n_out : n_out + 1;
   if (n_params != need || !params) {
-    ctb_set_error("ctb_pull_pack_daily_steps: step_op %d with n_out=%d needs %d params, got %d", step_op, n_out,
+    ctb_set_error("%s: step_op %d with n_out=%d needs %d params, got %d", fn, step_op, n_out,
                   need, n_params);
     return CTB_ERR_INVALID;
   }
   for (int j = 0; j < n_params && step_op != CTB_STEP_BINS; ++j) {
     if (!std::isfinite(params[j]) || (step_op == CTB_STEP_GDD && j % 2 == 1 && !(params[j - 1] < params[j]))) {
-      ctb_set_error("ctb_pull_pack_daily_steps: thresholds must be finite, with lo < hi in every GDD pair: "
-                    "param %d is %g", j, params[j]);
+      ctb_set_error("%s: thresholds must be finite, with lo < hi in every GDD pair: "
+                    "param %d is %g", fn, j, params[j]);
       return CTB_ERR_INVALID;
     }
   }
@@ -1202,18 +1404,18 @@ extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int d
     rc = ctb_pack_transform(step_op == CTB_STEP_EDD ? CTB_TR_EDD : CTB_TR_GDD, params, n_params, n_out, &tr);
   }
   if (rc != CTB_OK) return rc;
-  if (!dst) { ctb_set_error("ctb_pull_pack_daily_steps: dst is null"); return CTB_ERR_INVALID; }
+  if (!dst) { ctb_set_error("%s: dst is null", fn); return CTB_ERR_INVALID; }
   StepDst planes{};
   for (int j = 0; j < n_out; ++j) {
-    if (!dst[j]) { ctb_set_error("ctb_pull_pack_daily_steps: dst[%d] is null", j); return CTB_ERR_INVALID; }
+    if (!dst[j]) { ctb_set_error("%s: dst[%d] is null", fn, j); return CTB_ERR_INVALID; }
     if ((uintptr_t)dst[j] % 16 != 0) {
-      ctb_set_error("ctb_pull_pack_daily_steps: dst[%d] is not 16-byte aligned", j);
+      ctb_set_error("%s: dst[%d] is not 16-byte aligned", fn, j);
       return CTB_ERR_UNSUPPORTED;
     }
     planes.p[j] = reinterpret_cast<double2*>(dst[j]);
   }
   if (P->elem_bytes != 8) {
-    ctb_set_error("ctb_pull_pack_daily_steps: the planes are float64, the plan was built for %d-byte elements",
+    ctb_set_error("%s: the planes are float64, the plan was built for %d-byte elements", fn,
                   P->elem_bytes);
     return CTB_ERR_INVALID;
   }
@@ -1228,7 +1430,40 @@ extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int d
     if (step_op == CTB_STEP_GDD) return ctb_dispatch_nout<CTB_STEP_GDD>(n_out, launch);
     return ctb_dispatch_nout<CTB_STEP_BINS>(n_out, launch);
   };
-  return pull_launch(P, n_days, [&] { return dtype == CTB_F32 ? go(float{}) : go(double{}); });
+  auto go_decode = [&](auto tag) {
+    using D = decltype(tag);
+    auto launch = [&](auto op, auto nout) {
+      subdaily_steps_decode_kernel<D, op, nout><<<sh.grid, 256, 0, (cudaStream_t)stream>>>(
+          static_cast<const uint2*>(x), sh.stride16, decode_src<D>(*dec), steps_per_day, day_index, t_begin,
+          (int)n_days, P->d_pack_src, sh.n_units, tr, planes);
+      return CTB_OK;
+    };
+    if (step_op == CTB_STEP_EDD) return ctb_dispatch_nout<CTB_STEP_EDD>(n_out, launch);
+    if (step_op == CTB_STEP_GDD) return ctb_dispatch_nout<CTB_STEP_GDD>(n_out, launch);
+    return ctb_dispatch_nout<CTB_STEP_BINS>(n_out, launch);
+  };
+  return pull_launch(P, n_days, [&] {
+    if (dec) return dec->dtype == CTB_F32 ? go_decode(float{}) : go_decode(double{});
+    return dtype == CTB_F32 ? go(float{}) : go(double{});
+  });
+}
+}  // namespace
+
+extern "C" int ctb_pull_pack_daily_steps(const ctb_plan* P, const void* x, int dtype, int64_t stride,
+                                         int steps_per_day, const int32_t* day_index, int64_t t_begin,
+                                         int64_t n_days, int step_op, const double* params, int n_params, int n_out,
+                                         double* const* dst, void* stream) {
+  return pull_pack_daily_steps("ctb_pull_pack_daily_steps", P, x, dtype, float_bytes(dtype), nullptr, stride,
+                               steps_per_day, day_index, t_begin, n_days, step_op, params, n_params, n_out, dst,
+                               stream);
+}
+
+extern "C" int ctb_pull_pack_daily_steps_decode(const ctb_plan* P, const int16_t* x, int64_t stride,
+                                                const ctb_decode* dec, int steps_per_day, const int32_t* day_index,
+                                                int64_t t_begin, int64_t n_days, int step_op, const double* params,
+                                                int n_params, int n_out, double* const* dst, void* stream) {
+  return pull_pack_daily_steps("ctb_pull_pack_daily_steps_decode", P, x, 0, 2, dec, stride, steps_per_day,
+                               day_index, t_begin, n_days, step_op, params, n_params, n_out, dst, stream);
 }
 
 // ---------------------------------------------------------------------------

@@ -19,10 +19,11 @@ __all__ = ["snyder_edd", "snyder_gdd", "subdaily_edd", "subdaily_gdd", "subdaily
 
 
 def _source(da):
-    """The stored data a transform reads: daily reductions of sub-daily data stay deferred (they are
-    reduced while the aggregation packs its inputs), other deferred variables are evaluated."""
+    """The stored data a transform reads: daily reductions of sub-daily data and decoded packed sources stay
+    deferred (they are reduced or decoded while the aggregation packs its inputs), other deferred variables are
+    evaluated."""
     v = da.variable
-    return v if v.deferred is None or v.deferred.kind == "daily" else Variable(v.dims, v.values, v.attrs)
+    return v if v.deferred is None or v.deferred.kind in ("daily", "decode") else Variable(v.dims, v.values, v.attrs)
 
 
 def _min_max_of_one_source(a, b):

@@ -27,7 +27,9 @@ def convert_kelvin_to_celsius(df, temp_name):
     var = ds._vars[temp_name]
     attrs = dict(var.attrs)
     attrs.update(units="C", valid_min=-108.78788, valid_max=62.02828)
-    src = var if var.deferred is None else Variable(var.dims, var.values, var.attrs)
+    # daily reductions and decoded packed sources stay deferred: they are evaluated while the aggregation packs
+    src = var if var.deferred is None or var.deferred.kind in ("daily", "decode") else \
+        Variable(var.dims, var.values, var.attrs)
     out = ds.copy()
     out._vars[temp_name] = Variable(var.dims, None, attrs, None,
                                     Deferred("poly", (273.15, 1.0), (src,)))
@@ -130,7 +132,7 @@ def resample_daily(ds, how="mean"):
     Variables over ``(time, lat, lon)`` become deferred daily variables over ``(time, lat, lon)`` with
     ``time`` as the day (``datetime64[D]``); other variables without ``time`` are kept.  The reduction runs
     on the GPU per gridcell while the referenced gridcells are packed for aggregation, so the daily grid is
-    never built: the result feeds ``tas_poly``, ``tas_bins``, ``tas_rcspline``, ``snyder_edd`` /
+    never built (a CF-packed source from ``io.decode_packed`` is decoded in the same read): the result feeds ``tas_poly``, ``tas_bins``, ``tas_rcspline``, ``snyder_edd`` /
     ``snyder_gdd``, ``remove_leap_days`` and ``weighted_aggregate_grid_to_regions`` (with ``time_groups=``,
     ``season_mask=``) and ``weighted_aggregate_grid_to_regions_multi`` directly, and ``.values`` computes it
     for the whole grid.  Transforms that are nonlinear in each step -- degree days and time per temperature
@@ -173,17 +175,21 @@ def _resample(ds, how, attrs=None):
                                       "(time, lat, lon)".format(name, var.dims))
         if var.dims != ("time", "lat", "lon"):
             raise ValueError("resample_daily: {!r} is over {}, expected (time, lat, lon)".format(name, var.dims))
-        if var.deferred is not None:
+        decode = var.deferred is not None and var.deferred.kind == "decode"
+        if var.deferred is not None and not decode:
             raise ValueError("resample_daily: {!r} is a deferred variable, not stored data".format(name))
+        raw = var.deferred.sources[0] if decode else var      # a decoded source: the takes are the raw source's
         # the kernel reads whole days from the first step on: a time take must be one run of steps
         t0 = 0
-        takes = dict(var.takes)
+        takes = dict(raw.takes)
         pos = takes.pop("time", None)
         if pos is not None:
             if len(pos) and not np.array_equal(pos, np.arange(pos[0], pos[0] + len(pos))):
                 raise NotImplementedError("resample_daily: {!r} selects time steps out of physical order".format(name))
             t0 = int(pos[0]) if len(pos) else 0
-        src = Variable(var.dims, var.physical, var.attrs, takes)
+        src = Variable(var.dims, raw.physical, raw.attrs, takes)
+        if decode:
+            src = Variable(var.dims, None, var.attrs, None, Deferred("decode", var.deferred.params, (src,)))
         if attrs is None:
             a = dict(var.attrs)
             a["cell_methods"] = "time: {}".format(how)

@@ -296,6 +296,37 @@ int ctb_pull_pack_daily_steps(const ctb_plan* plan, const void* x, int dtype, in
                               const int32_t* day_index, int64_t t_begin, int64_t n_days, int step_op,
                               const double* params, int n_params, int n_out, double* const* dst, void* stream);
 
+/* ---- CF-packed int16 sources (netCDF short with scale_factor / add_offset / _FillValue / missing_value) ---- *
+ * Each raw value r of x (int16, TIME_MAJOR, DEVICE or pinned HOST memory) is decoded to y in D = dec->dtype:
+ *   y = NaN                                        if r is one of dec->fill[0 .. n_fill - 1]
+ *   y = fl_D(fl_D(D(r) * D(scale)) + D(offset))    otherwise: two rounded operations, no contraction
+ * which is numpy's r.astype(D) * D(scale) + D(offset) bit for bit.  Downstream, y is exactly what a float source
+ * of dtype D holding the decoded values gives.  Each entry point is its float counterpart with `dtype` replaced
+ * by `dec`:
+ *   ctb_pull_pack_decode:             packed planes of D (plan elem_bytes = sizeof(D)), time_index as in ctb_pull_pack;
+ *   ctb_pull_pack_daily_decode:       mean planes float64 (elem_bytes 8), min / max planes of D (elem_bytes sizeof(D));
+ *   ctb_pull_pack_daily_steps_decode: float64 planes (elem_bytes 8); for D = float32 the thresholds are compared
+ *                                     in fp32 as for float sources.
+ * Source planes must be 8-byte aligned and hold a multiple of 4 gridcells (else CTB_ERR_UNSUPPORTED).  A null dec,
+ * a non-finite scale or offset, n_fill outside 0..4 or a dtype other than CTB_F32 / CTB_F64 is CTB_ERR_INVALID;
+ * every refused call writes nothing. */
+typedef struct ctb_decode {      /* CF packing of an int16 (netCDF short) source */
+  double scale;                  /* finite (1 when the attribute is absent) */
+  double offset;                 /* finite (0 when absent) */
+  int32_t dtype;                 /* CTB_F32 / CTB_F64: D, the type y is computed and stored in */
+  int32_t n_fill;                /* 0..4 */
+  int16_t fill[4];               /* raw values that decode to NaN */
+} ctb_decode;
+int ctb_pull_pack_decode(const ctb_plan* plan, const int16_t* x, int64_t stride, const ctb_decode* dec,
+                         const int32_t* time_index, int64_t t_begin, int64_t T, void* dst, void* stream);
+int ctb_pull_pack_daily_decode(const ctb_plan* plan, const int16_t* x, int64_t stride, const ctb_decode* dec,
+                               int steps_per_day, const int32_t* day_index, int64_t t_begin, int64_t n_days, int ops,
+                               void* dst_mean, void* dst_min, void* dst_max, void* stream);
+int ctb_pull_pack_daily_steps_decode(const ctb_plan* plan, const int16_t* x, int64_t stride, const ctb_decode* dec,
+                                     int steps_per_day, const int32_t* day_index, int64_t t_begin, int64_t n_days,
+                                     int step_op, const double* params, int n_params, int n_out, double* const* dst,
+                                     void* stream);
+
 /* rows of a pitched DEVICE array -> pitched HOST (pinned) array, one asynchronous 2-D copy on `stream`:
  * the host path returns out[:, :, t0:t1] of a finished time chunk while the next chunk is in flight */
 int ctb_copy_rows_to_host(void* dst, size_t dst_pitch, const void* src, size_t src_pitch, size_t width_bytes,
